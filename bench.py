@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the SNR-aligned diffusion enhancement hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): sebridge_v3 NCSN++ (65.6 M parameters, seeded synthetic
 "de-degenerated" weights), a batch of 16 synthetic 4 s / 16 kHz utterances per GPU, the full
@@ -348,7 +348,13 @@ def run_b200(args):
     stream = torch.cuda.Stream(device=dev)
 
     from snr_aligned_diffse_b200.pipeline import GraphedEnhancer
-    pipe = GraphedEnhancer(model, BATCH, L, dev, oracle=False, stream=stream)
+
+    def noise_generator(k):
+        # a seeded generator per enhancer: the enhancers' replays overlap, and graphs that share torch's default generator
+        # would read each other's noise offsets (pipeline.GraphedEnhancer)
+        return torch.Generator(device=dev).manual_seed(100 * rank + k)
+
+    pipe = GraphedEnhancer(model, BATCH, L, dev, oracle=False, stream=stream, generator=noise_generator(0))
     pipe.y_dev.copy_(y_dev)
     y_dev = pipe.y_dev
     # --streams 2: a second, independent enhancer (own network workspace, own streams); consecutive steps alternate
@@ -356,9 +362,9 @@ def run_b200(args):
     # front end, the SNR estimator, the iSTFT) overlap the other batch's work.  Every step is still one full pass over
     # one batch of 16 utterances.
     pipes = [pipe]
-    for _ in range(args.streams - 1):
+    for k in range(1, args.streams):
         model2, _ = build_models(dev, with_estimator=False)   # the estimator (weights, read-only) is shared
-        pipe2 = GraphedEnhancer(model2, BATCH, L, dev, oracle=False)
+        pipe2 = GraphedEnhancer(model2, BATCH, L, dev, oracle=False, generator=noise_generator(k))
         pipe2.y_dev.copy_(y_dev)
         with torch.cuda.stream(pipe2.stream):
             pipe2._step()
@@ -407,6 +413,8 @@ def run_b200(args):
         clocks = ClockSampler(local) if rank == 0 else None
         # the three timed regions run back to back (no idle gaps between them): W warm-up steps above, then K steps each
         ms_dev = timed(lambda i: pipes[i % len(pipes)].replay())
+        # the enhanced batch of the last timed step; later regions overwrite the enhancers' output buffers
+        last_out = pipes[(args.steps - 1) % len(pipes)].out_dev.clone() if args.dump_outputs else None
         ms_single = timed(lambda i: pipes[0].replay()) if len(pipes) > 1 else ms_dev
 
         host_outs = [host_out] + [torch.empty_like(host_out).pin_memory() for _ in pipes[1:]]
@@ -525,6 +533,12 @@ def run_b200(args):
         except Exception as ex:                       # an extra must never take the headline down with it
             extras["error"] = f"{type(ex).__name__}: {str(ex)[:300]}"
 
+    if args.dump_outputs:
+        # inputs, weights and noise draws (seeded per enhancer) are identical from run to run for the same arguments
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, f"enhanced_rank{rank}.npy"), last_out.cpu().numpy())
+
     if rank == 0:
         cpu, eager = None, None
         if world == 1 and not args.no_cpu_baseline:
@@ -592,7 +606,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the sweep824 / longform60 / pc60 sub-records")
     ap.add_argument("--streams", type=int, default=2, choices=[1, 2, 3, 4],
                     help="independent enhancers per GPU whose steps alternate (2: small kernels of one batch overlap the other batch)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the enhanced waveforms [16, 64000] of the last timed step as DIR/enhanced_rank<R>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -17,8 +17,12 @@ import torch
 
 class GraphedEnhancer:
     def __init__(self, model, batch, length, device, oracle=False, noise_over_clean=None, noise=None, stream=None,
-                 ragged=False):
+                 ragged=False, generator=None):
         self.model, self.batch, self.length, self.device = model, batch, length, torch.device(device)
+        # generator: CUDA torch.Generator for this enhancer's noise draws.  Every graph that draws from torch's default
+        # generator reads its seed / offset from one shared device slot, which each replay rewrites, so enhancers whose
+        # replays overlap on different streams need a generator each for reproducible draws.
+        self.generator = generator
         self.stream = stream or torch.cuda.Stream(device=self.device)
         # separate streams for the two copy directions: on one in-order stream the upload of batch i+1 would queue
         # behind the read-back of batch i, i.e. behind the end of batch i's computation
@@ -29,7 +33,8 @@ class GraphedEnhancer:
         self.out_stage = torch.zeros_like(self.y_dev)
         if noise_over_clean is not None:   # device-resident before capture (no host copy inside the graph)
             noise_over_clean = torch.as_tensor(noise_over_clean, dtype=torch.float32).reshape(-1).to(self.device)
-        self._kw = dict(oracle=oracle, noise_over_clean=noise_over_clean, noise=noise)   # noise: fixed draw (tests)
+        self._kw = dict(oracle=oracle, noise_over_clean=noise_over_clean, noise=noise,   # noise: fixed draw (tests)
+                        generator=generator)
         # ragged: per-utterance valid lengths live in a device buffer read by the captured graph
         self.len_dev = torch.full((batch,), length, dtype=torch.int32, device=self.device) if ragged else None
         self.graph = None
@@ -50,6 +55,8 @@ class GraphedEnhancer:
                 self.out_dev = self._step()
             self.stream.synchronize()
             self.graph = torch.cuda.CUDAGraph()
+            if self.generator is not None:
+                self.graph.register_generator_state(self.generator)
             with torch.cuda.graph(self.graph, stream=self.stream):
                 self.out_dev = self._step()
         return self

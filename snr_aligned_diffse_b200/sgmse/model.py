@@ -215,12 +215,14 @@ class ScoreModel(CheckpointedModule):
         return dm.transform_code, float(dm.spec_abs_exponent), float(dm.spec_factor)
 
     # ------------------------------------------------------------------------------ enhancement
-    def enhance_batch(self, y, lengths=None, oracle=False, noise_over_clean=None, noise=None, return_aux=False):
+    def enhance_batch(self, y, lengths=None, oracle=False, noise_over_clean=None, noise=None, return_aux=False,
+                      generator=None):
         """sebridge_v3 / snr_conditioned='true' enhancement of a padded batch, entirely on the GPU.
 
         y: [B, Lmax] float32 (host or device); lengths: optional [B] valid sample counts;
         noise_over_clean: [B] noise_rms/clean_rms when oracle=True; noise: optional explicit complex
-        normal Z [B,1,256,Tpad].  Returns the enhanced batch [B, Lmax] on the GPU (zeros past each length).
+        normal Z [B,1,256,Tpad], otherwise drawn from `generator` (a CUDA torch.Generator; default: torch's
+        default CUDA generator).  Returns the enhanced batch [B, Lmax] on the GPU (zeros past each length).
         One pass = model.py:713-752,810-830 for every utterance, with no host synchronisation."""
         if not (self.snr_conditioned == 'true' and self.model_type == 'sebridge_v3'):
             raise NotImplementedError("enhance_batch implements the sebridge_v3 SNR-conditioned path")
@@ -241,7 +243,7 @@ class ScoreModel(CheckpointedModule):
             ratio = est.dnn.engine.noise_over_clean(g)                             # (:721)
         t, norm, idx = ops.v3_scalars(ratio, peak, self.fixed_snr)                # (:732-740)
         Y = ops.stft(yd, ld, scale=norm, scale_is_divisor=True, transform=tr, alpha=alpha, beta=beta)   # (:746-751)
-        Z = torch.randn_like(Y) if noise is None else noise.to("cuda").reshape(Y.shape).contiguous()
+        Z = torch.randn_like(Y, generator=generator) if noise is None else noise.to("cuda").reshape(Y.shape).contiguous()
         X_T = axpby(y=Y, b=1.0, z=Z, d=t * float(self.sigma_max))                 # (:822-823)
         sample = self.dnn.engine.forward(X_T, Y, t, mode=MODE_SEBRIDGE)           # (:824, 537-541)
         x_hat = ops.istft(sample, L, ld, scale=norm, transform=tr, alpha=alpha, beta=beta)   # (:828-830)

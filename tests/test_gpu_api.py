@@ -216,6 +216,43 @@ def test_graphed_enhancer_pipeline_matches_eager(v3):
         assert torch.equal(o, ref)
 
 
+def test_graphed_enhancers_with_own_generators_are_reproducible_when_replays_overlap(v3, sd):
+    """Two GraphedEnhancers drawing their noise from their own generators, replayed alternately on their two streams (as
+    bench.py runs them): every replay draws fresh noise, and each enhancer returns exactly what an enhancer with an
+    equally seeded generator returns when it is replayed alone."""
+    from snr_aligned_diffse_b200.pipeline import GraphedEnhancer
+    from snr_aligned_diffse_b200.sgmse.model import ScoreModel
+    B, L, n = 2, 8100, 3
+    y = (torch.randn(B, L, generator=torch.Generator().manual_seed(23)) * 0.05).cuda()
+    # a second model: enhancers whose replays overlap need their own network workspace
+    models = (v3, ScoreModel.from_state_dict(sd, backbone="ncsnpp", sde="ouve", model_type="sebridge_v3",
+                                             snr_conditioned="true", fixed_snr=0.17783, theta=1.5, sigma_min=0.05,
+                                             sigma_max=1.0, base_dir="").eval(no_ema=True))
+
+    def make(k):
+        p = GraphedEnhancer(models[k], B, L, "cuda", oracle=True, noise_over_clean=[0.4, 0.2],
+                            generator=torch.Generator(device="cuda").manual_seed(k + 1))
+        p.y_dev.copy_(y)
+        torch.cuda.synchronize()
+        return p.capture()
+
+    def replays(pipes, count):
+        outs = [[] for _ in pipes]
+        for i in range(count * len(pipes)):
+            p = pipes[i % len(pipes)]
+            with torch.cuda.stream(p.stream):
+                outs[i % len(pipes)].append(p.replay().clone())
+        torch.cuda.synchronize()
+        return outs
+
+    overlapped = replays([make(0), make(1)], n)
+    alone = [replays([make(k)], n)[0] for k in (0, 1)]
+    for k in range(2):
+        assert all(torch.equal(a, b) for a, b in zip(overlapped[k], alone[k])), k
+        assert not torch.equal(overlapped[k][0], overlapped[k][1]) and torch.isfinite(overlapped[k][0]).all()
+    assert not torch.equal(overlapped[0][0], overlapped[1][0])
+
+
 def test_snr_sweep_batch_equals_per_snr_calls(v3):
     """deep_eval.py's nine-SNR loop as one batch == nine separate enhance() calls (same noise draws), bit for bit."""
     g = torch.Generator().manual_seed(31)
