@@ -112,13 +112,8 @@ int snrse_ncsnpp_param_info(void* handle, int i, char* name, int name_cap, int* 
 int snrse_ncsnpp_param_shape(void* handle, int i, int64_t* dims, int* ndim); /* shape of the state-dict tensor */
 int snrse_ncsnpp_set_weights(void* handle, const void* device_blob);
 /* Plan for inputs [B][F][T]: returns the workspace size (or -1).  flags bit0: keep all activations
- * (debug taps); bit1: CUDA-core cross-check convolutions instead of tcgen05; bit2: single-CTA tcgen05 GEMM kernel only;
- * bit3: unused; bit4: GroupNorm+SiLU as a separate pass (no in-kernel fusion);
- * bit5: GroupNorm+SiLU of the up / down blocks inside single-output FIR kernels (two FIR launches per block);
- * bit6: up / down blocks as a GroupNorm pass + two FIR passes (default: ONE dual-output FIR launch over x writing
- * FIR(silu(GroupNorm(x))) and FIR(x) from shared-memory staged rows); bit7: GroupNorm scale/shift of the normalising
- * convolutions derived inside the convolution kernel from the statistics (default: one gn_finalize launch per
- * normalisation).  Bits 5-7 select measured alternatives (profiles/r02_step_ab.md); all give identical bits. */
+ * (debug taps, snrse_ncsnpp_read_tap); bit1: fp32 CUDA-core cross-check path (convolutions, attention and input packing
+ * instead of tcgen05 / bf16 operands).  Any other bit is rejected (-1). */
 int64_t snrse_ncsnpp_plan_bytes(void* handle, int B, int F, int T, int flags);
 int snrse_ncsnpp_plan_bind(void* handle, int B, int F, int T, void* workspace, int64_t bytes);
 /* x (state), y (noisy), out: complex64 [B][F][T]; t [B] f32.  mode 0: dnn(cat[x,y], t);

@@ -1,8 +1,9 @@
 /* snrse_b200_debug.h -- measurement and debugging entry points of libsnrse_b200.so.
  *
  * NOT part of the drop-in ABI (snrse_b200.h): nothing in the product path calls these.  They exist for bench.py's
- * roofline record (per-launch-group CUDA-event timing), the parity tests (per-module activation taps) and the
- * kernel-tuning tools under tools/ (cycle counters of the convolution kernels).  Same conventions as snrse_b200.h.
+ * roofline record (per-launch-group CUDA-event timing), the parity tests (per-module activation taps, the executor's
+ * dual-output FIR pass as an operator) and the kernel-tuning tools under tools/ (cycle counters of the convolution
+ * kernels).  Same conventions as snrse_b200.h.
  */
 #ifndef SNRSE_B200_DEBUG_H
 #define SNRSE_B200_DEBUG_H
@@ -27,11 +28,11 @@ int snrse_ncsnpp_read_tap(void* handle, int B, int F, int T, int module_idx, flo
 /* cycle counters of the convolution kernels: [grid][8] int64 (a / b / accumulator waits of the MMA warp, total,
  * epilogue wait / body, producer waits), filled by every later launch; NULL switches them off */
 void snrse_conv_halo_set_debug(long long* dev_counters);
-/* measurement switches of the 2-CTA convolution kernel.  bit0: L2 prefetch of the next tile's operand and residual boxes
- * (default 0: measured +0.1 ms per step); bit1: two A slots + double-buffered staging on the GroupNorm-in-flight layers;
- * bit2: 4 KB smaller shared-memory budget; bit3: the 1x1 shortcut operand of the 128-channel layers shares the halo ring
- * (the r02 schedule before the separate shortcut ring; different K order, so not bit-identical).  See profiles/r02_step_ab.md. */
-void snrse_conv_halo_set_prefetch(int on);
+/* the dual-output FIR pass of the up / down residual blocks as one operator (NHWC bf16, x [B][H][W][C]):
+ * out_n = FIR(silu(GroupNorm(32, eps)(x))), out_r = FIR(x), both [B][2H][2W][C] (up) or [B][H/2][W/2][C] (down);
+ * workspace: the size snrse_groupnorm_workspace_bytes gives for B, as for snrse_gn_silu_fir_nhwc */
+int snrse_fir_dual_nhwc(const void* x, const float* gamma, const float* beta, float eps, void* out_n, void* out_r, int B,
+                        int H, int W, int C, int up, void* workspace, void* stream);
 
 #ifdef __cplusplus
 }

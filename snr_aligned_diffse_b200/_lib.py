@@ -50,7 +50,7 @@ PROTOTYPES = {
     "snrse_ncsnpp_read_tap": (i32, [vp, i32, i32, i32, i32, vp, i64, POINTER(i64), vp]),
     "snrse_conv_nhwc": (i32, [vp, i32, i32, vp, i32, vp, i32, vp, vp, i32, vp, f32, vp, i32, i32, i32, i32, vp]),
     "snrse_conv_halo_set_debug": (None, [vp]),
-    "snrse_conv_halo_set_prefetch": (None, [i32]),
+    "snrse_fir_dual_nhwc": (i32, [vp, vp, vp, f32, vp, vp, i32, i32, i32, i32, i32, vp, vp]),
     "snrse_gn_silu_conv3x3_nhwc": (i32, [vp, i32, vp, vp, f32, vp, i32, vp, i32, vp, vp, i32, vp, f32, vp, i32, i32, i32, vp, vp]),
     "snrse_conv3x3_nhwc_stats": (i32, [vp, i32, vp, i32, vp, i32, vp, vp, i32, vp, f32, vp, i32, i32, i32, vp, vp]),
     "snrse_groupnorm_workspace_bytes": (i64, [i32]),

@@ -253,6 +253,19 @@ int snrse_attention_nhwc(const void* q, const void* k, const void* v, void* scor
 long long* g_halo_dbg_shared = nullptr;
 // device buffer of [grid][8] cycle counters filled by subsequent conv_halo2 / conv_gemm launches (null: off)
 extern "C" void snrse_conv_halo_set_debug(long long* dev_counters) { g_halo_dbg_shared = dev_counters; }
-// L2 prefetch of the next tile's boxes in the 2-CTA convolution kernel: 1 (default) on, 0 off (A/B measurements)
-extern int g_halo2_prefetch;
-extern "C" void snrse_conv_halo_set_prefetch(int on) { g_halo2_prefetch = on; }
+
+// The dual-output FIR pass of the NCSN++ up / down residual blocks on its own: out_n = FIR(silu(GroupNorm(x))),
+// out_r = FIR(x).  workspace: snrse_groupnorm_workspace_bytes(B).
+extern "C" int snrse_fir_dual_nhwc(const void* x, const float* gamma, const float* beta, float eps, void* out_n, void* out_r,
+                                   int B, int H, int W, int C, int up, void* workspace, void* stream) {
+    SNRSE_CHECK_ARG(x && gamma && beta && out_n && out_r && workspace, "fir_dual: null pointer");
+    const ActView vx = mk_view(x, B, H, W, C, C);
+    const int oh = up ? 2 * H : H / 2, ow = up ? 2 * W : W / 2;
+    const ActView vn = mk_view(out_n, B, oh, ow, C, C), vr = mk_view(out_r, B, oh, ow, C, C);
+    unsigned long long* ust = static_cast<unsigned long long*>(workspace);
+    float* scsh = reinterpret_cast<float*>(ust + (int64_t)B * 128 * 2);
+    SNRSE_CUDA(cudaMemsetAsync(ust, 0, (size_t)B * (C / 4) * 16, S(stream)));
+    SNRSE_TRY(gn_stats_launch(&vx, ust, S(stream)));
+    SNRSE_TRY(gn_finalize_launch(ust, C / 4, nullptr, 0, B, (int64_t)H * W * (C / 32), gamma, beta, eps, scsh, S(stream)));
+    return fir_dual_launch(&vx, &vn, &vr, up, scsh, S(stream));
+}

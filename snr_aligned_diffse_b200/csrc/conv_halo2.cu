@@ -37,11 +37,6 @@
 #include "ptx.cuh"
 #include "tma_host.h"
 
-// Measurement switches (snrse_conv_halo_set_prefetch, include/snrse_b200_debug.h).  bit0: L2 prefetch of the next tile's
-// boxes -- measured on the graphed step, interleaved: 20.05 ms with, 19.95 ms without (profiles/r02_step_ab.md), so OFF;
-// bit1 / bit2: ring-depth variants of the GroupNorm layers; bit3: shared ring for the shortcut operand (the r02 schedule).
-int g_halo2_prefetch = 0;
-
 namespace {
 
 constexpr int HALO_THREADS = 384;        // + 256 (warps 12..19) when GroupNorm+SiLU is applied to the operand in flight
@@ -67,14 +62,11 @@ struct Halo2Args {
     int acc_bufs;                  // 1 or 2 TMEM accumulator sets
     int stg_bufs;                  // 1 or 2 staging tiles per epilogue warp
     int has_res;
-    int prefetch;                  // L2 prefetch of the next tile's operand / residual boxes (0: off, for A/B measurements)
     float4* out4;                  // N == 16 only: fp32 4-channel output [B,H,W,4] = acc[:, 0:4] + bias (+ addend4)
     const float4* addend4;
     unsigned long long* ustats;    // null, or GroupNorm sums of the result, accumulated: [B][N/4][2] fixed point (gn_fixed.cuh)
     const float* scsh;             // null, or GroupNorm scale/shift [B][2][norm_c] applied (+SiLU) to operand 0 in shared memory
     int norm_c;
-    GnSrc gn;                      // has_gn: scale/shift derived in the kernel from these statistics instead of read from scsh
-    int has_gn;
     const float* bias;
     const float* tbias;
     int tb_stride;
@@ -164,7 +156,7 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
     const uint32_t a_tx = (uint32_t)(SUB_ROWS * g.sub + 2) * HALO_W * ROW_B;            // bytes one halo TMA box delivers
     const uint32_t a1_tx = (uint32_t)(SUB_ROWS * g.sub) * TW * ROW_B;                   // shortcut operand: no halo
     const uint32_t b_bytes = (uint32_t)(g.N / 2) * ROW_B;   // this CTA's half of the weight tile
-    // shared-memory map: halo ring | shortcut ring | weight ring | epilogue staging | per-warp additive terms | GroupNorm table
+    // shared-memory map: halo ring | shortcut ring | weight ring | epilogue staging | per-warp additive terms
     const uint32_t a_base = smem_base, sc_base = a_base + (uint32_t)g.na * a_bytes;
     const uint32_t sc_bytes = a1_tx;                        // 16 KB per sub-tile: a multiple of the 1 KB swizzle atom
     const uint32_t b_base = sc_base + (uint32_t)g.nsc * sc_bytes;
@@ -172,10 +164,9 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
     const int n_astage = g.c0_chunks + g.c1_chunks;   // halo tiles consumed per super-tile
     const uint32_t acc_cols = (uint32_t)(g.sub * g.N);
     const uint32_t tmem_cols = acc_cols * (uint32_t)g.acc_bufs;  // 128/256/512: power of two
-    const bool norm_on = g.scsh != nullptr || g.has_gn;          // GroupNorm + SiLU applied to operand 0 in flight
+    const bool norm_on = g.scsh != nullptr;                      // GroupNorm + SiLU applied to operand 0 in flight
     // per epilogue warp: (bias + time-embedding bias) * scale for its N/2 columns
     const uint32_t bs_base = stg_base + (uint32_t)(EPI_WARPS * g.stg_bufs) * 4096u;
-    const uint32_t gn_tab = bs_base + halo_bsum_bytes(g.N);   // has_gn: scale[512] | shift[512] floats
 
     if (warp == W_MMA1) {
         if (lane == 0) {
@@ -281,22 +272,9 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
             const int tile = 2 * ct + (int)rank;
             const int b = tile / tiles_per_img, rem = tile % tiles_per_img;   // tile == n_tiles -> b == B: zero fill
             const int h0 = (rem / g.tiles_w) * SUB_ROWS * g.sub, w0 = (rem % g.tiles_w) * TW;
-            // optional (off by default, see g_halo2_prefetch): the boxes of the tile this CTA walks next are prefetched into
-            // L2 one whole tile ahead.  The MMA warp of the fused-shortcut layers waits on A 41 % of its time
-            // (profiles/r02_conv_ncu.md), but the prefetch does not change that: the limit is the bytes the two- or
-            // three-stage ring can keep in flight against 512-clk shortcut stages, not the DRAM latency.
-            const int ctn = ct + n_clusters;
-            const int tile_n = 2 * ctn + (int)rank;
-            const int bn = tile_n / tiles_per_img, remn = tile_n % tiles_per_img;
-            const int h0n = (remn / g.tiles_w) * SUB_ROWS * g.sub, w0n = (remn % g.tiles_w) * TW;
-            const bool pf = g.prefetch && ctn < n_ctiles && bn < g.B;
             for (int j = 0; j < n_astage; ++j) {
                 const bool seg0 = !(g.seq[j] & 0x80);
                 const int chunk = g.seq[j] & 0x7f;
-                if (pf && elected) {
-                    if (seg0) ptx::tma_prefetch_4d(&mapA0, chunk * 64, w0n - 1, h0n - 1, bn);
-                    else ptx::tma_prefetch_4d(&mapA1, chunk * 64, w0n, h0n, bn);
-                }
                 if (g.dbg) t0__ = clock64();
                 ptx::mbar_wait(ptx::smem_u32(&a_empty[s]), ph ^ 1u);
                 DBG_ADD(w_a);
@@ -428,8 +406,6 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
         // the image stay zero (the convolution pads the NORMALISED activation).  Same arithmetic as gn_apply_kernel.
         if (norm_on) {
             const int tid = (warp - NORM_WARP0) * 32 + lane;
-            float* tab = reinterpret_cast<float*>(smem_raw + (gn_tab - ptx::smem_u32(smem_raw)));
-            int tab_b = -1;                                       // image whose scale / shift the table holds
             const uint32_t q = (uint32_t)(tid & 7);
             const int rg = tid >> 3;
             const int rows_total = (SUB_ROWS * g.sub + 2) * HALO_W;
@@ -441,34 +417,6 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
                 const int tile = 2 * ct + (int)rank;
                 const int b = tile / tiles_per_img, rem = tile % tiles_per_img;
                 const int h0 = (rem / g.tiles_w) * SUB_ROWS * g.sub, w0 = (rem % g.tiles_w) * TW;
-                if (g.has_gn && b < g.B && b != tab_b) {
-                    // In-kernel finalize (replaces a gn_finalize launch per normalised convolution): per-channel scale /
-                    // shift of image b from the fixed-point unit sums, same arithmetic as gn_finalize_kernel.  A cluster
-                    // walks consecutive tiles, so this runs once or twice per CTA.
-                    asm volatile("bar.sync 1, 256;" ::: "memory");   // everyone holds the previous image's values in registers
-                    const int C = g.norm_c, cpg = C >> 5, upg = cpg >> 2;
-                    for (int c = tid; c < C; c += NORM_THREADS) {
-                        const int grp = c / cpg;
-                        long long sm = 0;
-                        double q = 0.0;
-                        for (int k = 0; k < upg; ++k) {
-                            const int u = grp * upg + k;
-                            const unsigned long long* p = u < g.gn.U0 ? g.gn.st0 + ((int64_t)b * g.gn.U0 + u) * 2
-                                                                       : g.gn.st1 + ((int64_t)b * g.gn.U1 + (u - g.gn.U0)) * 2;
-                            sm += (long long)__ldg(p);
-                            q += gn_unfix_sq(__ldg(p + 1));
-                        }
-                        const double mean = gn_unfix_sum(sm) * g.gn.inv_count;
-                        double var = q * g.gn.inv_count - mean * mean;
-                        if (var < 0.0) var = 0.0;
-                        const float mean_f = (float)mean, rstd = (float)(1.0 / sqrt(var + (double)g.gn.eps));
-                        const float scv = rstd * __ldg(g.gn.gamma + c);
-                        tab[c] = scv;
-                        tab[512 + c] = __ldg(g.gn.beta + c) - mean_f * scv;
-                    }
-                    asm volatile("bar.sync 1, 256;" ::: "memory");
-                    tab_b = b;
-                }
                 for (int j = 0; j < n_astage; ++j) {
                     if ((g.seq[j] & 0x80) && g.nsc > 0) continue;        // shortcut tiles bypass the halo ring
                     const bool live = (b < g.B) && !(g.seq[j] & 0x80);   // the 1x1 shortcut operand is used raw
@@ -476,16 +424,9 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
                     // h = x * (scale/2) + shift/2  ==  (x*scale + shift)/2 exactly;  silu(t) = h + h*tanh(h)  (silu_f)
                     float sc[8], sh[8];
                     if (live) {
-                        float4 a0, a1, c0, c1;
-                        if (g.has_gn) {
-                            const float4* pa = reinterpret_cast<const float4*>(tab + chunk * 64 + q * 8);
-                            const float4* pc = reinterpret_cast<const float4*>(tab + 512 + chunk * 64 + q * 8);
-                            a0 = pa[0]; a1 = pa[1]; c0 = pc[0]; c1 = pc[1];
-                        } else {
-                            const float4* pa = reinterpret_cast<const float4*>(g.scsh + ((int64_t)b * 2) * g.norm_c + chunk * 64 + q * 8);
-                            const float4* pc = reinterpret_cast<const float4*>(g.scsh + ((int64_t)b * 2 + 1) * g.norm_c + chunk * 64 + q * 8);
-                            a0 = __ldg(pa); a1 = __ldg(pa + 1); c0 = __ldg(pc); c1 = __ldg(pc + 1);
-                        }
+                        const float4* pa = reinterpret_cast<const float4*>(g.scsh + ((int64_t)b * 2) * g.norm_c + chunk * 64 + q * 8);
+                        const float4* pc = reinterpret_cast<const float4*>(g.scsh + ((int64_t)b * 2 + 1) * g.norm_c + chunk * 64 + q * 8);
+                        const float4 a0 = __ldg(pa), a1 = __ldg(pa + 1), c0 = __ldg(pc), c1 = __ldg(pc + 1);
                         sc[0] = a0.x; sc[1] = a0.y; sc[2] = a0.z; sc[3] = a0.w; sc[4] = a1.x; sc[5] = a1.y; sc[6] = a1.z; sc[7] = a1.w;
                         sh[0] = c0.x; sh[1] = c0.y; sh[2] = c0.z; sh[3] = c0.w; sh[4] = c1.x; sh[5] = c1.y; sh[6] = c1.z; sh[7] = c1.w;
 #pragma unroll
@@ -610,17 +551,6 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
                 }
                 __syncwarp();
             }
-            if (g.has_res && g.prefetch && elected) {   // this warp's residual boxes of the NEXT tile -> L2
-                const int ctn = ct + n_clusters;
-                const int tile_n = 2 * ctn + (int)rank;
-                const int bn = tile_n / tiles_per_img, remn = tile_n % tiles_per_img;
-                if (ctn < n_ctiles && bn < g.B) {
-                    const int h0n = (remn / g.tiles_w) * SUB_ROWS * g.sub, w0n = (remn % g.tiles_w) * TW;
-                    for (int u = 0; u < g.sub; ++u)
-                        for (int p = 0; p < n_pass; ++p)
-                            ptx::tma_prefetch_4d(&mapRes, n_off + half * half_cols + 64 * p, w0n, h0n + SUB_ROWS * u + 4 * quarter, bn);
-                }
-            }
             if (g.dbg) t0__ = clock64();
             ptx::mbar_wait(ptx::smem_u32(&acc_full[buf]), use & 1u);
             DBG_ADD(w_full);
@@ -735,7 +665,6 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
 int g_num_sms2 = 0;
 }  // namespace
 extern long long* g_halo_dbg_shared;
-extern int g_halo2_prefetch;   // measurement switch (snrse_conv_halo_set_prefetch, include/snrse_b200_debug.h)
 
 bool conv_halo2_eligible(const ActView* a0, int taps0, int n_rows) {
     return taps0 == 9 && a0->W >= TW && a0->H >= 8 && (n_rows == 128 || n_rows == 256);
@@ -743,12 +672,8 @@ bool conv_halo2_eligible(const ActView* a0, int taps0, int n_rows) {
 
 int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, const bf16* wt, int n_rows,
                          const float* bias, const float* tbias, int tb_stride, const ActView* res, float scale, bf16* out,
-                         int out_ld, const float* scsh, unsigned long long* ustats, const GnSrc* gn) {
+                         int out_ld, const float* scsh, unsigned long long* ustats) {
     SNRSE_CHECK_ARG(conv_halo2_eligible(a0, 9, n_rows), "conv_halo2: shape not eligible");
-    SNRSE_CHECK_ARG(!(scsh && gn), "conv_halo2: give either a scale/shift table or the statistics, not both");
-    SNRSE_CHECK_ARG(!gn || (a0->C <= 512 && gn->st0 && gn->gamma && gn->beta && 4 * (gn->U0 + gn->U1) == a0->C),
-                    "conv_halo2: bad GroupNorm statistics source");
-    const bool norm = scsh || gn;
     SNRSE_CHECK_ARG(a0->C % 64 == 0 && a0->ld % 8 == 0, "conv_halo2: Cin must be a multiple of 64");
     SNRSE_CHECK_ARG(!a1 || (a1->C % 64 == 0 && a1->ld % 8 == 0 && a1->H == a0->H && a1->W == a0->W && a1->B == a0->B),
                     "conv_halo2: bad shortcut operand");
@@ -780,13 +705,13 @@ int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, 
     p->N = n_loc;
     p->acc_bufs = (sub * n_loc <= 256) ? 2 : 1;
     const int a_bytes = (int)halo_stage_bytes(sub), b_bytes = (n_loc / 2) * 128;
-    // dynamic shared memory (static: barriers + per-warp bias slices, ~4.3 KB); the in-kernel GroupNorm table takes 4 KB
-    const int budget = 220 * 1024 - ((gn || (g_halo2_prefetch & 4)) ? 4096 : 0);   // bit2: A/B measurement of the smaller budget alone
+    // dynamic shared memory (static: barriers + per-warp bias slices, ~4.3 KB)
+    const int budget = 220 * 1024;
     // One A slot feeds 9 taps x SUB x 4 MMAs (>= 2300 clk): two slots hide the next tile's load.  With in-flight
     // normalisation the slot also waits for the normalising warps (load + ~2500 clk); at N=128 (64-clock MMAs) that
     // needs a third slot, paid for with single-buffered epilogue staging.
     int na = 2, stg = 2, nsc = 0;
-    if (norm && n_loc == 128 && sub == 2 && !(g_halo2_prefetch & 2)) { na = 3; stg = 1; }   // bit1: A/B measurement of na=2 / stg=2
+    if (scsh && n_loc == 128 && sub == 2) { na = 3; stg = 1; }
     int nb = (budget - na * a_bytes - stg * EPI_WARPS * 4096) / b_bytes;
     if (nb < 6 && stg == 2) {
         stg = 1;
@@ -802,22 +727,21 @@ int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, 
     // Only for the 128-output-channel layers (where N = 128 whatever the batch): the K order then depends on the layer alone,
     // never on the batch-dependent tiling, so results stay batch-invariant bit for bit.  The 256-channel layers keep the
     // shared ring: at N = 256 / SUB = 2 two extra slots leave room for only two weight slots.
-    if (a1 && n_rows == 128 && !(g_halo2_prefetch & 8)) {   // bit3: A/B measurement of the shared ring
+    if (a1 && n_rows == 128) {
         const int sc_bytes = SUB_ROWS * sub * TW * 128;
-        const int limit = 227 * 1024 - 1024 /*alignment*/ - 768 /*static: barriers*/ - (int)halo_bsum_bytes(n_loc) - (gn ? 4096 : 0);
+        const int limit = 227 * 1024 - 1024 /*alignment*/ - 768 /*static: barriers*/ - (int)halo_bsum_bytes(n_loc);
         const int nb2 = (limit - 2 * a_bytes - MAX_SC * sc_bytes - EPI_WARPS * 4096) / b_bytes;
         if (nb2 >= 4) { na = 2; nsc = MAX_SC; stg = 1; nb = nb2 > MAX_B ? MAX_B : nb2; }
     }
     p->na = na; p->nb = nb; p->stg_bufs = stg; p->nsc = nsc;
     p->smem_bytes = na * a_bytes + nsc * SUB_ROWS * sub * TW * 128 + nb * b_bytes + stg * EPI_WARPS * 4096 +
-                    (int)halo_bsum_bytes(n_loc) + (gn ? 4096 : 0) + 1024;
+                    (int)halo_bsum_bytes(n_loc) + 1024;
     const int n_ctiles = (p->n_tiles + 1) / 2, max_clusters = g_num_sms2 / 2;
     p->grid = nsplit == 2 ? 4 * n_ctiles : 2 * (n_ctiles < max_clusters ? n_ctiles : max_clusters);
     p->bias = bias; p->tbias = tbias; p->tb_stride = tb_stride;
     p->res = res ? res->ptr : nullptr; p->res_ld = res ? res->ld : 0;
     p->scale = scale; p->out = out; p->out_ld = out_ld;
     p->scsh = scsh;
-    if (gn) { p->gn = *gn; p->has_gn = 1; }
     p->ustats = ustats;
     const int box_h = SUB_ROWS * sub + 2;
     SNRSE_TRY(tma_make_act_map(&p->mapA0, a0->ptr, a0->C, a0->W, a0->H, a0->B, a0->ld, 64, HALO_W, box_h));
@@ -835,11 +759,8 @@ int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, 
 // Thin output convolution on the same kernel: 3x3, C -> 4 (weights packed as 16 rows, rows 4..15 zero), optional
 // GroupNorm+SiLU of the operand in flight, fp32 output [B,H,W,4] = conv + bias (+ addend4).
 int conv_halo2_make_plan_out4(ConvHaloPlan* p, const ActView* a0, const bf16* wt16, const float* bias4, const float* addend4,
-                              float* out4, const float* scsh, const GnSrc* gn) {
+                              float* out4, const float* scsh) {
     SNRSE_CHECK_ARG(a0->W >= TW && a0->H >= 8 && a0->C % 64 == 0 && a0->ld % 8 == 0, "conv_halo2 out4: shape not eligible");
-    SNRSE_CHECK_ARG(!(scsh && gn), "conv_halo2 out4: give either a scale/shift table or the statistics, not both");
-    SNRSE_CHECK_ARG(!gn || (a0->C <= 512 && gn->st0 && gn->gamma && gn->beta && 4 * (gn->U0 + gn->U1) == a0->C),
-                    "conv_halo2 out4: bad GroupNorm statistics source");
     SNRSE_CHECK_ARG(bias4 && out4, "conv_halo2 out4: null pointer");
     if (g_num_sms2 == 0) {
         int dev = 0;
@@ -863,12 +784,11 @@ int conv_halo2_make_plan_out4(ConvHaloPlan* p, const ActView* a0, const bf16* wt
     p->acc_bufs = 2;
     const int a_bytes = (int)halo_stage_bytes(sub);
     p->na = 3; p->nb = MAX_B; p->stg_bufs = 0;   // no epilogue staging: the result leaves from registers
-    p->smem_bytes = p->na * a_bytes + p->nb * 1024 + (int)halo_bsum_bytes(16) + (gn ? 4096 : 0) + 1024;
+    p->smem_bytes = p->na * a_bytes + p->nb * 1024 + (int)halo_bsum_bytes(16) + 1024;
     const int n_ctiles = (p->n_tiles + 1) / 2, max_clusters = g_num_sms2 / 2;
     p->grid = 2 * (n_ctiles < max_clusters ? n_ctiles : max_clusters);
     p->bias = bias4; p->scale = 1.0f;
     p->scsh = scsh;
-    if (gn) { p->gn = *gn; p->has_gn = 1; }
     p->out4 = out4; p->addend4 = addend4;
     SNRSE_TRY(tma_make_act_map(&p->mapA0, a0->ptr, a0->C, a0->W, a0->H, a0->B, a0->ld, 64, HALO_W, SUB_ROWS * sub + 2));
     p->mapA1 = p->mapA0; p->mapOut = p->mapA0; p->mapRes = p->mapA0;
@@ -912,15 +832,13 @@ int conv_halo2_launch(const ConvHaloPlan* p, cudaStream_t s) {
     g.sub = p->sub; g.tiles_h = p->tiles_h; g.tiles_w = p->tiles_w; g.n_tiles = p->n_tiles;
     g.N = p->N; g.nsplit = p->nsplit; g.n_total = p->n_total; g.na = p->na; g.nb = p->nb; g.nsc = p->nsc; g.acc_bufs = p->acc_bufs; g.stg_bufs = p->stg_bufs;
     g.has_res = p->res != nullptr;
-    g.prefetch = g_halo2_prefetch & 1;
     g.bias = p->bias; g.tbias = p->tbias; g.tb_stride = p->tb_stride;
     g.scale = p->scale;
     g.scsh = p->scsh; g.norm_c = p->c0_chunks * 64;
-    g.gn = p->gn; g.has_gn = p->has_gn;
     g.ustats = p->ustats;
     g.out4 = reinterpret_cast<float4*>(p->out4); g.addend4 = reinterpret_cast<const float4*>(p->addend4);
     g.dbg = g_halo_dbg_shared;
-    snrse_launch_m(2, conv_halo2_kernel, dim3(p->grid), dim3(HALO_THREADS + ((p->scsh || p->has_gn) ? NORM_THREADS : 0)), p->smem_bytes, s, p->mapA0, p->mapA1, p->mapB, p->mapOut, p->mapRes, g);
+    snrse_launch_m(2, conv_halo2_kernel, dim3(p->grid), dim3(HALO_THREADS + (p->scsh ? NORM_THREADS : 0)), p->smem_bytes, s, p->mapA0, p->mapA1, p->mapB, p->mapOut, p->mapRes, g);
     SNRSE_LAUNCH_CHECK();
     return SNRSE_OK;
 }

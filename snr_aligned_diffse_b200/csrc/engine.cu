@@ -332,22 +332,12 @@ const float INV_SQRT2 = 0.70710678118654752440f;
 constexpr int MAX_STAT_ENTRIES = 192;   // tensors with GroupNorm statistics per forward (NCSN++ default: ~110)
 enum { LK_OTHER = 0, LK_GEMM = 1, LK_GN = 2, LK_FIR = 3, LK_ATTN = 4, LK_THIN = 5, LK_HEAD = 6 };
 
-// GroupNorm of a convolution operand, resolved inside the 2-CTA kernel (no gn_finalize launch): statistics entries of the
-// tensor (or of the two halves of a concatenation), units per source, elements per group, affine parameters
-struct GnRef {
-    int s0 = -1, s1 = -1, u0 = 0, u1 = 0;
-    int64_t cnt = 0, g_off = 0, b_off = 0;
-};
-
 int rec_gemm(Plan& P, int a0, int taps0, int a1, int64_t w_off, int n_rows, int64_t bias_off, int tb_row, int res,
-             float scale, int out, int norm = 0, int want_stats = 0, int algo_cin = 0, const GnRef* gnref = nullptr) {
-    const bool has_gn = gnref != nullptr;
-    GnRef gr;
-    if (has_gn) gr = *gnref;
+             float scale, int out, int norm = 0, int want_stats = 0, int algo_cin = 0) {
     // algo_cin > 0: channel count the ALGORITHM contracts over when the operand is a zero-padded copy (the 4-channel
     // network input enters as a 64-channel hi/lo tile): FLOPs and bytes are booked at algo_cin, not at the padded width
     P.use(a0);
-    if (norm && !has_gn) P.use(P.t_scsh);
+    if (norm) P.use(P.t_scsh);
     int st = -1;
     if (want_stats) {   // the epilogue also accumulates the GroupNorm sums of `out`
         st = P.n_stat_entries++;
@@ -387,21 +377,11 @@ int rec_gemm(Plan& P, int a0, int taps0, int a1, int64_t w_off, int n_rows, int6
         const double kt = (double)taps0 * c0 + (a1 >= 0 ? va1.C : 0);
         // algorithmic bytes: each operand / result once (bf16), weights once
         const double by = 2.0 * (px * (c0 + (a1 >= 0 ? va1.C : 0) + n_rows + (res >= 0 ? n_rows : 0)) + kt * n_rows);
-        if (!(p.flags & 4) && conv_halo2_eligible(&va0, taps0, n_rows)) {   // 2-CTA (cta_group::2) halo kernel
+        if (conv_halo2_eligible(&va0, taps0, n_rows)) {   // 2-CTA (cta_group::2) halo kernel
             ConvHaloPlan hp;
-            GnSrc src{};
-            if (has_gn) {
-                src.st0 = p.stat_ptr(gr.s0);
-                src.st1 = gr.s1 >= 0 ? p.stat_ptr(gr.s1) : nullptr;
-                src.U0 = gr.u0; src.U1 = gr.u1;
-                src.inv_count = 1.0 / (double)gr.cnt;
-                src.gamma = e.wf(gr.g_off); src.beta = e.wf(gr.b_off);
-                src.eps = 1e-6f;
-            }
             SNRSE_TRY(conv_halo2_make_plan(&hp, &va0, a1 >= 0 ? &va1 : nullptr, e.wb(w_off), n_rows, bias, tb, tb_stride,
                                            res >= 0 ? &vres : nullptr, scale, vout.ptr, vout.ld,
-                                           (norm && !has_gn) ? p.fptr(p.t_scsh) : nullptr, st >= 0 ? p.stat_ptr(st) : nullptr,
-                                           (norm && has_gn) ? &src : nullptr));
+                                           norm ? p.fptr(p.t_scsh) : nullptr, st >= 0 ? p.stat_ptr(st) : nullptr));
             p.add(LK_GEMM, 2.0 * px * n_rows * kt, by, [hp](cudaStream_t s) { return conv_halo2_launch(&hp, s); });
             return SNRSE_OK;
         }
@@ -469,36 +449,6 @@ void rec_gn_finalize(Plan& P, int x, int64_t g_off, int64_t b_off) {
     });
 }
 
-// GroupNorm feeding a convolution on the 2-CTA kernel.  Default: a gn_finalize launch writes the scale / shift table into
-// t_scsh (returns false).  Flag bit7: the kernel derives scale / shift from the statistics itself (returns true and fills
-// `ref`; nothing is launched here beyond a stand-alone statistics pass where the tensor's writer did not emit them).
-// Measured on the graphed 16 x 4 s step, variants interleaved (tools/step_ab.py, profiles/r02_step_ab.md): 77 launches
-// fewer but +0.2 ms per step -- the table costs the weight ring a slot and stalls the normalising warps at every image
-// change, and under the power cap the saved launch gaps buy nothing -- so the launches stay the default.
-bool rec_gn_for_conv(Plan& P, int x, int64_t g_off, int64_t b_off, GnRef* ref) {
-    if (!(P.flags & 128)) {
-        rec_gn_finalize(P, x, g_off, b_off);
-        return false;
-    }
-    GnRef r;
-    auto cc = P.cat_children.find(x);
-    if (cc != P.cat_children.end()) {
-        r.s0 = get_stats(P, cc->second.first);
-        r.s1 = get_stats(P, cc->second.second);
-        r.u0 = P.tens[cc->second.first].C / 4;
-        r.u1 = P.tens[cc->second.second].C / 4;
-    } else {
-        r.s0 = get_stats(P, x);
-        r.u0 = P.tens[x].C / 4;
-    }
-    const LT tx = P.tens[x];
-    r.cnt = (int64_t)tx.H * tx.W * (tx.C / 32);
-    r.g_off = g_off;
-    r.b_off = b_off;
-    *ref = r;
-    return true;
-}
-
 // GroupNorm (+SiLU) as its own pass -> new dense tensor
 int rec_gn(Plan& P, int x, int64_t g_off, int64_t b_off, int silu) {
     rec_gn_finalize(P, x, g_off, b_off);
@@ -518,28 +468,11 @@ int rec_gn(Plan& P, int x, int64_t g_off, int64_t b_off, int silu) {
 
 // can the 2-CTA kernel run (and therefore normalise in flight) a 3x3 convolution on this tensor?
 bool fusable(const Plan& P, int x, int n_rows) {
-    if (P.flags & (2 | 4 | 8 | 16)) return false;   // cross-check kernels / fusion disabled
+    if (P.flags & 2) return false;   // CUDA-core cross-check kernels
     const LT& t = P.tens[x];
     ActView v;
     v.ptr = nullptr; v.B = t.B; v.H = t.H; v.W = t.W; v.C = t.C; v.ld = t.C;
     return conv_halo2_eligible(&v, 9, n_rows);
-}
-
-// norm: the input is GroupNorm'ed + SiLU'ed on load with the scale/shift currently in t_scsh
-int rec_fir(Plan& P, int x, int up, int norm = 0) {
-    const LT tx = P.tens[x];
-    const int out = up ? P.new_t(tx.B, tx.H * 2, tx.W * 2, tx.C, 2) : P.new_t(tx.B, tx.H / 2, tx.W / 2, tx.C, 2);
-    P.use(x); P.use(out);
-    if (norm) P.use(P.t_scsh);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
-        const ActView vx = p.view(x), vo = p.view(out);
-        const float* scsh = norm ? p.fptr(p.t_scsh) : nullptr;
-        const double el = (double)vx.B * vx.H * vx.W * vx.C + (double)vo.B * vo.H * vo.W * vo.C;
-        p.add(LK_FIR, 0.0, 2.0 * el, [=](cudaStream_t s) { return up ? fir_up2_launch(&vx, &vo, s, scsh) : fir_down2_launch(&vx, &vo, s, scsh); });
-        return SNRSE_OK;
-    });
-    return out;
 }
 
 // a = FIR(silu(GroupNorm(x))) and xs = FIR(x) from ONE pass over x (scale/shift currently in t_scsh)
@@ -563,51 +496,35 @@ void rec_fir_dual(Plan& P, int x, int up, int* a, int* xs) {
 int rec_resblock(Plan& P, const Mod& m, int x) {
     // GroupNorm_0 + SiLU (+ FIR resampling of both branches) + Conv_0 + Dense_0(temb)
     int a, xs = x, fuse0 = 0;
-    GnRef gn0, gn1;
-    bool has_gn0 = false, has_gn1 = false;
-    if (!m.up && !m.down && fusable(P, x, m.cout)) {
-        has_gn0 = rec_gn_for_conv(P, x, m.o[0], m.o[1], &gn0);  // normalisation itself happens inside Conv_0
+    if (m.up || m.down) {
+        // one dual-output FIR launch over x produces both branches; every row segment is staged in shared memory once,
+        // raw and normalised, so x comes from DRAM once instead of three times and SiLU is evaluated once per element
+        rec_gn_finalize(P, x, m.o[0], m.o[1]);
+        rec_fir_dual(P, x, m.up ? 1 : 0, &a, &xs);
+    } else if (fusable(P, x, m.cout)) {
+        rec_gn_finalize(P, x, m.o[0], m.o[1]);   // normalisation itself happens inside Conv_0
         a = x;
         fuse0 = 1;
     } else {
-        if ((m.up || m.down) && (P.flags & 32)) {
-            // h = FIR(silu(GroupNorm(x))) with the normalisation applied by the FIR kernel on load (flag bit5).  Measured
-            // on the 16 x 4 s step: GroupNorm -0.34 ms, FIR +0.67 ms (every input element is normalised by the 2-3
-            // threads that load it and the FIR kernels are issue-bound), so the separate pass stays the default.
-            rec_gn_finalize(P, x, m.o[0], m.o[1]);
-            a = rec_fir(P, x, m.up ? 1 : 0, 1);
-            xs = rec_fir(P, x, m.up ? 1 : 0, 0);
-        } else if ((m.up || m.down) && !(P.flags & 64) && !(P.flags & 16)) {
-            // default: one dual-output FIR launch over x produces both branches; every row segment is staged in shared
-            // memory once, raw and normalised, so x comes from DRAM once instead of three times and SiLU is evaluated once
-            // per element.  Measured against the three-pass form (flag bit6): GroupNorm + FIR launches 2.63 -> 2.37 ms per
-            // step, graphed step 20.04 -> 19.98 ms (profiles/r02_step_ab.md); bit-identical.
-            rec_gn_finalize(P, x, m.o[0], m.o[1]);
-            rec_fir_dual(P, x, m.up ? 1 : 0, &a, &xs);
-        } else {
-            a = rec_gn(P, x, m.o[0], m.o[1], 1);
-            if (m.up) { a = rec_fir(P, a, 1); xs = rec_fir(P, x, 1); }
-            if (m.down) { a = rec_fir(P, a, 0); xs = rec_fir(P, x, 0); }
-        }
+        a = rec_gn(P, x, m.o[0], m.o[1], 1);
     }
     const LT ta = P.tens[a];
     const int h = P.new_t(ta.B, ta.H, ta.W, m.cout, 2);
     // the 2-CTA kernel's epilogue also emits the GroupNorm partial sums of what it writes
     const int stats0 = fusable(P, a, m.cout);
-    rec_gemm(P, a, 9, -1, m.o[2], m.cout, m.o[3], m.tb_row, -1, 1.0f, h, fuse0, stats0, 0, has_gn0 ? &gn0 : nullptr);
+    rec_gemm(P, a, 9, -1, m.o[2], m.cout, m.o[3], m.tb_row, -1, 1.0f, h, fuse0, stats0);
     // GroupNorm_1 + SiLU + Conv_1 (+ Conv_2 shortcut or identity residual), / sqrt(2)
     int a2 = h, fuse1 = 0;
     if (fusable(P, h, m.cout)) {
-        has_gn1 = rec_gn_for_conv(P, h, m.o[4], m.o[5], &gn1);
+        rec_gn_finalize(P, h, m.o[4], m.o[5]);
         fuse1 = 1;
     } else {
         a2 = rec_gn(P, h, m.o[4], m.o[5], 1);
     }
     const int out = P.new_t(ta.B, ta.H, ta.W, m.cout, 2);
     const int stats1 = fusable(P, a2, m.cout);
-    const GnRef* g1 = has_gn1 ? &gn1 : nullptr;
-    if (m.has_c2) rec_gemm(P, a2, 9, xs, m.o[6], m.cout, m.o[7], -1, -1, INV_SQRT2, out, fuse1, stats1, 0, g1);
-    else rec_gemm(P, a2, 9, -1, m.o[6], m.cout, m.o[7], -1, xs, INV_SQRT2, out, fuse1, stats1, 0, g1);
+    if (m.has_c2) rec_gemm(P, a2, 9, xs, m.o[6], m.cout, m.o[7], -1, -1, INV_SQRT2, out, fuse1, stats1);
+    else rec_gemm(P, a2, 9, -1, m.o[6], m.cout, m.o[7], -1, xs, INV_SQRT2, out, fuse1, stats1);
     return out;
 }
 
@@ -759,9 +676,7 @@ int record_plan(Plan& P) {
             // tensor-core kernel with the normalisation in flight when the map is large enough, CUDA cores otherwise
             const bool tc = fusable(P, h, 128);
             int a = h;
-            GnRef gnh;
-            bool has_gnh = false;
-            if (tc) has_gnh = rec_gn_for_conv(P, h, mg.o[0], mg.o[1], &gnh);
+            if (tc) rec_gn_finalize(P, h, mg.o[0], mg.o[1]);
             else a = rec_gn(P, h, mg.o[0], mg.o[1], 1);
             const LT th = P.tens[h];
             const int np = P.new_t(th.B, th.H, th.W, 4, 4);
@@ -769,7 +684,7 @@ int record_plan(Plan& P) {
             if (pyr >= 0) up = P.new_t(th.B, th.H, th.W, 4, 4);
             const int prev = pyr;
             P.use(a); P.use(np);
-            if (tc && !has_gnh) P.use(P.t_scsh);
+            if (tc) P.use(P.t_scsh);
             if (prev >= 0) { P.use(prev); P.use(up); }
             P.step++;
             P.builders.push_back([=](Plan& p) -> int {
@@ -781,17 +696,7 @@ int record_plan(Plan& P) {
                 const double px = (double)va.B * va.H * va.W;
                 if (tc) {
                     ConvHaloPlan hp;
-                    GnSrc src{};
-                    if (has_gnh) {
-                        src.st0 = p.stat_ptr(gnh.s0);
-                        src.st1 = gnh.s1 >= 0 ? p.stat_ptr(gnh.s1) : nullptr;
-                        src.U0 = gnh.u0; src.U1 = gnh.u1;
-                        src.inv_count = 1.0 / (double)gnh.cnt;
-                        src.gamma = e.wf(gnh.g_off); src.beta = e.wf(gnh.b_off);
-                        src.eps = 1e-6f;
-                    }
-                    SNRSE_TRY(conv_halo2_make_plan_out4(&hp, &va, e.wb(mc.o[2]), e.wf(mc.o[1]), upp, dst,
-                                                        has_gnh ? nullptr : p.fptr(p.t_scsh), has_gnh ? &src : nullptr));
+                    SNRSE_TRY(conv_halo2_make_plan_out4(&hp, &va, e.wb(mc.o[2]), e.wf(mc.o[1]), upp, dst, p.fptr(p.t_scsh)));
                     p.add(LK_THIN, 2.0 * px * 36 * va.C, px * (2.0 * va.C + 16 + (pv ? 20 : 0)), [=](cudaStream_t s) {
                         if (pv) SNRSE_TRY(fir_up2_f4_launch(pv, upp, va.B, va.H / 2, va.W / 2, s));
                         return conv_halo2_launch(&hp, s);
@@ -972,12 +877,14 @@ int snrse_ncsnpp_set_weights(void* handle, const void* device_blob) {
     return SNRSE_OK;
 }
 
-// flags: bit0 = keep every activation alive (debug taps), bit1 = CUDA-core cross-check convolutions,
-//        bit2 = first-generation (non-halo) tcgen05 kernel for every convolution, bit3 = single-CTA halo kernel,
-//        bit4 = GroupNorm applied by its own kernel instead of inside the following convolution,
-//        bit5 = GroupNorm of the up / down blocks applied inside the FIR kernels (slower, kept for measurement)
+// flags: bit0 = keep every activation alive (debug taps), bit1 = fp32 CUDA-core cross-check path (convolutions,
+//        attention and input packing); no other bit is defined
 int64_t snrse_ncsnpp_plan_bytes(void* handle, int B, int F, int T, int flags) {
     Engine* e = static_cast<Engine*>(handle);
+    if (flags & ~3) {
+        snrse_set_error("plan: unknown flags 0x%x (bit0: keep every activation, bit1: CUDA-core cross-check)", flags);
+        return -1;
+    }
     if (!e || B < 1 || F < 1 || T < 1 || (F % (1 << (e->n_levels - 1))) || (T % (1 << (e->n_levels - 1)))) {
         snrse_set_error("plan: F and T must be positive multiples of 2^(levels-1) (got B=%d F=%d T=%d)", B, F, T);
         return -1;

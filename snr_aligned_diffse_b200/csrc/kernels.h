@@ -51,18 +51,6 @@ int conv_gemm_make_plan_ex(ConvGemmPlan* p, const ActView* a0, int taps0, const 
 int conv_gemm_launch(const ConvGemmPlan* p, cudaStream_t s);
 
 // ----------------------------------------------------------------------------- conv_halo2.cu
-// GroupNorm statistics of the operand for the 2-CTA kernel's in-kernel finalize: the normalising warps turn the
-// fixed-point unit sums (gn_fixed.cuh; one or two sources = the halves of a concatenation) into per-channel scale /
-// shift themselves, with the arithmetic of gn_finalize_kernel, instead of reading a table a gn_finalize launch wrote.
-struct GnSrc {
-    const unsigned long long* st0;
-    const unsigned long long* st1;
-    int U0, U1;            // 4-channel units per source (U1 = 0: single source)
-    double inv_count;      // 1 / (elements per group)
-    const float* gamma;
-    const float* beta;
-    float eps;
-};
 // Plan of the persistent 2-CTA halo-reuse kernel: 3x3 convolutions with W >= 8, H >= 8, N in {128, 256}.
 struct ConvHaloPlan {
     CUtensorMap mapA0, mapA1, mapB, mapOut, mapRes;   // mapOut / mapRes: 2-CTA kernel only (TMA epilogue)
@@ -77,9 +65,7 @@ struct ConvHaloPlan {
     float scale;
     bf16* out;
     int out_ld;
-    const float* scsh;            // precomputed GroupNorm scale / shift table, or
-    GnSrc gn;                     // ... the statistics to derive it from inside the kernel (has_gn)
-    int has_gn;
+    const float* scsh;            // GroupNorm scale / shift table of operand 0, or null
     unsigned long long* ustats;
     float* out4;                  // 2-CTA kernel, thin C -> 4 output convolution only
     const float* addend4;
@@ -88,10 +74,9 @@ struct ConvHaloPlan {
 bool conv_halo2_eligible(const ActView* a0, int taps0, int n_rows);
 // scsh (nullable): GroupNorm scale/shift [B][2][C0] (gn_finalize_launch); when given, operand 0 is replaced by
 // silu(x*scale + shift) inside the kernel (GroupNorm+SiLU+conv3x3 of ResnetBlockBigGANpp without the HBM round trip).
-// gn (nullable, instead of scsh): the same normalisation with scale / shift computed in the kernel from the statistics.
 int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, const bf16* wt, int n_rows,
                          const float* bias, const float* tbias, int tb_stride, const ActView* res, float scale, bf16* out,
-                         int out_ld, const float* scsh, unsigned long long* ustats, const GnSrc* gn = nullptr);
+                         int out_ld, const float* scsh, unsigned long long* ustats);
 // ustats (nullable): the epilogue also accumulates the GroupNorm sums of the result into [B][N/4][2] (zeroed by the
 // caller; gn_finalize_launch source format), so the following GroupNorm needs no pass over the tensor.
 int conv_halo2_launch(const ConvHaloPlan* p, cudaStream_t s);
@@ -99,7 +84,7 @@ int conv_halo2_launch(const ConvHaloPlan* p, cudaStream_t s);
 // Thin 3x3 output convolution C -> 4 on the 2-CTA kernel (N = 16, weights [16][9*C] bf16 with rows 4..15 zero), fp32
 // result [B,H,W,4] = conv + bias4 (+ addend4); scsh as above.  Needs W >= 8, H >= 8.
 int conv_halo2_make_plan_out4(ConvHaloPlan* p, const ActView* a0, const bf16* wt16, const float* bias4, const float* addend4,
-                              float* out4, const float* scsh, const GnSrc* gn = nullptr);
+                              float* out4, const float* scsh);
 
 // ----------------------------------------------------------------------------- conv_simt.cu
 // Reference-grade direct convolution on CUDA cores (debug / cross-check path, fp32 accumulate).

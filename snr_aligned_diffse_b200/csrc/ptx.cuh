@@ -77,12 +77,6 @@ __device__ __forceinline__ void tma_load_4d(uint32_t smem_dst, const CUtensorMap
         ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
         : "memory");
 }
-// TMA prefetch of a box into L2 (a hint: no shared memory, no completion to wait for)
-__device__ __forceinline__ void tma_prefetch_4d(const CUtensorMap* map, int c0, int c1, int c2, int c3) {
-    asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];"
-                 ::"l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-                 : "memory");
-}
 __device__ __forceinline__ void tma_load_3d(uint32_t smem_dst, const CUtensorMap* map, uint32_t bar, int c0, int c1,
                                             int c2) {
     asm volatile(

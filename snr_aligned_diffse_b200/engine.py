@@ -40,7 +40,6 @@ class NCSNppEngine:
         self._ws = {}       # (B,F,T) -> (workspace tensor, flags)
         self._graphs = {}
         self.weights_generation = 0    # bumped by every load_state_dict: tag for caches of captured CUDA graphs
-        self.default_flags = 0         # plan flags used when forward() is called without `flags` (A/B measurements)
 
     def __del__(self):
         try:
@@ -216,10 +215,8 @@ class NCSNppEngine:
         self._ws[key] = (ws, flags)
         self._graphs = {k: v for k, v in self._graphs.items() if k[:3] != key}
 
-    def forward(self, x, y, t, mode=MODE_RAW, out=None, flags=None):
+    def forward(self, x, y, t, mode=MODE_RAW, out=None, flags=0):
         """x, y: complex64 [B,F,T] (or [B,1,F,T]); t: float32 [B].  Enqueues on the current stream."""
-        if flags is None:
-            flags = self.default_flags
         assert x.is_cuda and x.dtype == torch.complex64 and y.dtype == torch.complex64
         shape = x.shape
         B, F, T = shape[0], shape[-2], shape[-1]

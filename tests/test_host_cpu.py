@@ -22,7 +22,7 @@ def test_abi_exports_every_declared_symbol():
     debug = set(re.findall(r"\b(snrse_[a-z0-9_]+)\s*\(", dbg))
     # measurement / debug entry points live in their own header, not in the product ABI
     assert debug == {"snrse_ncsnpp_num_launch_groups", "snrse_ncsnpp_profile_forward", "snrse_ncsnpp_read_tap",
-                     "snrse_conv_halo_set_debug", "snrse_conv_halo_set_prefetch"} and not (debug & product)
+                     "snrse_conv_halo_set_debug", "snrse_fir_dual_nhwc"} and not (debug & product)
     declared = product | debug
     lib = _lib.load()
     assert declared, "no declarations found"
@@ -71,6 +71,10 @@ def test_native_param_table_matches_reference_inventory(golden_dir):
         eng.workspace_bytes(1, 256, 96)      # T must be a multiple of 64 (6 halvings, util/other.py:83-90)
     with pytest.raises(RuntimeError):
         eng.workspace_bytes(1, 128, 64)      # attention placement was built for F = image_size
+    assert all(eng.workspace_bytes(1, 256, 64, flags=f) > 0 for f in (1, 2, 3))
+    for f in (4, 128, -1):                   # only bit0 (keep every activation) and bit1 (cross-check) are defined
+        with pytest.raises(RuntimeError, match="unknown flags"):
+            eng.workspace_bytes(1, 256, 64, flags=f)
 
 
 def test_weight_packing_layouts():

@@ -32,11 +32,8 @@ def main():
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--only", type=int, default=-1)
     ap.add_argument("--debug", action="store_true")
-    ap.add_argument("--prefetch", type=int, default=0, help="L2 prefetch of the next tile's boxes in the 2-CTA kernel (0: off)")
     args = ap.parse_args()
     impls = [int(i) for i in args.impl.split(",")]
-    from snr_aligned_diffse_b200 import _lib
-    _lib.load().snrse_conv_halo_set_prefetch(args.prefetch)
     g = torch.Generator().manual_seed(0)
     for idx, (B, H, W, Ci, Co, Cs) in enumerate(SHAPES):
         if args.only >= 0 and idx != args.only:

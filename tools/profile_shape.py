@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Per-kind time of one NCSN++ forward for a (B, T) bucket, measured with CUDA events between launch groups
-(snrse_ncsnpp_profile_forward).  Usage: python tools/profile_shape.py B T [flags] [prefetch 0|1]"""
+(snrse_ncsnpp_profile_forward).  Usage: python tools/profile_shape.py B T [flags]   (0 default, 2 CUDA-core cross-check)"""
 import os
 import sys
 
@@ -13,9 +13,8 @@ from snr_aligned_diffse_b200.synth import synth_state_dict  # noqa: E402
 
 B, T = int(sys.argv[1]), int(sys.argv[2])
 flags = int(sys.argv[3]) if len(sys.argv) > 3 else 0
-prefetch = int(sys.argv[4]) if len(sys.argv) > 4 else 0
-from snr_aligned_diffse_b200 import _lib  # noqa: E402
-_lib.load().snrse_conv_halo_set_prefetch(prefetch)
+if flags not in (0, 1, 2):
+    sys.exit("flags: 0 (default), 1 (keep every activation) or 2 (CUDA-core cross-check)")
 eng = NCSNppEngine()
 eng.load_state_dict(synth_state_dict(eng.param_shapes(), seed=0), "cuda")
 g = torch.Generator().manual_seed(0)
@@ -29,7 +28,7 @@ for _ in range(3 + int(os.environ.get("STEADY", "0"))):
 runs = [eng.profile_forward(x, y, t, mode=1, flags=flags) for _ in range(5)]
 runs.sort(key=lambda pr: sum(q["ms"] for q in pr))
 prof = runs[2]                      # median of five back-to-back passes
-print(f"flags={flags} prefetch={prefetch}")
+print(f"flags={flags}")
 tot = sum(p["ms"] for p in prof)
 by = {}
 for p in prof:

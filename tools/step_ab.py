@@ -1,9 +1,8 @@
 #!/usr/bin/env python
-"""A/B of engine plan flags on the REAL step: one captured CUDA graph of the full 16 x 4 s sebridge_v3 pass per variant
-(own model, own activation arena), replayed back to back; the variants are interleaved round-robin so that thermal /
-power drift hits them equally.  Usage: python tools/step_ab.py [flags ...]   (default: 0 128 64 192)
-  bit6 (64): GroupNorm pass + two FIR passes in the up / down blocks instead of the dual-output FIR launch (default)
-  bit7 (128): in-kernel GroupNorm finalize of the normalising convolutions instead of gn_finalize launches"""
+"""A/B of programmatic-dependent-launch masks (snrse_set_pdl) on the REAL step: one captured CUDA graph of the full
+16 x 4 s sebridge_v3 pass per variant (own model, own activation arena), replayed back to back; the variants are
+interleaved round-robin so that thermal / power drift hits them equally.  Usage: python tools/step_ab.py [mask ...]
+(default: 2 0, the library default against plain stream-ordered launches)"""
 import json
 import os
 import sys
@@ -16,22 +15,17 @@ import bench  # noqa: E402
 from snr_aligned_diffse_b200.pipeline import GraphedEnhancer  # noqa: E402
 
 from snr_aligned_diffse_b200 import _lib  # noqa: E402
-# a variant is FLAGS[:PREFETCH[:PDL]] (L2 prefetch switch of the 2-CTA convolution kernel; programmatic dependent launch
-# on / off -- both are read when the graph is captured)
-variants = sys.argv[1:] or ["0", "128", "64", "192"]
-flags = variants
+# the mask is read when the graph is captured
+variants = sys.argv[1:] or ["2", "0"]
 dev = torch.device("cuda", 0)
 torch.cuda.set_device(0)
 L = int(bench.SECONDS * bench.SR)
 y = bench.synth_waves(bench.BATCH, L, seed=1000).to(dev)
 pipes = []
 for i, v in enumerate(variants):
-    f, pf, pdl = (v.split(":") + ["0", "1"])[:3]     # FLAGS[:PREFETCH[:PDL]]
-    _lib.load().snrse_conv_halo_set_prefetch(int(pf))
-    _lib.load().snrse_set_pdl(int(pdl))
+    _lib.load().snrse_set_pdl(int(v))
     model, _ = bench.build_models(dev, with_estimator=(i == 0))
     model.dnn._ensure_device_weights()
-    model.dnn.engine.default_flags = int(f)
     p = GraphedEnhancer(model, bench.BATCH, L, dev, oracle=False)
     p.y_dev.copy_(y)
     p.capture(warmup=2)
@@ -41,9 +35,9 @@ for p in pipes:
     for _ in range(10):
         p.replay()
 torch.cuda.synchronize()
-tot = {f: [] for f in flags}
+tot = {v: [] for v in variants}
 for rnd in range(6):
-    for f, p in zip(flags, pipes):
+    for v, p in zip(variants, pipes):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         with torch.cuda.stream(p.stream):
             e0.record(p.stream)
@@ -51,6 +45,6 @@ for rnd in range(6):
                 p.graph.replay()
             e1.record(p.stream)
         torch.cuda.synchronize()
-        tot[f].append(e0.elapsed_time(e1) / 25)
-print(json.dumps({str(f): dict(ms_per_step_rounds=[round(v, 3) for v in tot[f]], median=round(sorted(tot[f])[len(tot[f]) // 2], 3))
-                  for f in flags}))
+        tot[v].append(e0.elapsed_time(e1) / 25)
+print(json.dumps({v: dict(ms_per_step_rounds=[round(ms, 3) for ms in tot[v]], median=round(sorted(tot[v])[len(tot[v]) // 2], 3))
+                  for v in variants}))
