@@ -131,7 +131,7 @@ int snrse_conv_nhwc(const void* x0, int c0, int taps0, const void* x1, int c1, c
         return conv_simt_launch(&a0, taps0, x1 ? &a1 : nullptr, static_cast<const bf16*>(wt), n, bias, tbias, tb_stride,
                                 res ? &r : nullptr, scale, static_cast<bf16*>(out), n, S(stream));
     }
-    if (impl == 0 && conv_halo2_eligible(&a0, taps0, n)) {
+    if (impl == 0 && conv_halo2_eligible(a0.H, a0.W, taps0, n)) {
         ConvHaloPlan hp;
         SNRSE_TRY(conv_halo2_make_plan(&hp, &a0, x1 ? &a1 : nullptr, static_cast<const bf16*>(wt), n, bias, tbias, tb_stride,
                                        res ? &r : nullptr, scale, static_cast<bf16*>(out), n, nullptr, nullptr));
@@ -153,7 +153,7 @@ int snrse_conv3x3_nhwc_stats(const void* x0, int c0, const void* x1, int c1, con
     ActView a0 = mk_view(x0, B, H, W, c0, c0), a1, r;
     if (x1) a1 = mk_view(x1, B, H, W, c1, c1);
     if (res) r = mk_view(res, B, H, W, n, n);
-    SNRSE_CHECK_ARG(conv_halo2_eligible(&a0, 9, n), "conv3x3_stats: needs W >= 8, H >= 8, N in {128, 256}");
+    SNRSE_CHECK_ARG(conv_halo2_eligible(a0.H, a0.W, 9, n), "conv3x3_stats: needs W >= 8, H >= 8, N in {128, 256}");
     SNRSE_CUDA(cudaMemsetAsync(ustats, 0, (size_t)B * (n / 4) * 16, S(stream)));
     ConvHaloPlan hp;
     SNRSE_TRY(conv_halo2_make_plan(&hp, &a0, x1 ? &a1 : nullptr, static_cast<const bf16*>(wt), n, bias, tbias, tb_stride,
@@ -188,7 +188,7 @@ int snrse_gn_silu_conv3x3_nhwc(const void* x0, int c0, const float* gamma, const
     ActView a0 = mk_view(x0, B, H, W, c0, c0), a1, r;
     if (x1) a1 = mk_view(x1, B, H, W, c1, c1);
     if (res) r = mk_view(res, B, H, W, n, n);
-    SNRSE_CHECK_ARG(conv_halo2_eligible(&a0, 9, n), "gn_silu_conv3x3: needs W >= 8, H >= 8, N in {128, 256}");
+    SNRSE_CHECK_ARG(conv_halo2_eligible(a0.H, a0.W, 9, n), "gn_silu_conv3x3: needs W >= 8, H >= 8, N in {128, 256}");
     unsigned long long* ust = static_cast<unsigned long long*>(workspace);
     float* scsh = reinterpret_cast<float*>(ust + (int64_t)B * 128 * 2);
     const int64_t hw = (int64_t)H * W;

@@ -13,6 +13,7 @@
 // (CUDA-graph capturable: no allocation, no sync, no host reads).
 #include <algorithm>
 #include <functional>
+#include <initializer_list>
 #include <map>
 #include <string>
 #include <tuple>
@@ -45,13 +46,16 @@ struct Param {
 struct Mod {
     int kind;  // 0 fourier 1 linear 2 conv_in 3 res 4 attn 5 combine 6 gn 7 conv_out
     int cin = 0, cout = 0, up = 0, down = 0, has_c2 = 0;
-    int64_t o[12] = {0};  // blob offsets (meaning per kind)
     int tb_row = 0;       // row offset into the concatenated Dense_0 matrix
+    // blob offsets of the parameters
+    int64_t gn_g = 0, gn_b = 0;    // GroupNorm affine: gn; GroupNorm_0 of res and attn
+    int64_t w = 0, b = 0;          // fourier W; linear; conv_in / conv_out (fp32 taps); combine Conv_0; res Conv_0;
+                                   // attn NIN_0..2 as one [3C][C] qkv matrix
+    int64_t w_tc = 0;              // conv_in / conv_out: bf16 tensor-core copy of w
+    int64_t gn1_g = 0, gn1_b = 0;  // res GroupNorm_1
+    int64_t w1 = 0, b1 = 0;        // res Conv_1 (| Conv_2 along K; b1 holds b1 + b2); attn NIN_3
 };
 enum { M_FOURIER, M_LINEAR, M_CONV_IN, M_RES, M_ATTN, M_COMBINE, M_GN, M_CONV_OUT };
-// res:   o[0]=gn0.g o[1]=gn0.b o[2]=W0 o[3]=b0 o[4]=gn1.g o[5]=gn1.b o[6]=W1(|W2) o[7]=b1(+b2)
-// attn:  o[0]=gn.g o[1]=gn.b o[2]=Wqkv[3C][C] o[3]=bqkv[3C] o[4]=W3 o[5]=b3
-// others: o[0]=weight o[1]=bias
 
 struct LT {  // logical tensor
     int B, H, W, C;
@@ -66,6 +70,7 @@ struct Engine;
 struct Plan {
     Engine* eng;
     int B, F, T, flags;
+    bool cross_check = false;   // flags bit1: fp32 CUDA-core convolutions and attention
     std::vector<LT> tens;
     std::vector<std::function<int(Plan&)>> builders;
     std::vector<std::function<int(cudaStream_t)>> launches;
@@ -82,7 +87,7 @@ struct Plan {
     int64_t ws_bytes = 0;
     uint8_t* ws = nullptr;
     // fixed slots
-    int t_x4, t_tb, t_tscr, t_stats, t_scsh, t_pyr_final;
+    int t_x4, t_tb, t_tscr, t_stats, t_scsh;
     // bound per call
     const float* t_ptr = nullptr;
     const float2 *x_ptr = nullptr, *y_ptr = nullptr;
@@ -108,10 +113,17 @@ struct Plan {
         tens.push_back(t);
         return (int)tens.size() - 1;
     }
-    void use(int id) {
-        LT& r = tens[root(id)];
-        r.first = std::min(r.first, step);
-        r.last = std::max(r.last, step);
+    // Record one step: every tensor it reads or writes (ids < 0 are absent operands) lives at least through this step,
+    // and `build` appends the step's launches once the buffers are placed.
+    void record(std::initializer_list<int> ids, std::function<int(Plan&)> build) {
+        for (int id : ids) {
+            if (id < 0) continue;
+            LT& r = tens[root(id)];
+            r.first = std::min(r.first, step);
+            r.last = std::max(r.last, step);
+        }
+        step++;
+        builders.push_back(std::move(build));
     }
     int concat(int a, int b) {
         LT &ta = tens[a], &tb = tens[b];
@@ -238,84 +250,84 @@ int build_topology(Engine& e, int image_size) {
         const std::string p = "dnn.all_modules." + std::to_string(i) + ".";
         switch (r.kind) {
             case M_FOURIER:
-                r.o[0] = e.alloc(nf * 4);
-                e.add_param(p + "W", {nf}, PK_RAW_F32, r.o[0]);
+                r.w = e.alloc(nf * 4);
+                e.add_param(p + "W", {nf}, PK_RAW_F32, r.w);
                 break;
             case M_LINEAR:
-                r.o[0] = e.alloc((int64_t)r.cout * r.cin * 4);
-                r.o[1] = e.alloc(r.cout * 4);
-                e.add_param(p + "weight", {r.cout, r.cin}, PK_RAW_F32, r.o[0]);
-                e.add_param(p + "bias", {r.cout}, PK_RAW_F32, r.o[1]);
+                r.w = e.alloc((int64_t)r.cout * r.cin * 4);
+                r.b = e.alloc(r.cout * 4);
+                e.add_param(p + "weight", {r.cout, r.cin}, PK_RAW_F32, r.w);
+                e.add_param(p + "bias", {r.cout}, PK_RAW_F32, r.b);
                 break;
             case M_CONV_IN:
             case M_CONV_OUT:
-                r.o[0] = e.alloc((int64_t)r.cout * r.cin * 9 * 4);
-                r.o[1] = e.alloc(r.cout * 4);
-                e.add_param(p + "weight", {r.cout, r.cin, 3, 3}, PK_CONV3_TAP_F32, r.o[0]);
-                e.add_param(p + "bias", {r.cout}, PK_RAW_F32, r.o[1]);
+                r.w = e.alloc((int64_t)r.cout * r.cin * 9 * 4);
+                r.b = e.alloc(r.cout * 4);
+                e.add_param(p + "weight", {r.cout, r.cin, 3, 3}, PK_CONV3_TAP_F32, r.w);
+                e.add_param(p + "bias", {r.cout}, PK_RAW_F32, r.b);
                 if (r.kind == M_CONV_IN) {    // tensor-core copy for the 64-channel hi/lo operand (pack_input64)
-                    r.o[2] = e.alloc((int64_t)r.cout * 9 * 64 * 2);
-                    e.add_param(p + "weight", {r.cout, r.cin, 3, 3}, PK_CONV3_K_BF16_HILO64, r.o[2], 9 * 64, 0);
+                    r.w_tc = e.alloc((int64_t)r.cout * 9 * 64 * 2);
+                    e.add_param(p + "weight", {r.cout, r.cin, 3, 3}, PK_CONV3_K_BF16_HILO64, r.w_tc, 9 * 64, 0);
                 }
                 if (r.kind == M_CONV_OUT) {   // tensor-core copy: bf16 K-major, 16 rows of which the first 4 are real
-                    r.o[2] = e.alloc((int64_t)16 * 9 * r.cin * 2);
-                    e.add_param(p + "weight", {r.cout, r.cin, 3, 3}, PK_CONV3_K_BF16, r.o[2], 9 * (int64_t)r.cin, 0);
+                    r.w_tc = e.alloc((int64_t)16 * 9 * r.cin * 2);
+                    e.add_param(p + "weight", {r.cout, r.cin, 3, 3}, PK_CONV3_K_BF16, r.w_tc, 9 * (int64_t)r.cin, 0);
                 }
                 break;
             case M_GN:
-                r.o[0] = e.alloc(r.cin * 4);
-                r.o[1] = e.alloc(r.cin * 4);
-                e.add_param(p + "weight", {r.cin}, PK_RAW_F32, r.o[0]);
-                e.add_param(p + "bias", {r.cin}, PK_RAW_F32, r.o[1]);
+                r.gn_g = e.alloc(r.cin * 4);
+                r.gn_b = e.alloc(r.cin * 4);
+                e.add_param(p + "weight", {r.cin}, PK_RAW_F32, r.gn_g);
+                e.add_param(p + "bias", {r.cin}, PK_RAW_F32, r.gn_b);
                 break;
             case M_COMBINE:
-                r.o[0] = e.alloc((int64_t)r.cout * 4 * 4);
-                r.o[1] = e.alloc(r.cout * 4);
-                e.add_param(p + "Conv_0.weight", {r.cout, 4, 1, 1}, PK_RAW_F32, r.o[0]);
-                e.add_param(p + "Conv_0.bias", {r.cout}, PK_RAW_F32, r.o[1]);
+                r.w = e.alloc((int64_t)r.cout * 4 * 4);
+                r.b = e.alloc(r.cout * 4);
+                e.add_param(p + "Conv_0.weight", {r.cout, 4, 1, 1}, PK_RAW_F32, r.w);
+                e.add_param(p + "Conv_0.bias", {r.cout}, PK_RAW_F32, r.b);
                 break;
             case M_ATTN: {
                 const int c = r.cin;
-                r.o[0] = e.alloc(c * 4);
-                r.o[1] = e.alloc(c * 4);
-                r.o[2] = e.alloc((int64_t)3 * c * c * 2);
-                r.o[3] = e.alloc(3 * c * 4);
-                r.o[4] = e.alloc((int64_t)c * c * 2);
-                r.o[5] = e.alloc(c * 4);
-                e.add_param(p + "GroupNorm_0.weight", {c}, PK_RAW_F32, r.o[0]);
-                e.add_param(p + "GroupNorm_0.bias", {c}, PK_RAW_F32, r.o[1]);
+                r.gn_g = e.alloc(c * 4);
+                r.gn_b = e.alloc(c * 4);
+                r.w = e.alloc((int64_t)3 * c * c * 2);
+                r.b = e.alloc(3 * c * 4);
+                r.w1 = e.alloc((int64_t)c * c * 2);
+                r.b1 = e.alloc(c * 4);
+                e.add_param(p + "GroupNorm_0.weight", {c}, PK_RAW_F32, r.gn_g);
+                e.add_param(p + "GroupNorm_0.bias", {c}, PK_RAW_F32, r.gn_b);
                 for (int j = 0; j < 3; ++j) {
-                    e.add_param(p + "NIN_" + std::to_string(j) + ".W", {c, c}, PK_NIN_K_BF16, r.o[2] + (int64_t)j * c * c * 2, c, 0);
-                    e.add_param(p + "NIN_" + std::to_string(j) + ".b", {c}, PK_RAW_F32, r.o[3] + (int64_t)j * c * 4);
+                    e.add_param(p + "NIN_" + std::to_string(j) + ".W", {c, c}, PK_NIN_K_BF16, r.w + (int64_t)j * c * c * 2, c, 0);
+                    e.add_param(p + "NIN_" + std::to_string(j) + ".b", {c}, PK_RAW_F32, r.b + (int64_t)j * c * 4);
                 }
-                e.add_param(p + "NIN_3.W", {c, c}, PK_NIN_K_BF16, r.o[4], c, 0);
-                e.add_param(p + "NIN_3.b", {c}, PK_RAW_F32, r.o[5]);
+                e.add_param(p + "NIN_3.W", {c, c}, PK_NIN_K_BF16, r.w1, c, 0);
+                e.add_param(p + "NIN_3.b", {c}, PK_RAW_F32, r.b1);
                 break;
             }
             case M_RES: {
                 const int ci = r.cin, co = r.cout;
                 const int64_t k1 = 9 * (int64_t)co + (r.has_c2 ? ci : 0);
-                r.o[0] = e.alloc(ci * 4);
-                r.o[1] = e.alloc(ci * 4);
-                r.o[2] = e.alloc((int64_t)co * 9 * ci * 2);
-                r.o[3] = e.alloc(co * 4);
-                r.o[4] = e.alloc(co * 4);
-                r.o[5] = e.alloc(co * 4);
-                r.o[6] = e.alloc((int64_t)co * k1 * 2);
-                r.o[7] = e.alloc(co * 4);
-                e.add_param(p + "GroupNorm_0.weight", {ci}, PK_RAW_F32, r.o[0]);
-                e.add_param(p + "GroupNorm_0.bias", {ci}, PK_RAW_F32, r.o[1]);
-                e.add_param(p + "Conv_0.weight", {co, ci, 3, 3}, PK_CONV3_K_BF16, r.o[2], 9 * (int64_t)ci, 0);
-                e.add_param(p + "Conv_0.bias", {co}, PK_RAW_F32, r.o[3]);
+                r.gn_g = e.alloc(ci * 4);
+                r.gn_b = e.alloc(ci * 4);
+                r.w = e.alloc((int64_t)co * 9 * ci * 2);
+                r.b = e.alloc(co * 4);
+                r.gn1_g = e.alloc(co * 4);
+                r.gn1_b = e.alloc(co * 4);
+                r.w1 = e.alloc((int64_t)co * k1 * 2);
+                r.b1 = e.alloc(co * 4);
+                e.add_param(p + "GroupNorm_0.weight", {ci}, PK_RAW_F32, r.gn_g);
+                e.add_param(p + "GroupNorm_0.bias", {ci}, PK_RAW_F32, r.gn_b);
+                e.add_param(p + "Conv_0.weight", {co, ci, 3, 3}, PK_CONV3_K_BF16, r.w, 9 * (int64_t)ci, 0);
+                e.add_param(p + "Conv_0.bias", {co}, PK_RAW_F32, r.b);
                 e.add_param(p + "Dense_0.weight", {co, d}, PK_RAW_F32, e.dense_w_off + (int64_t)r.tb_row * d * 4);
                 e.add_param(p + "Dense_0.bias", {co}, PK_RAW_F32, e.dense_b_off + (int64_t)r.tb_row * 4);
-                e.add_param(p + "GroupNorm_1.weight", {co}, PK_RAW_F32, r.o[4]);
-                e.add_param(p + "GroupNorm_1.bias", {co}, PK_RAW_F32, r.o[5]);
-                e.add_param(p + "Conv_1.weight", {co, co, 3, 3}, PK_CONV3_K_BF16, r.o[6], k1, 0);
-                e.add_param(p + "Conv_1.bias", {co}, PK_RAW_F32, r.o[7]);
+                e.add_param(p + "GroupNorm_1.weight", {co}, PK_RAW_F32, r.gn1_g);
+                e.add_param(p + "GroupNorm_1.bias", {co}, PK_RAW_F32, r.gn1_b);
+                e.add_param(p + "Conv_1.weight", {co, co, 3, 3}, PK_CONV3_K_BF16, r.w1, k1, 0);
+                e.add_param(p + "Conv_1.bias", {co}, PK_RAW_F32, r.b1);
                 if (r.has_c2) {
-                    e.add_param(p + "Conv_2.weight", {co, ci, 1, 1}, PK_CONV1_K_BF16, r.o[6], k1, 9 * (int64_t)co);
-                    e.add_param(p + "Conv_2.bias", {co}, PK_RAW_F32, r.o[7], 0, 0, 1);
+                    e.add_param(p + "Conv_2.weight", {co, ci, 1, 1}, PK_CONV1_K_BF16, r.w1, k1, 9 * (int64_t)co);
+                    e.add_param(p + "Conv_2.bias", {co}, PK_RAW_F32, r.b1, 0, 0, 1);
                 }
                 break;
             }
@@ -325,77 +337,102 @@ int build_topology(Engine& e, int image_size) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// Plan recording helpers.  Each helper (a) creates output tensors, (b) marks tensor lifetimes at the
-// current step, (c) registers a builder that, once buffers are placed, appends the launch closures.
+// Plan recording helpers.  Each helper creates its output tensors and records its steps with Plan::record; the
+// builders turn the steps into launch closures once the buffers are placed.
 // ------------------------------------------------------------------------------------------------
 const float INV_SQRT2 = 0.70710678118654752440f;
 constexpr int MAX_STAT_ENTRIES = 192;   // tensors with GroupNorm statistics per forward (NCSN++ default: ~110)
 enum { LK_OTHER = 0, LK_GEMM = 1, LK_GN = 2, LK_FIR = 3, LK_ATTN = 4, LK_THIN = 5, LK_HEAD = 6 };
 
-int rec_gemm(Plan& P, int a0, int taps0, int a1, int64_t w_off, int n_rows, int64_t bias_off, int tb_row, int res,
-             float scale, int out, int norm = 0, int want_stats = 0, int algo_cin = 0) {
-    // algo_cin > 0: channel count the ALGORITHM contracts over when the operand is a zero-padded copy (the 4-channel
-    // network input enters as a 64-channel hi/lo tile): FLOPs and bytes are booked at algo_cin, not at the padded width
-    P.use(a0);
-    if (norm) P.use(P.t_scsh);
+// The kernel that runs a convolution, chosen once, when the step is recorded.  The steps around a convolution depend on
+// it: only the 2-CTA kernel normalises its operand in flight and gathers the GroupNorm sums of its output.
+enum ConvPath {
+    CONV_SIMT,    // fp32 CUDA cores
+    CONV_HALO2,   // 2-CTA (cta_group::2) tcgen05 halo kernel
+    CONV_GEMM,    // single-CTA tcgen05 implicit GEMM
+};
+// Convolution of an H x W operand with `taps` taps (9: 3x3, 1: 1x1) to n_rows output channels:
+//   - cross-check plans (flags bit1): CUDA cores everywhere; the input convolution reads the fp32 input (conv_in4)
+//   - the C -> 4 output head (n_rows 4): the 2-CTA kernel with a 16-row weight tile where the map fits its tiles,
+//     CUDA cores (conv_out4) otherwise
+//   - every other convolution, the input convolution on its 64-channel hi/lo operand included: the 2-CTA kernel where
+//     it is eligible, the single-CTA implicit GEMM otherwise
+ConvPath conv_path(const Plan& P, int H, int W, int taps, int n_rows) {
+    if (P.cross_check) return CONV_SIMT;
+    if (n_rows == 4) return conv_halo2_fits(H, W) ? CONV_HALO2 : CONV_SIMT;
+    return conv_halo2_eligible(H, W, taps, n_rows) ? CONV_HALO2 : CONV_GEMM;
+}
+
+// out = (conv(x) [+ conv1x1(shortcut)] + bias + time-embedding bias [+ res]) * scale; ids < 0 and offsets < 0 are absent
+struct Conv {
+    int x = -1;           // operand
+    int taps = 9;         // taps of x: 9 (3x3, padding 1) or 1
+    int shortcut = -1;    // 1x1 operand appended along K (Conv_2 of a residual block)
+    int64_t w = -1;       // blob offset of the bf16 K-major weights [n_rows][taps * C(x) + C(shortcut)]
+    int n_rows = 0;       // output channels
+    int64_t bias = -1;    // blob offset of the fp32 bias
+    int tb_row = -1;      // first row of this layer in the time-embedding bias block t_tb
+    int res = -1;         // identity residual
+    float scale = 1.0f;
+    int out = -1;
+    // channel count the ALGORITHM contracts over when x is a zero-padded copy (the 4-channel network input enters as a
+    // 64-channel hi/lo tile): FLOPs and bytes are booked at algo_cin, not at the padded width
+    int algo_cin = 0;
+    bool norm = false;    // x is normalised in flight: GroupNorm + SiLU with the scale/shift in t_scsh
+};
+
+int rec_conv(Plan& P, const Conv& c) {
+    const ConvPath path = conv_path(P, P.tens[c.x].H, P.tens[c.x].W, c.taps, c.n_rows);
     int st = -1;
-    if (want_stats) {   // the epilogue also accumulates the GroupNorm sums of `out`
+    if (path == CONV_HALO2) {   // the epilogue also accumulates the GroupNorm sums of `out`
         st = P.n_stat_entries++;
-        P.stats_of[out] = st;
+        P.stats_of[c.out] = st;
     }
-    if (a1 >= 0) P.use(a1);
-    if (res >= 0) P.use(res);
-    P.use(out);
-    if (tb_row >= 0) P.use(P.t_tb);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
+    P.record({c.x, c.norm ? P.t_scsh : -1, c.shortcut, c.res, c.out, c.tb_row >= 0 ? P.t_tb : -1}, [=](Plan& p) -> int {
         Engine& e = *p.eng;
-        ActView va0 = p.view(a0), va1, vres, vout = p.view(out);
-        if (a1 >= 0) va1 = p.view(a1);
-        if (res >= 0) vres = p.view(res);
-        const float* bias = bias_off >= 0 ? e.wf(bias_off) : nullptr;
-        const float* tb = tb_row >= 0 ? p.fptr(p.t_tb) + tb_row : nullptr;
+        ActView va0 = p.view(c.x), va1, vres, vout = p.view(c.out);
+        if (c.shortcut >= 0) va1 = p.view(c.shortcut);
+        if (c.res >= 0) vres = p.view(c.res);
+        const float* bias = c.bias >= 0 ? e.wf(c.bias) : nullptr;
+        const float* tb = c.tb_row >= 0 ? p.fptr(p.t_tb) + c.tb_row : nullptr;
         const int tb_stride = e.dense_rows;
-        if (p.flags & 2) {  // CUDA-core cross-check path
-            const int64_t ktot = (int64_t)taps0 * va0.C + (a1 >= 0 ? va1.C : 0);
-            for (int n0 = 0; n0 < n_rows; n0 += 256) {
-                const int nn = std::min(256, n_rows - n0);
-                const bf16* w = e.wb(w_off) + (int64_t)n0 * ktot;
+        const double px = (double)va0.B * va0.H * va0.W;
+        const int c1 = c.shortcut >= 0 ? va1.C : 0;
+        if (path == CONV_SIMT) {
+            const int64_t ktot = (int64_t)c.taps * va0.C + c1;
+            for (int n0 = 0; n0 < c.n_rows; n0 += 256) {
+                const int nn = std::min(256, c.n_rows - n0);
+                const bf16* w = e.wb(c.w) + (int64_t)n0 * ktot;
                 ActView r2 = vres;
-                if (res >= 0) r2.ptr += n0;
-                const double px1 = (double)va0.B * va0.H * va0.W;
-                p.add(LK_GEMM, 2.0 * px1 * nn * (double)ktot, 0.0, [=](cudaStream_t s) {
-                    return conv_simt_launch(&va0, taps0, a1 >= 0 ? &va1 : nullptr, w, nn, bias ? bias + n0 : nullptr,
-                                            tb ? tb + n0 : nullptr, tb_stride, res >= 0 ? &r2 : nullptr, scale,
-                                            vout.ptr + n0, vout.ld, s);
+                if (c.res >= 0) r2.ptr += n0;
+                p.add(LK_GEMM, 2.0 * px * nn * (double)ktot, 0.0, [=](cudaStream_t s) {
+                    return conv_simt_launch(&va0, c.taps, c.shortcut >= 0 ? &va1 : nullptr, w, nn,
+                                            bias ? bias + n0 : nullptr, tb ? tb + n0 : nullptr, tb_stride,
+                                            c.res >= 0 ? &r2 : nullptr, c.scale, vout.ptr + n0, vout.ld, s);
                 });
             }
             return SNRSE_OK;
         }
-        const double px = (double)va0.B * va0.H * va0.W;
-        const double c0 = algo_cin > 0 ? algo_cin : va0.C;
-        const double kt = (double)taps0 * c0 + (a1 >= 0 ? va1.C : 0);
+        const double c0 = c.algo_cin > 0 ? c.algo_cin : va0.C;
+        const double kt = (double)c.taps * c0 + c1;
         // algorithmic bytes: each operand / result once (bf16), weights once
-        const double by = 2.0 * (px * (c0 + (a1 >= 0 ? va1.C : 0) + n_rows + (res >= 0 ? n_rows : 0)) + kt * n_rows);
-        if (conv_halo2_eligible(&va0, taps0, n_rows)) {   // 2-CTA (cta_group::2) halo kernel
+        const double by = 2.0 * (px * (c0 + c1 + c.n_rows + (c.res >= 0 ? c.n_rows : 0)) + kt * c.n_rows);
+        const ActView* a1 = c.shortcut >= 0 ? &va1 : nullptr;
+        const ActView* res = c.res >= 0 ? &vres : nullptr;
+        if (path == CONV_HALO2) {
             ConvHaloPlan hp;
-            SNRSE_TRY(conv_halo2_make_plan(&hp, &va0, a1 >= 0 ? &va1 : nullptr, e.wb(w_off), n_rows, bias, tb, tb_stride,
-                                           res >= 0 ? &vres : nullptr, scale, vout.ptr, vout.ld,
-                                           norm ? p.fptr(p.t_scsh) : nullptr, st >= 0 ? p.stat_ptr(st) : nullptr));
-            p.add(LK_GEMM, 2.0 * px * n_rows * kt, by, [hp](cudaStream_t s) { return conv_halo2_launch(&hp, s); });
+            SNRSE_TRY(conv_halo2_make_plan(&hp, &va0, a1, e.wb(c.w), c.n_rows, bias, tb, tb_stride, res, c.scale,
+                                           vout.ptr, vout.ld, c.norm ? p.fptr(p.t_scsh) : nullptr, p.stat_ptr(st)));
+            p.add(LK_GEMM, 2.0 * px * c.n_rows * kt, by, [hp](cudaStream_t s) { return conv_halo2_launch(&hp, s); });
             return SNRSE_OK;
         }
-        if (norm || st >= 0) {
-            snrse_set_error("internal: fused GroupNorm requested for a convolution the 2-CTA kernel cannot run");
-            return SNRSE_ERR_STATE;
-        }
         ConvGemmPlan g;
-        SNRSE_TRY(conv_gemm_make_plan(&g, &va0, taps0, a1 >= 0 ? &va1 : nullptr, e.wb(w_off), n_rows, 0, 0, bias, tb,
-                                      tb_stride, res >= 0 ? &vres : nullptr, scale, vout.ptr, vout.ld, 0));
-        p.add(LK_GEMM, 2.0 * px * n_rows * kt, by, [g](cudaStream_t s) { return conv_gemm_launch(&g, s); });
+        SNRSE_TRY(conv_gemm_make_plan(&g, &va0, c.taps, a1, e.wb(c.w), c.n_rows, 0, 0, bias, tb, tb_stride, res, c.scale,
+                                      vout.ptr, vout.ld, 0));
+        p.add(LK_GEMM, 2.0 * px * c.n_rows * kt, by, [g](cudaStream_t s) { return conv_gemm_launch(&g, s); });
         return SNRSE_OK;
     });
-    return out;
+    return c.out;
 }
 
 // Sums of tensor x for GroupNorm: accumulated by its writer when that was the 2-CTA convolution, otherwise by one
@@ -405,9 +442,7 @@ int get_stats(Plan& P, int x) {
     if (it != P.stats_of.end()) return it->second;
     const int st = P.n_stat_entries++;
     P.stats_of[x] = st;
-    P.use(x);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
+    P.record({x}, [=](Plan& p) -> int {
         const ActView vx = p.view(x);
         unsigned long long* dst = p.stat_ptr(st);
         const double el = (double)vx.B * vx.H * vx.W * vx.C;
@@ -431,9 +466,7 @@ void rec_gn_finalize(Plan& P, int x, int64_t g_off, int64_t b_off) {
         u0 = P.tens[x].C / 4;
     }
     const LT tx = P.tens[x];
-    P.use(P.t_scsh);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
+    P.record({P.t_scsh}, [=](Plan& p) -> int {
         Engine& e = *p.eng;
         const unsigned long long* a0 = p.stat_ptr(s0);
         const unsigned long long* a1 = s1 >= 0 ? p.stat_ptr(s1) : nullptr;
@@ -454,9 +487,7 @@ int rec_gn(Plan& P, int x, int64_t g_off, int64_t b_off, int silu) {
     rec_gn_finalize(P, x, g_off, b_off);
     const LT tx = P.tens[x];
     const int out = P.new_t(tx.B, tx.H, tx.W, tx.C, 2);
-    P.use(x); P.use(out); P.use(P.t_scsh);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
+    P.record({x, out, P.t_scsh}, [=](Plan& p) -> int {
         const ActView vx = p.view(x), vo = p.view(out);
         float* scsh = p.fptr(p.t_scsh);
         const double el = (double)vx.B * vx.H * vx.W * vx.C;
@@ -466,13 +497,12 @@ int rec_gn(Plan& P, int x, int64_t g_off, int64_t b_off, int silu) {
     return out;
 }
 
-// can the 2-CTA kernel run (and therefore normalise in flight) a 3x3 convolution on this tensor?
-bool fusable(const Plan& P, int x, int n_rows) {
-    if (P.flags & 2) return false;   // CUDA-core cross-check kernels
-    const LT& t = P.tens[x];
-    ActView v;
-    v.ptr = nullptr; v.B = t.B; v.H = t.H; v.W = t.W; v.C = t.C; v.ld = t.C;
-    return conv_halo2_eligible(&v, 9, n_rows);
+// GroupNorm + SiLU of x for the convolution that reads it: in flight (scale/shift into t_scsh, x stays the operand),
+// or as a pass of its own whose output is the operand
+int rec_gn_silu_operand(Plan& P, int x, int64_t g_off, int64_t b_off, bool in_flight) {
+    if (!in_flight) return rec_gn(P, x, g_off, b_off, 1);
+    rec_gn_finalize(P, x, g_off, b_off);
+    return x;
 }
 
 // a = FIR(silu(GroupNorm(x))) and xs = FIR(x) from ONE pass over x (scale/shift currently in t_scsh)
@@ -480,9 +510,7 @@ void rec_fir_dual(Plan& P, int x, int up, int* a, int* xs) {
     const LT tx = P.tens[x];
     const int on = up ? P.new_t(tx.B, tx.H * 2, tx.W * 2, tx.C, 2) : P.new_t(tx.B, tx.H / 2, tx.W / 2, tx.C, 2);
     const int orw = up ? P.new_t(tx.B, tx.H * 2, tx.W * 2, tx.C, 2) : P.new_t(tx.B, tx.H / 2, tx.W / 2, tx.C, 2);
-    P.use(x); P.use(on); P.use(orw); P.use(P.t_scsh);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
+    P.record({x, on, orw, P.t_scsh}, [=](Plan& p) -> int {
         const ActView vx = p.view(x), vn = p.view(on), vr = p.view(orw);
         const float* scsh = p.fptr(p.t_scsh);
         const double el = (double)vx.B * vx.H * vx.W * vx.C + 2.0 * vn.B * vn.H * vn.W * vn.C;
@@ -495,50 +523,39 @@ void rec_fir_dual(Plan& P, int x, int up, int* a, int* xs) {
 
 int rec_resblock(Plan& P, const Mod& m, int x) {
     // GroupNorm_0 + SiLU (+ FIR resampling of both branches) + Conv_0 + Dense_0(temb)
-    int a, xs = x, fuse0 = 0;
+    Conv c0{.w = m.w, .n_rows = m.cout, .bias = m.b, .tb_row = m.tb_row};
+    int xs = x;
     if (m.up || m.down) {
         // one dual-output FIR launch over x produces both branches; every row segment is staged in shared memory once,
         // raw and normalised, so x comes from DRAM once instead of three times and SiLU is evaluated once per element
-        rec_gn_finalize(P, x, m.o[0], m.o[1]);
-        rec_fir_dual(P, x, m.up ? 1 : 0, &a, &xs);
-    } else if (fusable(P, x, m.cout)) {
-        rec_gn_finalize(P, x, m.o[0], m.o[1]);   // normalisation itself happens inside Conv_0
-        a = x;
-        fuse0 = 1;
+        rec_gn_finalize(P, x, m.gn_g, m.gn_b);
+        rec_fir_dual(P, x, m.up ? 1 : 0, &c0.x, &xs);
     } else {
-        a = rec_gn(P, x, m.o[0], m.o[1], 1);
+        c0.norm = conv_path(P, P.tens[x].H, P.tens[x].W, 9, m.cout) == CONV_HALO2;
+        c0.x = rec_gn_silu_operand(P, x, m.gn_g, m.gn_b, c0.norm);
     }
-    const LT ta = P.tens[a];
-    const int h = P.new_t(ta.B, ta.H, ta.W, m.cout, 2);
-    // the 2-CTA kernel's epilogue also emits the GroupNorm partial sums of what it writes
-    const int stats0 = fusable(P, a, m.cout);
-    rec_gemm(P, a, 9, -1, m.o[2], m.cout, m.o[3], m.tb_row, -1, 1.0f, h, fuse0, stats0);
+    const LT ta = P.tens[c0.x];
+    c0.out = P.new_t(ta.B, ta.H, ta.W, m.cout, 2);
+    const int h = rec_conv(P, c0);
     // GroupNorm_1 + SiLU + Conv_1 (+ Conv_2 shortcut or identity residual), / sqrt(2)
-    int a2 = h, fuse1 = 0;
-    if (fusable(P, h, m.cout)) {
-        rec_gn_finalize(P, h, m.o[4], m.o[5]);
-        fuse1 = 1;
-    } else {
-        a2 = rec_gn(P, h, m.o[4], m.o[5], 1);
-    }
-    const int out = P.new_t(ta.B, ta.H, ta.W, m.cout, 2);
-    const int stats1 = fusable(P, a2, m.cout);
-    if (m.has_c2) rec_gemm(P, a2, 9, xs, m.o[6], m.cout, m.o[7], -1, -1, INV_SQRT2, out, fuse1, stats1);
-    else rec_gemm(P, a2, 9, -1, m.o[6], m.cout, m.o[7], -1, xs, INV_SQRT2, out, fuse1, stats1);
-    return out;
+    Conv c1{.w = m.w1, .n_rows = m.cout, .bias = m.b1, .scale = INV_SQRT2};
+    c1.norm = conv_path(P, P.tens[h].H, P.tens[h].W, 9, m.cout) == CONV_HALO2;
+    c1.x = rec_gn_silu_operand(P, h, m.gn1_g, m.gn1_b, c1.norm);
+    if (m.has_c2) c1.shortcut = xs;
+    else c1.res = xs;
+    c1.out = P.new_t(ta.B, ta.H, ta.W, m.cout, 2);
+    return rec_conv(P, c1);
 }
 
 int rec_attn(Plan& P, const Mod& m, int x) {
     const LT tx = P.tens[x];
     const int c = m.cin, n = tx.H * tx.W;
-    const int a = rec_gn(P, x, m.o[0], m.o[1], 0);
+    const int a = rec_gn(P, x, m.gn_g, m.gn_b, 0);
     const int qkv = P.new_t(tx.B, tx.H, tx.W, 3 * c, 2);
-    rec_gemm(P, a, 1, -1, m.o[2], 3 * c, m.o[3], -1, -1, 1.0f, qkv);
+    rec_conv(P, {.x = a, .taps = 1, .w = m.w, .n_rows = 3 * c, .bias = m.b, .out = qkv});
     const int sc = P.new_t(1, 1, 1, (int)((attention_workspace_bytes(tx.B, n, c) + 3) / 4), 4);   // scores | probabilities | V^T
     const int o = P.new_t(tx.B, tx.H, tx.W, c, 2);
-    P.use(qkv); P.use(sc); P.use(o);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
+    P.record({qkv, sc, o}, [=](Plan& p) -> int {
         const ActView vqkv = p.view(qkv), vo = p.view(o);
         ActView q = vqkv, k = vqkv, v = vqkv;
         q.C = k.C = v.C = c;
@@ -546,31 +563,17 @@ int rec_attn(Plan& P, const Mod& m, int x) {
         v.ptr += 2 * c;
         float* scores = p.fptr(sc);
         const double nn = (double)q.H * q.W;
-        const int tc = (p.flags & 2) ? 0 : 1;   // cross-check mode keeps the fp32 CUDA-core kernels
+        const int tc = p.cross_check ? 0 : 1;   // cross-check mode keeps the fp32 CUDA-core kernels
         p.add(LK_ATTN, 4.0 * q.B * nn * nn * c, 2.0 * q.B * nn * c * 4, [=](cudaStream_t s) { return attention_launch(&q, &k, &v, scores, &vo, s, tc); });
         return SNRSE_OK;
     });
     const int out = P.new_t(tx.B, tx.H, tx.W, c, 2);
-    rec_gemm(P, o, 1, -1, m.o[4], c, m.o[5], -1, x, INV_SQRT2, out);
-    return out;
+    return rec_conv(P, {.x = o, .taps = 1, .w = m.w1, .n_rows = c, .bias = m.b1, .res = x, .scale = INV_SQRT2, .out = out});
 }
 
-int record_plan(Plan& P) {
-    Engine& e = *P.eng;
-    const int B = P.B, F = P.F, T = P.T, L = e.n_levels, nf = e.nf;
-    P.t_x4 = P.new_t(B, F, T, 4, 4);
-    P.t_tb = P.new_t(B, 1, 1, e.dense_rows, 4);
-    P.t_tscr = P.new_t(B, 1, 1, 10 * nf, 4);   // act(temb) [4nf] | Fourier features [2nf] | hidden [4nf] per sample
-    P.t_stats = P.new_t(B, 1, 1, MAX_STAT_ENTRIES * 512, 4);   // statistics arena: entries of [B][128 units][2] x 8 bytes
-    P.t_scsh = P.new_t(B, 1, 1, 2 * 512, 4);
-    const int persistent[] = {P.t_x4, P.t_tb, P.t_tscr, P.t_stats, P.t_scsh};
-    size_t mi = 0;
-    // --- input packing + time embedding (+ the bf16 hi/lo operand of the tensor-core input convolution)
-    const int x64 = (P.flags & 2) ? -1 : P.new_t(B, F, T, 64, 2);
-    P.use(P.t_x4); P.use(P.t_tb); P.use(P.t_tscr);
-    if (x64 >= 0) P.use(x64);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
+// input packing + time embedding (+ the bf16 hi/lo operand x64 of the tensor-core input convolution, when x64 >= 0)
+void rec_pack_temb(Plan& P, int x64) {
+    P.record({P.t_x4, P.t_tb, P.t_tscr, x64}, [=](Plan& p) -> int {
         Engine& e = *p.eng;
         Plan* pp = &p;
         float* x4 = p.fptr(p.t_x4);
@@ -585,152 +588,87 @@ int record_plan(Plan& P) {
             SNRSE_CUDA(cudaMemsetAsync(stats0, 0, stats_bytes, s));   // GroupNorm sums are accumulated with atomics
             if (x64p) SNRSE_TRY(pack_input64_launch(pp->x_ptr, pp->y_ptr, x4, x64p, pp->B, n, s));
             else SNRSE_TRY(pack_input_launch(pp->x_ptr, pp->y_ptr, x4, pp->B, n, s));
-            return temb_launch(pp->t_ptr, pp->B, e.nf, e.wf(mf.o[0]), e.wf(m1.o[0]), e.wf(m1.o[1]), e.wf(m2.o[0]),
-                               e.wf(m2.o[1]), e.wf(e.dense_w_off), e.wf(e.dense_b_off), e.dense_rows, scr, tb, s);
+            return temb_launch(pp->t_ptr, pp->B, e.nf, e.wf(mf.w), e.wf(m1.w), e.wf(m1.b), e.wf(m2.w), e.wf(m2.b),
+                               e.wf(e.dense_w_off), e.wf(e.dense_b_off), e.dense_rows, scr, tb, s);
         });
         return SNRSE_OK;
     });
-    mi = 3;
-    // --- input conv 4 -> nf (ncsnpp.py:285): tensor cores on the 64-channel hi/lo operand, or fp32 CUDA cores (flag bit1)
-    int h = P.new_t(B, F, T, nf, 2);
-    if (x64 >= 0) {
-        const Mod m = e.mods[mi];
-        rec_gemm(P, x64, 9, -1, m.o[2], nf, m.o[1], -1, -1, 1.0f, h, 0, fusable(P, x64, nf) ? 1 : 0, /*algo_cin=*/4);
-        P.taps[(int)mi] = h;
-        ++mi;
-    } else {
-        const Mod m = e.mods[mi];
-        const int out = h;
-        P.use(P.t_x4); P.use(out);
-        P.step++;
-        P.builders.push_back([=](Plan& p) -> int {
-            Engine& e = *p.eng;
-            const ActView vo = p.view(out);
-            const float* x4 = p.fptr(p.t_x4);
-            const double px = (double)vo.B * vo.H * vo.W;
-            p.add(LK_THIN, 2.0 * px * 36 * vo.C, px * (16 + 2.0 * vo.C), [=, &e](cudaStream_t s) { return conv_in4_launch(x4, e.wf(m.o[0]), e.wf(m.o[1]), &vo, s); });
-            return SNRSE_OK;
+}
+
+// input conv 4 -> nf (ncsnpp.py:285): tensor cores on the 64-channel hi/lo operand x64, or fp32 CUDA cores on x4
+int rec_conv_in(Plan& P, const Mod& m, int x64) {
+    const int out = P.new_t(P.B, P.F, P.T, m.cout, 2);
+    if (x64 >= 0) return rec_conv(P, {.x = x64, .w = m.w_tc, .n_rows = m.cout, .bias = m.b, .out = out, .algo_cin = 4});
+    P.record({P.t_x4, out}, [=](Plan& p) -> int {
+        Engine& e = *p.eng;
+        const ActView vo = p.view(out);
+        const float* x4 = p.fptr(p.t_x4);
+        const double px = (double)vo.B * vo.H * vo.W;
+        p.add(LK_THIN, 2.0 * px * 36 * vo.C, px * (16 + 2.0 * vo.C), [=, &e](cudaStream_t s) { return conv_in4_launch(x4, e.wf(m.w), e.wf(m.b), &vo, s); });
+        return SNRSE_OK;
+    });
+    return out;
+}
+
+// input pyramid: FIR-downsample the 4-channel input *pyr, 1x1 conv 4->C, add to h (ncsnpp.py:310-311); *pyr becomes
+// the downsampled level
+int rec_combine(Plan& P, const Mod& m, int h, int* pyr) {
+    const int src = *pyr, ih = P.tens[src].H, iw = P.tens[src].W;
+    const int np = P.new_t(P.B, ih / 2, iw / 2, 4, 4);
+    const int out = P.new_t(P.B, ih / 2, iw / 2, m.cout, 2);
+    P.record({src, np, h, out}, [=](Plan& p) -> int {
+        Engine& e = *p.eng;
+        const float* sp = p.fptr(src);
+        float* dp = p.fptr(np);
+        const ActView vh = p.view(h), vo = p.view(out);
+        const double px = (double)vh.B * vh.H * vh.W;
+        p.add(LK_THIN, 2.0 * px * 4 * vh.C, px * (4.0 * vh.C + 16 + 64), [=, &e](cudaStream_t s) {
+            SNRSE_TRY(fir_down2_f4_launch(sp, dp, vh.B, ih, iw, s));
+            return combine4_launch(dp, &vh, e.wf(m.w), e.wf(m.b), &vo, s);
         });
-        P.taps[(int)mi] = h;
-        ++mi;
-    }
-    std::vector<int> hs{h};
-    int ipyr = P.t_x4, ipyr_h = F, ipyr_w = T;
-    for (int lv = 0; lv < L; ++lv) {
-        for (int b = 0; b < e.num_res_blocks; ++b) {
-            h = rec_resblock(P, e.mods[mi], hs.back());
-            P.taps[(int)mi] = h; ++mi;
-            if (in_list(e.attn_res, P.tens[h].H)) {
-                h = rec_attn(P, e.mods[mi], h);
-                P.taps[(int)mi] = h; ++mi;
-            }
-            hs.push_back(h);
-        }
-        if (lv != L - 1) {
-            h = rec_resblock(P, e.mods[mi], hs.back());
-            P.taps[(int)mi] = h; ++mi;
-            // input pyramid: FIR-downsample the 4-channel input, 1x1 conv 4->C, add (ncsnpp.py:310-311)
-            const int np = P.new_t(B, ipyr_h / 2, ipyr_w / 2, 4, 4);
-            const int out = P.new_t(B, ipyr_h / 2, ipyr_w / 2, e.mods[mi].cout, 2);
-            const Mod m = e.mods[mi];
-            const int src = ipyr, hin = h, ih = ipyr_h, iw = ipyr_w;
-            P.use(src); P.use(np); P.use(hin); P.use(out);
-            P.step++;
-            P.builders.push_back([=](Plan& p) -> int {
-                Engine& e = *p.eng;
-                const float* sp = p.fptr(src);
-                float* dp = p.fptr(np);
-                const ActView vh = p.view(hin), vo = p.view(out);
-                const double px = (double)vh.B * vh.H * vh.W;
-                p.add(LK_THIN, 2.0 * px * 4 * vh.C, px * (4.0 * vh.C + 16 + 64), [=, &e](cudaStream_t s) {
-                    SNRSE_TRY(fir_down2_f4_launch(sp, dp, vh.B, ih, iw, s));
-                    return combine4_launch(dp, &vh, e.wf(m.o[0]), e.wf(m.o[1]), &vo, s);
-                });
-                return SNRSE_OK;
+        return SNRSE_OK;
+    });
+    *pyr = np;
+    return out;
+}
+
+// GroupNorm + SiLU + conv3x3 C -> 4, added to the FIR-upsampled output pyramid prev (ncsnpp.py:348-366); returns the
+// new pyramid level.  On the 2-CTA tensor-core kernel with the normalisation in flight when the map is large enough,
+// CUDA cores otherwise.
+int rec_conv_out(Plan& P, const Mod& mg, const Mod& mc, int h, int prev) {
+    const LT th = P.tens[h];
+    const bool tc = conv_path(P, th.H, th.W, 9, 4) == CONV_HALO2;
+    const int a = rec_gn_silu_operand(P, h, mg.gn_g, mg.gn_b, tc);
+    const int np = P.new_t(th.B, th.H, th.W, 4, 4);
+    const int up = prev >= 0 ? P.new_t(th.B, th.H, th.W, 4, 4) : -1;
+    P.record({a, np, tc ? P.t_scsh : -1, prev, up}, [=](Plan& p) -> int {
+        Engine& e = *p.eng;
+        const ActView va = p.view(a);
+        float* dst = p.fptr(np);
+        float* upp = up >= 0 ? p.fptr(up) : nullptr;
+        const float* pv = prev >= 0 ? p.fptr(prev) : nullptr;
+        const double px = (double)va.B * va.H * va.W;
+        if (tc) {
+            ConvHaloPlan hp;
+            SNRSE_TRY(conv_halo2_make_plan_out4(&hp, &va, e.wb(mc.w_tc), e.wf(mc.b), upp, dst, p.fptr(p.t_scsh)));
+            p.add(LK_THIN, 2.0 * px * 36 * va.C, px * (2.0 * va.C + 16 + (pv ? 20 : 0)), [=](cudaStream_t s) {
+                if (pv) SNRSE_TRY(fir_up2_f4_launch(pv, upp, va.B, va.H / 2, va.W / 2, s));
+                return conv_halo2_launch(&hp, s);
             });
-            ipyr = np; ipyr_h /= 2; ipyr_w /= 2;
-            h = out;
-            P.taps[(int)mi] = h; ++mi;
-            hs.push_back(h);
+            return SNRSE_OK;
         }
-    }
-    h = hs.back();
-    h = rec_resblock(P, e.mods[mi], h); P.taps[(int)mi] = h; ++mi;
-    h = rec_attn(P, e.mods[mi], h); P.taps[(int)mi] = h; ++mi;
-    h = rec_resblock(P, e.mods[mi], h); P.taps[(int)mi] = h; ++mi;
-    int pyr = -1;
-    for (int lv = L - 1; lv >= 0; --lv) {
-        for (int b = 0; b < e.num_res_blocks + 1; ++b) {
-            const int cat = P.concat(h, hs.back());
-            hs.pop_back();
-            h = rec_resblock(P, e.mods[mi], cat);
-            P.taps[(int)mi] = h; ++mi;
-        }
-        if (in_list(e.attn_res, P.tens[h].H)) {
-            h = rec_attn(P, e.mods[mi], h);
-            P.taps[(int)mi] = h; ++mi;
-        }
-        {
-            const Mod mg = e.mods[mi], mc = e.mods[mi + 1];
-            // GroupNorm + SiLU + conv3x3 C -> 4, added to the FIR-upsampled pyramid (ncsnpp.py:348-366): on the 2-CTA
-            // tensor-core kernel with the normalisation in flight when the map is large enough, CUDA cores otherwise
-            const bool tc = fusable(P, h, 128);
-            int a = h;
-            if (tc) rec_gn_finalize(P, h, mg.o[0], mg.o[1]);
-            else a = rec_gn(P, h, mg.o[0], mg.o[1], 1);
-            const LT th = P.tens[h];
-            const int np = P.new_t(th.B, th.H, th.W, 4, 4);
-            int up = -1;
-            if (pyr >= 0) up = P.new_t(th.B, th.H, th.W, 4, 4);
-            const int prev = pyr;
-            P.use(a); P.use(np);
-            if (tc) P.use(P.t_scsh);
-            if (prev >= 0) { P.use(prev); P.use(up); }
-            P.step++;
-            P.builders.push_back([=](Plan& p) -> int {
-                Engine& e = *p.eng;
-                const ActView va = p.view(a);
-                float* dst = p.fptr(np);
-                float* upp = up >= 0 ? p.fptr(up) : nullptr;
-                const float* pv = prev >= 0 ? p.fptr(prev) : nullptr;
-                const double px = (double)va.B * va.H * va.W;
-                if (tc) {
-                    ConvHaloPlan hp;
-                    SNRSE_TRY(conv_halo2_make_plan_out4(&hp, &va, e.wb(mc.o[2]), e.wf(mc.o[1]), upp, dst, p.fptr(p.t_scsh)));
-                    p.add(LK_THIN, 2.0 * px * 36 * va.C, px * (2.0 * va.C + 16 + (pv ? 20 : 0)), [=](cudaStream_t s) {
-                        if (pv) SNRSE_TRY(fir_up2_f4_launch(pv, upp, va.B, va.H / 2, va.W / 2, s));
-                        return conv_halo2_launch(&hp, s);
-                    });
-                    return SNRSE_OK;
-                }
-                p.add(LK_THIN, 2.0 * px * 36 * va.C, px * (2.0 * va.C + 16 + (pv ? 20 : 0)), [=, &e](cudaStream_t s) {
-                    if (pv) SNRSE_TRY(fir_up2_f4_launch(pv, upp, va.B, va.H / 2, va.W / 2, s));
-                    return conv_out4_launch(&va, e.wf(mc.o[0]), e.wf(mc.o[1]), upp, dst, s);
-                });
-                return SNRSE_OK;
-            });
-            pyr = np;
-            P.taps[(int)mi + 1] = pyr;
-            mi += 2;
-        }
-        if (lv != 0) {
-            h = rec_resblock(P, e.mods[mi], h);
-            P.taps[(int)mi] = h; ++mi;
-        }
-    }
-    if (P.n_stat_entries > MAX_STAT_ENTRIES) {
-        snrse_set_error("internal: %d GroupNorm statistics entries exceed the arena (%d)", P.n_stat_entries, MAX_STAT_ENTRIES);
-        return SNRSE_ERR_STATE;
-    }
-    if (!hs.empty() || mi != e.mods.size()) {
-        snrse_set_error("internal: plan/topology mismatch (mi=%d of %d)", (int)mi, (int)e.mods.size());
-        return SNRSE_ERR_STATE;
-    }
-    // --- head: h / t, 1x1 conv 4->2, preconditioning (ncsnpp.py:398-403, model.py:488,537-541)
-    P.t_pyr_final = pyr;
-    P.use(pyr);
-    P.step++;
-    P.builders.push_back([=](Plan& p) -> int {
+        p.add(LK_THIN, 2.0 * px * 36 * va.C, px * (2.0 * va.C + 16 + (pv ? 20 : 0)), [=, &e](cudaStream_t s) {
+            if (pv) SNRSE_TRY(fir_up2_f4_launch(pv, upp, va.B, va.H / 2, va.W / 2, s));
+            return conv_out4_launch(&va, e.wf(mc.w), e.wf(mc.b), upp, dst, s);
+        });
+        return SNRSE_OK;
+    });
+    return np;
+}
+
+// head: h / t, 1x1 conv 4->2, preconditioning (ncsnpp.py:398-403, model.py:488,537-541)
+void rec_final(Plan& P, int pyr) {
+    P.record({pyr}, [=](Plan& p) -> int {
         Engine& e = *p.eng;
         Plan* pp = &p;
         const float* pf = p.fptr(pyr);
@@ -741,6 +679,64 @@ int record_plan(Plan& P) {
         });
         return SNRSE_OK;
     });
+}
+
+int record_plan(Plan& P) {
+    Engine& e = *P.eng;
+    const int B = P.B, F = P.F, T = P.T, L = e.n_levels, nf = e.nf;
+    P.t_x4 = P.new_t(B, F, T, 4, 4);
+    P.t_tb = P.new_t(B, 1, 1, e.dense_rows, 4);
+    P.t_tscr = P.new_t(B, 1, 1, 10 * nf, 4);   // act(temb) [4nf] | Fourier features [2nf] | hidden [4nf] per sample
+    P.t_stats = P.new_t(B, 1, 1, MAX_STAT_ENTRIES * 512, 4);   // statistics arena: entries of [B][128 units][2] x 8 bytes
+    P.t_scsh = P.new_t(B, 1, 1, 2 * 512, 4);
+    const int persistent[] = {P.t_x4, P.t_tb, P.t_tscr, P.t_stats, P.t_scsh};
+    // the tensor-core input convolution reads a 64-channel bf16 hi/lo copy of the input, written by the input packing
+    const int x64 = conv_path(P, F, T, 9, nf) == CONV_SIMT ? -1 : P.new_t(B, F, T, 64, 2);
+    rec_pack_temb(P, x64);   // modules 0-2: Fourier embedding and the two time-embedding layers
+    size_t mi = 3;
+    auto tap = [&](int t) {   // t is the output of module mi: keep it as the module's activation tap
+        P.taps[(int)mi++] = t;
+        return t;
+    };
+    int h = tap(rec_conv_in(P, e.mods[mi], x64));
+    std::vector<int> hs{h};
+    int ipyr = P.t_x4;
+    for (int lv = 0; lv < L; ++lv) {
+        for (int b = 0; b < e.num_res_blocks; ++b) {
+            h = tap(rec_resblock(P, e.mods[mi], hs.back()));
+            if (in_list(e.attn_res, P.tens[h].H)) h = tap(rec_attn(P, e.mods[mi], h));
+            hs.push_back(h);
+        }
+        if (lv != L - 1) {
+            h = tap(rec_resblock(P, e.mods[mi], hs.back()));
+            h = tap(rec_combine(P, e.mods[mi], h, &ipyr));
+            hs.push_back(h);
+        }
+    }
+    h = tap(rec_resblock(P, e.mods[mi], hs.back()));
+    h = tap(rec_attn(P, e.mods[mi], h));
+    h = tap(rec_resblock(P, e.mods[mi], h));
+    int pyr = -1;
+    for (int lv = L - 1; lv >= 0; --lv) {
+        for (int b = 0; b < e.num_res_blocks + 1; ++b) {
+            const int cat = P.concat(h, hs.back());
+            hs.pop_back();
+            h = tap(rec_resblock(P, e.mods[mi], cat));
+        }
+        if (in_list(e.attn_res, P.tens[h].H)) h = tap(rec_attn(P, e.mods[mi], h));
+        const Mod& gn = e.mods[mi++];   // the head's GroupNorm has no tap of its own
+        pyr = tap(rec_conv_out(P, gn, e.mods[mi], h, pyr));
+        if (lv != 0) h = tap(rec_resblock(P, e.mods[mi], h));
+    }
+    if (P.n_stat_entries > MAX_STAT_ENTRIES) {
+        snrse_set_error("internal: %d GroupNorm statistics entries exceed the arena (%d)", P.n_stat_entries, MAX_STAT_ENTRIES);
+        return SNRSE_ERR_STATE;
+    }
+    if (!hs.empty() || mi != e.mods.size()) {
+        snrse_set_error("internal: plan/topology mismatch (mi=%d of %d)", (int)mi, (int)e.mods.size());
+        return SNRSE_ERR_STATE;
+    }
+    rec_final(P, pyr);
     for (int id : persistent) { P.tens[id].first = 0; P.tens[id].last = 1 << 29; }
     if (P.flags & 1)
         for (auto& t : P.tens) t.last = 1 << 29;  // debug: keep every tensor alive (activation taps stay readable)
@@ -902,6 +898,7 @@ int64_t snrse_ncsnpp_plan_bytes(void* handle, int B, int F, int T, int flags) {
     if (!p) {
         p = new Plan();
         p->eng = e; p->B = B; p->F = F; p->T = T; p->flags = flags;
+        p->cross_check = (flags & 2) != 0;
         if (record_plan(*p) != SNRSE_OK) {
             delete p;
             return -1;

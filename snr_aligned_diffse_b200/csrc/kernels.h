@@ -70,8 +70,10 @@ struct ConvHaloPlan {
     float* out4;                  // 2-CTA kernel, thin C -> 4 output convolution only
     const float* addend4;
 };
-// 2-CTA (cta_group::2) single-halo-tile version, same plan structure (conv_halo2.cu): W >= 8, H >= 8
-bool conv_halo2_eligible(const ActView* a0, int taps0, int n_rows);
+// 2-CTA (cta_group::2) single-halo-tile version, same plan structure (conv_halo2.cu).  Its tiles need an H x W map with
+// W >= 8, H >= 8; conv_halo2_make_plan also needs a 3x3 convolution with N in {128, 256}.
+bool conv_halo2_fits(int H, int W);
+bool conv_halo2_eligible(int H, int W, int taps0, int n_rows);
 // scsh (nullable): GroupNorm scale/shift [B][2][C0] (gn_finalize_launch); when given, operand 0 is replaced by
 // silu(x*scale + shift) inside the kernel (GroupNorm+SiLU+conv3x3 of ResnetBlockBigGANpp without the HBM round trip).
 int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, const bf16* wt, int n_rows,

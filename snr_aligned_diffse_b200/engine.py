@@ -38,7 +38,6 @@ class NCSNppEngine:
         self.blob = None
         self.device = None
         self._ws = {}       # (B,F,T) -> (workspace tensor, flags)
-        self._graphs = {}
         self.weights_generation = 0    # bumped by every load_state_dict: tag for caches of captured CUDA graphs
 
     def __del__(self):
@@ -127,7 +126,6 @@ class NCSNppEngine:
         self.blob = self.pack_state_dict(sd).to(self.device)
         _lib.check(self.lib.snrse_ncsnpp_set_weights(self.h, _lib.ptr(self.blob)), "set_weights")
         self._ws.clear()
-        self._graphs.clear()
         self.weights_generation += 1
         return self
 
@@ -181,7 +179,6 @@ class NCSNppEngine:
         self.blob = blob.to(self.device)
         _lib.check(self.lib.snrse_ncsnpp_set_weights(self.h, _lib.ptr(self.blob)), "set_weights")
         self._ws.clear()
-        self._graphs.clear()
         self.weights_generation += 1
         return self
 
@@ -213,7 +210,6 @@ class NCSNppEngine:
         aligned = (base + 1023) // 1024 * 1024
         _lib.check(self.lib.snrse_ncsnpp_plan_bind(self.h, B, F, T, c_void_p(aligned), n), "plan_bind")
         self._ws[key] = (ws, flags)
-        self._graphs = {k: v for k, v in self._graphs.items() if k[:3] != key}
 
     def forward(self, x, y, t, mode=MODE_RAW, out=None, flags=0):
         """x, y: complex64 [B,F,T] (or [B,1,F,T]); t: float32 [B].  Enqueues on the current stream."""
