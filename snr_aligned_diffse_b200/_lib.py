@@ -69,6 +69,24 @@ PROTOTYPES = {
     "snrse_snrnet_forward": (i32, [vp, vp, vp, i32, i32, vp, vp]),
 }
 
+# every symbol declared in include/snrse_b200_layers.h (the executor's launchers, for the layer tests); snrse_view
+# arguments are passed by reference (ctypes.byref of a structure mirroring snrse_view)
+LAYER_PROTOTYPES = {
+    "snrse_dbg_conv": (i32, [vp, i32, vp, vp, i32, vp, vp, i32, vp, f32, vp, vp, vp, i32, vp]),
+    "snrse_dbg_gn_stats": (i32, [vp, vp, vp]),
+    "snrse_dbg_gn_finalize": (i32, [vp, i32, vp, i32, i32, i64, vp, vp, f32, vp, vp]),
+    "snrse_dbg_gn_apply": (i32, [vp, vp, i32, vp, vp]),
+    "snrse_dbg_fir": (i32, [vp, vp, i32, vp, vp]),
+    "snrse_dbg_fir_dual": (i32, [vp, vp, vp, i32, vp, vp]),
+    "snrse_dbg_conv_out4": (i32, [vp, vp, vp, vp, vp, vp, i32, vp]),
+    "snrse_dbg_pack_input": (i32, [vp, vp, vp, vp, i32, i64, vp]),
+    "snrse_dbg_conv_in4": (i32, [vp, vp, vp, vp, vp]),
+    "snrse_dbg_combine4": (i32, [vp, vp, vp, vp, vp, vp]),
+    "snrse_dbg_temb": (i32, [vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]),
+    "snrse_dbg_final": (i32, [vp, vp, vp, vp, vp, vp, i32, i64, i32, vp]),
+    "snrse_dbg_attention": (i32, [vp, vp, vp, vp, vp, i32, vp]),
+}
+
 
 def load():
     """Load the shared library (once).  Raises RuntimeError when it has not been built."""
@@ -80,7 +98,7 @@ def load():
             f"{LIB_PATH} is missing: build it with `python -m snr_aligned_diffse_b200.build` "
             "(nvcc, sm_100a).  This package has no CPU or PyTorch fallback.")
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (res, args) in PROTOTYPES.items():
+    for name, (res, args) in {**PROTOTYPES, **LAYER_PROTOTYPES}.items():
         fn = getattr(lib, name)  # AttributeError if the ABI and the header drifted apart
         fn.restype = res
         fn.argtypes = args

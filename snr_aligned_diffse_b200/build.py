@@ -34,6 +34,7 @@ def _newest_header():
     hs = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".h", ".cuh"))]
     hs.append(os.path.join(os.path.dirname(HERE), "include", "snrse_b200.h"))
     hs.append(os.path.join(os.path.dirname(HERE), "include", "snrse_b200_debug.h"))
+    hs.append(os.path.join(os.path.dirname(HERE), "include", "snrse_b200_layers.h"))
     return max(os.path.getmtime(h) for h in hs if os.path.exists(h))
 
 

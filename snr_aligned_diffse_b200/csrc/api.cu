@@ -269,3 +269,118 @@ extern "C" int snrse_fir_dual_nhwc(const void* x, const float* gamma, const floa
     SNRSE_TRY(gn_finalize_launch(ust, C / 4, nullptr, 0, B, (int64_t)H * W * (C / 32), gamma, beta, eps, scsh, S(stream)));
     return fir_dual_launch(&vx, &vn, &vr, up, scsh, S(stream));
 }
+
+// ---- the NCSN++ executor's launchers (include/snrse_b200_layers.h), one entry point each, on caller-made views
+// (channel slices of concatenation buffers, views into the fused qkv buffer).  Each converts its arguments and calls the
+// kernels.h launcher of the same name, so a test runs exactly the code the executor runs.
+struct snrse_view {
+    void* ptr;
+    int B, H, W, C, ld;
+};
+static_assert(sizeof(snrse_view) == sizeof(ActView), "snrse_view must mirror ActView");
+
+static ActView AV(const snrse_view* v) { return mk_view(v->ptr, v->B, v->H, v->W, v->C, v->ld); }
+
+extern "C" {
+
+// path 0: 2-CTA kernel, 1: CUDA cores, 2: single-CTA implicit GEMM.  scsh / ustats: 2-CTA kernel only.
+int snrse_dbg_conv(const snrse_view* x0, int taps0, const snrse_view* x1, const void* wt, int n, const float* bias,
+                   const float* tbias, int tb_stride, const snrse_view* res, float scale, const snrse_view* out,
+                   const float* scsh, void* ustats, int path, void* stream) {
+    SNRSE_CHECK_ARG(x0 && wt && out, "dbg_conv: null pointer");
+    SNRSE_CHECK_ARG(path == 0 || !(scsh || ustats), "dbg_conv: scsh / ustats need path 0");
+    const ActView a0 = AV(x0), a1 = x1 ? AV(x1) : ActView{}, r = res ? AV(res) : ActView{};
+    const ActView* pa1 = x1 ? &a1 : nullptr;
+    const ActView* pr = res ? &r : nullptr;
+    bf16* o = static_cast<bf16*>(out->ptr);
+    const bf16* w = static_cast<const bf16*>(wt);
+    if (path == 0) {
+        ConvHaloPlan hp;
+        SNRSE_TRY(conv_halo2_make_plan(&hp, &a0, pa1, w, n, bias, tbias, tb_stride, pr, scale, o, out->ld, scsh,
+                                       static_cast<unsigned long long*>(ustats)));
+        return conv_halo2_launch(&hp, S(stream));
+    }
+    if (path == 1) return conv_simt_launch(&a0, taps0, pa1, w, n, bias, tbias, tb_stride, pr, scale, o, out->ld, S(stream));
+    SNRSE_CHECK_ARG(path == 2, "dbg_conv: path must be 0, 1 or 2");
+    ConvGemmPlan g;
+    SNRSE_TRY(conv_gemm_make_plan(&g, &a0, taps0, pa1, w, n, 0, 0, bias, tbias, tb_stride, pr, scale, o, out->ld, 0));
+    return conv_gemm_launch(&g, S(stream));
+}
+
+int snrse_dbg_gn_stats(const snrse_view* x, void* ustats, void* stream) {
+    const ActView vx = AV(x);
+    return gn_stats_launch(&vx, static_cast<unsigned long long*>(ustats), S(stream));
+}
+
+int snrse_dbg_gn_finalize(const void* src0, int U0, const void* src1, int U1, int B, int64_t count, const float* gamma,
+                          const float* beta, float eps, float* scsh, void* stream) {
+    return gn_finalize_launch(static_cast<const unsigned long long*>(src0), U0, static_cast<const unsigned long long*>(src1),
+                              U1, B, count, gamma, beta, eps, scsh, S(stream));
+}
+
+int snrse_dbg_gn_apply(const snrse_view* x, const float* scsh, int silu, const snrse_view* out, void* stream) {
+    const ActView vx = AV(x), vo = AV(out);
+    return gn_apply_launch(&vx, scsh, silu, &vo, S(stream));
+}
+
+int snrse_dbg_fir(const snrse_view* x, const snrse_view* out, int up, const float* scsh, void* stream) {
+    const ActView vx = AV(x), vo = AV(out);
+    return up ? fir_up2_launch(&vx, &vo, S(stream), scsh) : fir_down2_launch(&vx, &vo, S(stream), scsh);
+}
+
+int snrse_dbg_fir_dual(const snrse_view* x, const snrse_view* out_n, const snrse_view* out_r, int up, const float* scsh,
+                       void* stream) {
+    const ActView vx = AV(x), vn = AV(out_n), vr = AV(out_r);
+    return fir_dual_launch(&vx, &vn, &vr, up, scsh, S(stream));
+}
+
+// path 0: 2-CTA kernel, bf16 weights [16][9C] (rows 4..15 unused); path 1: CUDA cores, fp32 weights [4][3][3][C], which
+// reads an operand that is already normalised (scsh must be null)
+int snrse_dbg_conv_out4(const snrse_view* a, const void* w, const float* bias, const float* addend4, float* out4,
+                        const float* scsh, int path, void* stream) {
+    const ActView va = AV(a);
+    if (path == 0) {
+        ConvHaloPlan hp;
+        SNRSE_TRY(conv_halo2_make_plan_out4(&hp, &va, static_cast<const bf16*>(w), bias, addend4, out4, scsh));
+        return conv_halo2_launch(&hp, S(stream));
+    }
+    SNRSE_CHECK_ARG(path == 1 && !scsh, "dbg_conv_out4: path 1 takes no scsh");
+    return conv_out4_launch(&va, static_cast<const float*>(w), bias, addend4, out4, S(stream));
+}
+
+// x64 null: pack_input_launch, otherwise pack_input64_launch
+int snrse_dbg_pack_input(const void* x, const void* y, float* x4, void* x64, int B, int64_t n, void* stream) {
+    if (!x64) return pack_input_launch(static_cast<const float2*>(x), static_cast<const float2*>(y), x4, B, n, S(stream));
+    return pack_input64_launch(static_cast<const float2*>(x), static_cast<const float2*>(y), x4, static_cast<bf16*>(x64), B,
+                               n, S(stream));
+}
+
+int snrse_dbg_conv_in4(const float* x4, const float* w, const float* bias, const snrse_view* out, void* stream) {
+    const ActView vo = AV(out);
+    return conv_in4_launch(x4, w, bias, &vo, S(stream));
+}
+
+int snrse_dbg_combine4(const float* p4, const snrse_view* h, const float* w, const float* bias, const snrse_view* out,
+                       void* stream) {
+    const ActView vh = AV(h), vo = AV(out);
+    return combine4_launch(p4, &vh, w, bias, &vo, S(stream));
+}
+
+int snrse_dbg_temb(const float* t, int B, int nf, const float* fourier_w, const float* w1, const float* b1, const float* w2,
+                   const float* b2, const float* dense_w, const float* dense_b, int rows, float* scratch, float* tb_out,
+                   void* stream) {
+    return temb_launch(t, B, nf, fourier_w, w1, b1, w2, b2, dense_w, dense_b, rows, scratch, tb_out, S(stream));
+}
+
+int snrse_dbg_final(const float* p4, const float* t, const float* w, const float* bias, const void* xres, void* out, int B,
+                    int64_t n, int mode, void* stream) {
+    return final_launch(p4, t, w, bias, static_cast<const float2*>(xres), static_cast<float2*>(out), B, n, mode, S(stream));
+}
+
+int snrse_dbg_attention(const snrse_view* q, const snrse_view* k, const snrse_view* v, void* workspace, const snrse_view* o,
+                        int allow_tensor_cores, void* stream) {
+    const ActView vq = AV(q), vk = AV(k), vv = AV(v), vo = AV(o);
+    return attention_launch(&vq, &vk, &vv, workspace, &vo, S(stream), allow_tensor_cores);
+}
+
+}  // extern "C"

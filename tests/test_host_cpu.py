@@ -32,6 +32,23 @@ def test_abi_exports_every_declared_symbol():
     assert lib.snrse_version() == 100
 
 
+def test_abi_exports_every_layer_entry_point():
+    """The executor's launchers as entry points (include/snrse_b200_layers.h): all exported, all in
+    _lib.LAYER_PROTOTYPES, none in the product ABI or the measurement header."""
+    from snr_aligned_diffse_b200 import _lib
+    found = lambda f: set(re.findall(r"\b(snrse_[a-z0-9_]+)\s*\(", open(os.path.join(ROOT, "include", f)).read()))  # noqa: E731
+    layers = found("snrse_b200_layers.h")
+    assert layers == {"snrse_dbg_conv", "snrse_dbg_gn_stats", "snrse_dbg_gn_finalize", "snrse_dbg_gn_apply",
+                      "snrse_dbg_fir", "snrse_dbg_fir_dual", "snrse_dbg_conv_out4", "snrse_dbg_pack_input",
+                      "snrse_dbg_conv_in4", "snrse_dbg_combine4", "snrse_dbg_temb", "snrse_dbg_final",
+                      "snrse_dbg_attention"}
+    assert not layers & (found("snrse_b200.h") | found("snrse_b200_debug.h"))
+    assert layers == set(_lib.LAYER_PROTOTYPES), layers ^ set(_lib.LAYER_PROTOTYPES)
+    lib = _lib.load()
+    for name in layers:
+        assert hasattr(lib, name), f"{name} declared in the header but not exported"
+
+
 def test_pdl_mask_round_trip():
     """snrse_set_pdl is host-only state: returns the previous mask, keeps three bits, a negative argument only queries."""
     from snr_aligned_diffse_b200 import _lib
