@@ -184,6 +184,14 @@ int64_t snrse_snrnet_weight_bytes(void);
 int64_t snrse_snrnet_workspace_bytes(int B, int T16);
 int snrse_snrnet_forward(const void* weights, const float* feat, float* out, int B, int T16, void* workspace,
                          void* stream);
+/* snrse_snrnet_forward on a ragged batch: the estimate of item b is SNRNet.forward of that utterance alone, i.e. over its
+ *   first clusters[b] 16-frame clusters (model.py:715-721 pads each file to its own multiple of 16 frames).
+ *   clusters: int32 [B] (device), read clamped to [1, T16/16]; NULL = every item has T16/16 clusters, which is
+ *   snrse_snrnet_forward.  Frames >= 16*clusters[b] of feat and the workspace rows of those clusters are never read.
+ *   Item b gives the same bits as a call with that utterance alone at T16 = 16*clusters[b]; one cluster gives NaN, as
+ *   the reference's unbiased std over one element.  Same feat layout and workspace size as snrse_snrnet_forward. */
+int snrse_snrnet_forward_varlen(const void* weights, const float* feat, const int* clusters, float* out, int B, int T16,
+                                void* workspace, void* stream);
 
 #ifdef __cplusplus
 }

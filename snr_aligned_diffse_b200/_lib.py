@@ -67,6 +67,7 @@ PROTOTYPES = {
     "snrse_snrnet_weight_bytes": (i64, []),
     "snrse_snrnet_workspace_bytes": (i64, [i32, i32]),
     "snrse_snrnet_forward": (i32, [vp, vp, vp, i32, i32, vp, vp]),
+    "snrse_snrnet_forward_varlen": (i32, [vp, vp, vp, vp, i32, i32, vp, vp]),
 }
 
 # every symbol declared in include/snrse_b200_layers.h (the executor's launchers, for the layer tests); snrse_view

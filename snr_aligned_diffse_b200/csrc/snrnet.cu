@@ -4,6 +4,9 @@
 // -> four (64 x k) convolutions, k = 1,2,4,8, each max-pooled over time -> 128 features; a BiLSTM(128->128)
 // runs over the clusters; [mean, unbiased std, min, max] over clusters -> Linear(1024->1) -> sigmoid.
 // ~1.2 MMAC per STFT frame (0.1 % of the score network): plain SIMT kernels, no tensor cores.
+// Ragged batches: every kernel takes an optional clusters[B] (the valid 16-frame clusters of each item, clamped to
+// [1, S]); the clusters of an item from there on are neither computed nor read, so item b gives the bits it gives when
+// run alone at T16 = 16 * clusters[b].  The layouts stay dense ([B][2][256][T16] features, B*S workspace rows).
 #include "kernels.h"
 
 namespace {
@@ -36,6 +39,22 @@ int64_t param_offset(int i) {  // bytes, 256-aligned slots
 }
 const float* P(const void* blob, int i) { return reinterpret_cast<const float*>(static_cast<const uint8_t*>(blob) + param_offset(i)); }
 
+// Valid clusters of item b.  Clamping keeps a bad value from moving any read outside the buffers.
+__device__ __forceinline__ int item_clusters(const int* __restrict__ clusters, int b, int S) {
+    return clusters ? min(max(clusters[b], 1), S) : S;
+}
+
+// Bit q set: workspace row nc0 + q (cluster (nc0 + q) % S of item (nc0 + q) / S) exists and is valid.
+__device__ __forceinline__ unsigned live_rows8(const int* __restrict__ clusters, int64_t nc0, int64_t ncl, int S) {
+    unsigned live = 0;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+        const int64_t nc = nc0 + q;
+        if (nc < ncl && (!clusters || (int)(nc % S) < item_clusters(clusters, (int)(nc / S), S))) live |= 1u << q;
+    }
+    return live;
+}
+
 __device__ __forceinline__ void cp_async4_zfill(float* smem_dst, const float* gsrc, bool valid) {
     // 4-byte asynchronous copy; !valid: nothing is read and the destination is zero-filled (src-size 0)
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc),
@@ -51,13 +70,14 @@ __device__ __forceinline__ void cp_async4_zfill(float* smem_dst, const float* gs
 constexpr int C5_TILES = 4;
 __global__ void __launch_bounds__(256)
 snr_conv5_pool_kernel(const float* __restrict__ feat, const float* __restrict__ w, const float* __restrict__ bias,
-                      float* __restrict__ a1, int T16) {
+                      float* __restrict__ a1, int T16, const int* __restrict__ clusters) {
     pdl_sync();
     __shared__ float sw[32 * 50];
     __shared__ float sbias[32];
     __shared__ float sxb[2][2 * 20 * 20];  // two stages of the input patch: 16 freq rows (+4 halo) x 16 frames (+4 halo)
-    const int nc = blockIdx.y, clusters = T16 / 16;
-    const int b = nc / clusters, cl = nc % clusters;
+    const int nc = blockIdx.y, S = T16 / 16;
+    const int b = nc / S, cl = nc % S;
+    if (cl >= item_clusters(clusters, b, S)) return;   // the whole block, before its first barrier
     auto load_tile = [&](int buf, int f0) {
         for (int i = threadIdx.x; i < 2 * 20 * 20; i += 256) {
             const int c = i / 400, r = (i / 20) % 20, t = i % 20;
@@ -124,12 +144,13 @@ constexpr int C3_SX = 32 * 18 * 10;
 constexpr int C3_SMEM = (32 * 9 * 32 + 2 * C3_SX) * 4;
 __global__ void __launch_bounds__(256)
 snr_conv3_pool_kernel(const float* __restrict__ a1, const float* __restrict__ w, const float* __restrict__ bias,
-                      float* __restrict__ a2) {
+                      float* __restrict__ a2, int S, const int* __restrict__ clusters) {
     pdl_sync();
     extern __shared__ __align__(16) float sm3[];
     float* sw = sm3;                       // [ci][k][co]   32*9*32 floats = 36 KB
     float* sxb = sm3 + 32 * 9 * 32;        // 2 x [ci][18][10]  2 x 23 KB
     const int nc = blockIdx.y, tile0 = blockIdx.x * C3_TILES;
+    if (nc % S >= item_clusters(clusters, nc / S, S)) return;   // the whole block, before its first barrier
     auto load_tile = [&](int buf, int f0) {
         float* dst = sxb + buf * C3_SX;
         for (int i = threadIdx.x; i < C3_SX; i += 256) {
@@ -202,7 +223,8 @@ snr_conv3_pool_kernel(const float* __restrict__ a1, const float* __restrict__ w,
 // ---- four (64 x k) convolutions + max over time.  a2 [NC][32][64][8] -> feats [NC][128]
 // Block = 8 clusters x one kernel width k; warp = cluster, lane = output channel.  Per 32-row chunk of the
 // (ci,f) axis the activations [8][32][8] and weights [32][k][32 co] are staged in shared memory; a lane keeps
-// the <= 8 output-frame accumulators of its channel.
+// the <= 8 output-frame accumulators of its channel.  A skipped cluster's stage is zero-filled instead of loaded and its
+// warp stores nothing.
 struct ConvtW {
     const float* w[4];
     const float* b[4];
@@ -216,7 +238,7 @@ constexpr int CONVT_SMEM = 2 * CONVT_STAGE * 4;            // two stages, 80 KB
 
 template <int K>   // kernel width in frames (1, 2, 4, 8): compile-time so that only the K * (9-K) useful FMAs per row are issued
 __device__ __forceinline__ void snr_convt_body(const float* __restrict__ a2, const float* __restrict__ wg,
-                                               const float* __restrict__ bg, float* __restrict__ feats, int64_t ncl, int ki,
+                                               const float* __restrict__ bg, float* __restrict__ feats, int ki, unsigned live,
                                                float* smem) {
     constexpr int NOUT = 9 - K;
     const int64_t nc0 = (int64_t)blockIdx.x * 8;
@@ -232,7 +254,7 @@ __device__ __forceinline__ void snr_convt_body(const float* __restrict__ a2, con
         for (int i = threadIdx.x; i < CONVT_SX / 4; i += 256) {     // per cluster 32 rows x 8 frames = 64 contiguous float4
             const int cl = i >> 6, q = i & 63;
             const int64_t nc = nc0 + cl;
-            if (nc < ncl) cp_async16(sx + cl * 256 + q * 4, a2 + nc * 16384 + (int64_t)r0 * 8 + q * 4);
+            if ((live >> cl) & 1) cp_async16(sx + cl * 256 + q * 4, a2 + nc * 16384 + (int64_t)r0 * 8 + q * 4);
             else *reinterpret_cast<float4*>(sx + cl * 256 + q * 4) = make_float4(0.f, 0.f, 0.f, 0.f);
         }
         // weights are pre-packed [r][dt][co]: the 32*K*32 floats of this chunk are one contiguous block
@@ -267,33 +289,39 @@ __device__ __forceinline__ void snr_convt_body(const float* __restrict__ a2, con
     float best = -INFINITY;
 #pragma unroll
     for (int t = 0; t < NOUT; ++t) best = fmaxf(best, acc[t]);
-    const int64_t nc = nc0 + warp;
-    if (nc < ncl) feats[nc * 128 + ki * 32 + lane] = best + bg[lane];
+    if ((live >> warp) & 1) feats[(nc0 + warp) * 128 + ki * 32 + lane] = best + bg[lane];
 }
 
 __global__ void __launch_bounds__(256)
-snr_convt_kernel(const float* __restrict__ a2, ConvtW cw, float* __restrict__ feats, int64_t ncl) {
+snr_convt_kernel(const float* __restrict__ a2, ConvtW cw, float* __restrict__ feats, int64_t ncl, int S,
+                 const int* __restrict__ clusters) {
     pdl_sync();
     extern __shared__ __align__(16) float convt_smem[];
+    const unsigned live = live_rows8(clusters, (int64_t)blockIdx.x * 8, ncl, S);
+    if (!live) return;                               // uniform over the block, before its first barrier
     const int ki = blockIdx.y;                       // weights packed [r (2048)][dt (k)][co (32)]
-    if (ki == 0) snr_convt_body<1>(a2, cw.w[0], cw.b[0], feats, ncl, 0, convt_smem);
-    else if (ki == 1) snr_convt_body<2>(a2, cw.w[1], cw.b[1], feats, ncl, 1, convt_smem);
-    else if (ki == 2) snr_convt_body<4>(a2, cw.w[2], cw.b[2], feats, ncl, 2, convt_smem);
-    else snr_convt_body<8>(a2, cw.w[3], cw.b[3], feats, ncl, 3, convt_smem);
+    if (ki == 0) snr_convt_body<1>(a2, cw.w[0], cw.b[0], feats, 0, live, convt_smem);
+    else if (ki == 1) snr_convt_body<2>(a2, cw.w[1], cw.b[1], feats, 1, live, convt_smem);
+    else if (ki == 2) snr_convt_body<4>(a2, cw.w[2], cw.b[2], feats, 2, live, convt_smem);
+    else snr_convt_body<8>(a2, cw.w[3], cw.b[3], feats, 3, live, convt_smem);
 }
 
 // ---- LSTM input projections for both directions: pre[dir][B*S][512] = W_ih x + b_ih + b_hh
-// Block = 8 rows (clusters); thread = 4 gate rows; a weight row is read once per 8 inputs.
+// Block = 8 rows (clusters); thread = 4 gate rows; a weight row is read once per 8 inputs.  Skipped clusters are
+// computed on zeros and not stored.
 __global__ void __launch_bounds__(256)
 snr_lstm_pre_kernel(const float* __restrict__ feats, const float* __restrict__ wih0, const float* __restrict__ bih0,
                     const float* __restrict__ bhh0, const float* __restrict__ wih1, const float* __restrict__ bih1,
-                    const float* __restrict__ bhh1, float* __restrict__ pre, int64_t rows) {
+                    const float* __restrict__ bhh1, float* __restrict__ pre, int64_t rows, int S,
+                    const int* __restrict__ clusters) {
     pdl_sync();
     __shared__ float sx[8][128];
     const int64_t row0 = (int64_t)blockIdx.x * 8;
+    const unsigned live = live_rows8(clusters, row0, rows, S);
+    if (!live) return;                               // uniform over the block, before its barrier
     for (int i = threadIdx.x; i < 8 * 128; i += 256) {
         const int64_t row = row0 + (i >> 7);
-        sx[i >> 7][i & 127] = row < rows ? feats[row * 128 + (i & 127)] : 0.f;
+        sx[i >> 7][i & 127] = ((live >> (i >> 7)) & 1) ? feats[row * 128 + (i & 127)] : 0.f;
     }
     __syncthreads();
     for (int o = threadIdx.x; o < 1024; o += 256) {
@@ -315,15 +343,16 @@ snr_lstm_pre_kernel(const float* __restrict__ feats, const float* __restrict__ w
         }
 #pragma unroll
         for (int q = 0; q < 8; ++q)
-            if (row0 + q < rows) pre[((int64_t)dir * rows + row0 + q) * 512 + g] = acc[q];
+            if ((live >> q) & 1) pre[((int64_t)dir * rows + row0 + q) * 512 + g] = acc[q];
     }
 }
 
 // ---- recurrence: one block per (batch item, direction); thread g owns gate row g of W_hh
-// (64 weights in registers, 64 in shared memory).  Gate order i, f, g, o (torch.nn.LSTM).
+// (64 weights in registers, 64 in shared memory).  Gate order i, f, g, o (torch.nn.LSTM).  The forward direction runs
+// over clusters 0 .. Sb-1, the reverse one from Sb-1 down to 0 (Sb = the item's valid clusters).
 __global__ void __launch_bounds__(512, 1)
 snr_lstm_rec_kernel(const float* __restrict__ pre, const float* __restrict__ whh0, const float* __restrict__ whh1,
-                    float* __restrict__ hout, int S, int64_t rows) {
+                    float* __restrict__ hout, int S, int64_t rows, const int* __restrict__ clusters) {
     pdl_sync();
     extern __shared__ float sm[];
     float* sw = sm;                  // [64][512]  second half of every W_hh row, transposed
@@ -337,9 +366,10 @@ snr_lstm_rec_kernel(const float* __restrict__ pre, const float* __restrict__ whh
     for (int j = 0; j < 64; ++j) sw[j * 512 + g] = wr[64 + j];
     if (g < 128) sh[g] = 0.f;
     float c = 0.f;
+    const int Sb = item_clusters(clusters, b, S);
     __syncthreads();
-    for (int step = 0; step < S; ++step) {
-        const int s = dir ? S - 1 - step : step;
+    for (int step = 0; step < Sb; ++step) {
+        const int s = dir ? Sb - 1 - step : step;
         float acc = pre[((int64_t)dir * rows + (int64_t)b * S + s) * 512 + g];
 #pragma unroll
         for (int j = 0; j < 64; ++j) acc = fmaf(wreg[j], sh[j], acc);
@@ -361,27 +391,28 @@ snr_lstm_rec_kernel(const float* __restrict__ pre, const float* __restrict__ whh
     }
 }
 
-// ---- [mean, unbiased std, min, max] over clusters -> fc -> sigmoid
+// ---- [mean, unbiased std, min, max] over the item's valid clusters -> fc -> sigmoid
 __global__ void __launch_bounds__(256)
 snr_head_kernel(const float* __restrict__ hout, const float* __restrict__ fcw, const float* __restrict__ fcb,
-                float* __restrict__ out, int S) {
+                float* __restrict__ out, int S, const int* __restrict__ clusters) {
     pdl_sync();
     __shared__ float red[8];
     const int b = blockIdx.x, j = threadIdx.x;
+    const int Sb = item_clusters(clusters, b, S);
     float sum = 0.f, mn = INFINITY, mx = -INFINITY;
-    for (int s = 0; s < S; ++s) {
+    for (int s = 0; s < Sb; ++s) {
         const float v = hout[((int64_t)b * S + s) * 256 + j];
         sum += v;
         mn = fminf(mn, v);
         mx = fmaxf(mx, v);
     }
-    const float mean = sum / (float)S;
+    const float mean = sum / (float)Sb;
     float ss = 0.f;
-    for (int s = 0; s < S; ++s) {
+    for (int s = 0; s < Sb; ++s) {
         const float d = hout[((int64_t)b * S + s) * 256 + j] - mean;
         ss = fmaf(d, d, ss);
     }
-    const float sd = sqrtf(ss / (float)(S - 1));  // S == 1 -> NaN, as torch.std (snrnet.py:84)
+    const float sd = sqrtf(ss / (float)(Sb - 1));  // Sb == 1 -> NaN, as torch.std (snrnet.py:84)
     float acc = mean * fcw[j] + sd * fcw[256 + j] + mn * fcw[512 + j] + mx * fcw[768 + j];
     acc = warp_sum(acc);
     if ((j & 31) == 0) red[j >> 5] = acc;
@@ -427,8 +458,8 @@ int64_t snrse_snrnet_workspace_bytes(int B, int T16) {
     return nc * (32768 + 16384 + 128 + 1024 + 256) * 4;
 }
 
-int snrse_snrnet_forward(const void* weights, const float* feat, float* out, int B, int T16, void* workspace,
-                         void* stream) {
+int snrse_snrnet_forward_varlen(const void* weights, const float* feat, const int* clusters, float* out, int B, int T16,
+                                void* workspace, void* stream) {
     SNRSE_CHECK_ARG(weights && feat && out && workspace, "snrnet_forward: null pointer");
     SNRSE_CHECK_ARG(B > 0 && T16 > 0 && T16 % 16 == 0, "snrnet_forward: T must be a positive multiple of 16");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -447,26 +478,31 @@ int snrse_snrnet_forward(const void* weights, const float* feat, float* out, int
         SNRSE_CUDA(cudaFuncSetAttribute(snr_convt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, CONVT_SMEM));
         attr_set = true;
     }
-    snrse_launch(snr_conv5_pool_kernel, dim3(dim3(16 / C5_TILES, (unsigned)nc)), dim3(256), 0, s, feat, P(weights, 0), P(weights, 1), a1, T16);
+    snrse_launch(snr_conv5_pool_kernel, dim3(dim3(16 / C5_TILES, (unsigned)nc)), dim3(256), 0, s, feat, P(weights, 0), P(weights, 1), a1, T16, clusters);
     SNRSE_LAUNCH_CHECK();
     snrse_launch(snr_conv3_pool_kernel, dim3(dim3(128 / (C3_ROWS * C3_TILES), (unsigned)nc)), dim3(256), C3_SMEM, s, 
-        a1, P(weights, 2), P(weights, 3), a2);
+        a1, P(weights, 2), P(weights, 3), a2, S, clusters);
     SNRSE_LAUNCH_CHECK();
     ConvtW cw;
     for (int i = 0; i < 4; ++i) {
         cw.w[i] = P(weights, 4 + 2 * i);
         cw.b[i] = P(weights, 5 + 2 * i);
     }
-    snrse_launch(snr_convt_kernel, dim3(dim3((unsigned)cdiv64(nc, 8), 4)), dim3(256), CONVT_SMEM, s, a2, cw, feats, nc);
+    snrse_launch(snr_convt_kernel, dim3(dim3((unsigned)cdiv64(nc, 8), 4)), dim3(256), CONVT_SMEM, s, a2, cw, feats, nc, S, clusters);
     SNRSE_LAUNCH_CHECK();
     snrse_launch(snr_lstm_pre_kernel, dim3((unsigned)cdiv64(nc, 8)), dim3(256), 0, s, feats, P(weights, 12), P(weights, 14), P(weights, 15), P(weights, 16),
-                                                     P(weights, 18), P(weights, 19), pre, nc);
+                                                     P(weights, 18), P(weights, 19), pre, nc, S, clusters);
     SNRSE_LAUNCH_CHECK();
-    snrse_launch(snr_lstm_rec_kernel, dim3(dim3(B, 2)), dim3(512), (64 * 512 + 128 + 512) * 4, s, pre, P(weights, 13), P(weights, 17), hout, S, nc);
+    snrse_launch(snr_lstm_rec_kernel, dim3(dim3(B, 2)), dim3(512), (64 * 512 + 128 + 512) * 4, s, pre, P(weights, 13), P(weights, 17), hout, S, nc, clusters);
     SNRSE_LAUNCH_CHECK();
-    snrse_launch(snr_head_kernel, dim3(B), dim3(256), 0, s, hout, P(weights, 20), P(weights, 21), out, S);
+    snrse_launch(snr_head_kernel, dim3(B), dim3(256), 0, s, hout, P(weights, 20), P(weights, 21), out, S, clusters);
     SNRSE_LAUNCH_CHECK();
     return SNRSE_OK;
+}
+
+int snrse_snrnet_forward(const void* weights, const float* feat, float* out, int B, int T16, void* workspace,
+                         void* stream) {
+    return snrse_snrnet_forward_varlen(weights, feat, nullptr, out, B, T16, workspace, stream);
 }
 
 }  // extern "C"

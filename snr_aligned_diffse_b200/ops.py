@@ -335,15 +335,26 @@ class SNRNetEngine:
         self.blob = blob.to(device)
         return self
 
-    def forward(self, feat):
-        """feat f32 [B,2,256,T16] cuda -> [B] = noise/(speech+noise)."""
+    def forward(self, feat, clusters=None):
+        """feat f32 [B,2,256,T16] cuda -> [B] = noise/(speech+noise).  clusters: optional int32 [B] cuda, the valid
+        16-frame clusters of each item (read clamped to [1, T16/16]); item b is then estimated over its first
+        clusters[b] clusters only, as if it had been run alone at T16 = 16 * clusters[b]."""
         assert self.blob is not None and feat.is_cuda and feat.dtype == torch.float32
         feat = feat.contiguous()
         B, _, _, T16 = feat.shape
+        if clusters is not None and not (torch.is_tensor(clusters) and clusters.device == feat.device
+                                         and clusters.dtype == torch.int32 and clusters.numel() == B):
+            raise ValueError(f"snrnet forward: clusters must be an int32 tensor of {B} elements on {feat.device}")
+        clusters = None if clusters is None else clusters.contiguous()
         ws = torch.empty(int(self.lib.snrse_snrnet_workspace_bytes(B, T16)), dtype=torch.uint8, device=feat.device)
         out = torch.empty(B, dtype=torch.float32, device=feat.device)
-        _lib.check(self.lib.snrse_snrnet_forward(_lib.ptr(self.blob), _lib.ptr(feat), _lib.ptr(out), B, T16, _lib.ptr(ws),
-                                                 _lib.stream_ptr()), "snrnet_forward")
+        if clusters is None:
+            _lib.check(self.lib.snrse_snrnet_forward(_lib.ptr(self.blob), _lib.ptr(feat), _lib.ptr(out), B, T16,
+                                                     _lib.ptr(ws), _lib.stream_ptr()), "snrnet_forward")
+        else:
+            _lib.check(self.lib.snrse_snrnet_forward_varlen(_lib.ptr(self.blob), _lib.ptr(feat),
+                                                            _lib.ptr(clusters), _lib.ptr(out), B, T16,
+                                                            _lib.ptr(ws), _lib.stream_ptr()), "snrnet_forward_varlen")
         return out
 
     def noise_over_clean(self, g):

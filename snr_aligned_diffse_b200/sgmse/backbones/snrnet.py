@@ -23,15 +23,18 @@ class SNRNet:
     def state_dict(self):
         return dict(self._sd or {})
 
-    def forward(self, x):
-        """x [B,2,256,T] float32, T % 16 == 0 -> [B,1]."""
+    def forward(self, x, clusters=None):
+        """x [B,2,256,T] float32, T % 16 == 0 -> [B,1].  clusters: optional int32 [B], the number of valid 16-frame
+        clusters of each item (see `SNRNetEngine.forward`); None runs every item over all T/16 clusters."""
         if self._sd is None:
             raise RuntimeError("SNRNet has no weights")
         if self._dirty:
             self.engine.load_state_dict({"dnn." + k: v for k, v in self._sd.items()}, "cuda")
             self._dirty = False
         dev = x.device
-        out = self.engine.forward(x if x.is_cuda else x.cuda())
+        xg = x if x.is_cuda else x.cuda()
+        cg = None if clusters is None else clusters.to(xg.device, torch.int32)
+        out = self.engine.forward(xg, cg)
         return out[:, None].to(dev)
 
     __call__ = forward
