@@ -162,10 +162,6 @@ int snrse_fir_f4(const float* x, float* out, int B, int H, int W, int up, void* 
 int snrse_upfirdn2d(const float* input, const float* kernel, float* out, int64_t major, int in_h, int in_w, int kernel_h,
                     int kernel_w, int up_x, int up_y, int down_x, int down_y, int pad_x0, int pad_x1, int pad_y0, int pad_y1,
                     void* stream);
-/* FIR resampling of silu(GroupNorm32(x)), normalisation applied on load (layerspp.py:245-257); workspace:
- * snrse_groupnorm_workspace_bytes(B) */
-int snrse_gn_silu_fir_nhwc(const void* x, const float* gamma, const float* beta, float eps, void* out, int B, int H, int W,
-                           int C, int up, void* workspace, void* stream);
 /* softmax(q k^T / sqrt(C)) v over n positions (ncsnpp_utils/layerspp.py:84-88); workspace:
  * snrse_attention_workspace_bytes(B, n, C) (fp32 scores, bf16 probabilities, V^T).  Tensor cores when n % 64 == 0. */
 int64_t snrse_attention_workspace_bytes(int B, int n, int C);

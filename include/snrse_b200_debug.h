@@ -1,9 +1,8 @@
 /* snrse_b200_debug.h -- measurement and debugging entry points of libsnrse_b200.so.
  *
  * NOT part of the drop-in ABI (snrse_b200.h): nothing in the product path calls these.  They exist for bench.py's
- * roofline record (per-launch-group CUDA-event timing), the parity tests (per-module activation taps, the executor's
- * dual-output FIR pass as an operator) and the kernel-tuning tools under tools/ (cycle counters of the convolution
- * kernels).  Same conventions as snrse_b200.h.
+ * roofline record (per-launch-group CUDA-event timing), the parity tests (per-module activation taps) and the
+ * kernel-tuning tools under tools/ (cycle counters of the convolution kernels).  Same conventions as snrse_b200.h.
  */
 #ifndef SNRSE_B200_DEBUG_H
 #define SNRSE_B200_DEBUG_H
@@ -28,11 +27,6 @@ int snrse_ncsnpp_read_tap(void* handle, int B, int F, int T, int module_idx, flo
 /* cycle counters of the convolution kernels: [grid][8] int64 (a / b / accumulator waits of the MMA warp, total,
  * epilogue wait / body, producer waits), filled by every later launch; NULL switches them off */
 void snrse_conv_halo_set_debug(long long* dev_counters);
-/* the dual-output FIR pass of the up / down residual blocks as one operator (NHWC bf16, x [B][H][W][C]):
- * out_n = FIR(silu(GroupNorm(32, eps)(x))), out_r = FIR(x), both [B][2H][2W][C] (up) or [B][H/2][W/2][C] (down);
- * workspace: the size snrse_groupnorm_workspace_bytes gives for B, as for snrse_gn_silu_fir_nhwc */
-int snrse_fir_dual_nhwc(const void* x, const float* gamma, const float* beta, float eps, void* out_n, void* out_r, int B,
-                        int H, int W, int C, int up, void* workspace, void* stream);
 
 #ifdef __cplusplus
 }

@@ -35,8 +35,10 @@ int snrse_dbg_gn_stats(const snrse_view* x, void* ustats, void* stream);
 int snrse_dbg_gn_finalize(const void* src0, int U0, const void* src1, int U1, int B, int64_t count, const float* gamma,
                           const float* beta, float eps, float* scsh, void* stream);
 int snrse_dbg_gn_apply(const snrse_view* x, const float* scsh, int silu, const snrse_view* out, void* stream);
-/* FIR x2 resampling (scsh non-null: of silu(x*scale + shift)) and the dual-output pass of the up / down blocks */
-int snrse_dbg_fir(const snrse_view* x, const snrse_view* out, int up, const float* scsh, void* stream);
+/* the stand-alone single-output FIR x2 resampling (snrse_fir_nhwc's launcher; the executor does not launch it), kept as
+ * the reference the dual pass is compared with, and the dual-output pass of the up / down blocks:
+ * out_n = FIR(silu(x*scale + shift)), out_r = FIR(x) */
+int snrse_dbg_fir(const snrse_view* x, const snrse_view* out, int up, void* stream);
 int snrse_dbg_fir_dual(const snrse_view* x, const snrse_view* out_n, const snrse_view* out_r, int up, const float* scsh,
                        void* stream);
 /* C -> 4 output head, out4 [B][H][W][4] f32 = conv3x3(a) + bias (+ addend4): path 0 2-CTA kernel, w bf16 [16][9C]

@@ -50,7 +50,6 @@ PROTOTYPES = {
     "snrse_ncsnpp_read_tap": (i32, [vp, i32, i32, i32, i32, vp, i64, POINTER(i64), vp]),
     "snrse_conv_nhwc": (i32, [vp, i32, i32, vp, i32, vp, i32, vp, vp, i32, vp, f32, vp, i32, i32, i32, i32, vp]),
     "snrse_conv_halo_set_debug": (None, [vp]),
-    "snrse_fir_dual_nhwc": (i32, [vp, vp, vp, f32, vp, vp, i32, i32, i32, i32, i32, vp, vp]),
     "snrse_gn_silu_conv3x3_nhwc": (i32, [vp, i32, vp, vp, f32, vp, i32, vp, i32, vp, vp, i32, vp, f32, vp, i32, i32, i32, vp, vp]),
     "snrse_conv3x3_nhwc_stats": (i32, [vp, i32, vp, i32, vp, i32, vp, vp, i32, vp, f32, vp, i32, i32, i32, vp, vp]),
     "snrse_groupnorm_workspace_bytes": (i64, [i32]),
@@ -58,7 +57,6 @@ PROTOTYPES = {
     "snrse_fir_nhwc": (i32, [vp, vp, i32, i32, i32, i32, i32, vp]),
     "snrse_fir_f4": (i32, [vp, vp, i32, i32, i32, i32, vp]),
     "snrse_upfirdn2d": (i32, [vp, vp, vp, i64] + [i32] * 12 + [vp]),
-    "snrse_gn_silu_fir_nhwc": (i32, [vp, vp, vp, f32, vp, i32, i32, i32, i32, i32, vp, vp]),
     "snrse_attention_workspace_bytes": (i64, [i32, i32, i32]),
     "snrse_attention_nhwc": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, vp]),
     "snrse_snrnet_num_params": (i32, []),
@@ -77,7 +75,7 @@ LAYER_PROTOTYPES = {
     "snrse_dbg_gn_stats": (i32, [vp, vp, vp]),
     "snrse_dbg_gn_finalize": (i32, [vp, i32, vp, i32, i32, i64, vp, vp, f32, vp, vp]),
     "snrse_dbg_gn_apply": (i32, [vp, vp, i32, vp, vp]),
-    "snrse_dbg_fir": (i32, [vp, vp, i32, vp, vp]),
+    "snrse_dbg_fir": (i32, [vp, vp, i32, vp]),
     "snrse_dbg_fir_dual": (i32, [vp, vp, vp, i32, vp, vp]),
     "snrse_dbg_conv_out4": (i32, [vp, vp, vp, vp, vp, vp, i32, vp]),
     "snrse_dbg_pack_input": (i32, [vp, vp, vp, vp, i32, i64, vp]),
@@ -100,9 +98,11 @@ def load():
             "(nvcc, sm_100a).  This package has no CPU or PyTorch fallback.")
     lib = ctypes.CDLL(LIB_PATH)
     for name, (res, args) in {**PROTOTYPES, **LAYER_PROTOTYPES}.items():
-        fn = getattr(lib, name)  # AttributeError if the ABI and the header drifted apart
-        fn.restype = res
-        fn.argtypes = args
+        # one flag per parameter makes a call with more arguments than the prototype a TypeError; a plain ctypes
+        # function would pass the extra ones on, e.g. a stale argument list's pointer in place of the stream.
+        # AttributeError if the ABI and the header drifted apart.
+        proto = ctypes.CFUNCTYPE(res, *args)
+        setattr(lib, name, proto((name, lib), tuple((1,) for _ in args)) if args else proto((name, lib)))
     _lib = lib
     return lib
 

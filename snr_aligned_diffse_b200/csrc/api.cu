@@ -31,6 +31,18 @@ static ActView mk_view(const void* p, int B, int H, int W, int C, int ld) {
     return v;
 }
 
+// GroupNorm(32, eps) statistics and scale/shift of x in a workspace of snrse_groupnorm_workspace_bytes(B): the unit sums
+// [B][128][2] (zeroed here) first, then the scale/shift [B][2][C] that *scsh points to.
+static int gn_scale_shift(const ActView* x, const float* gamma, const float* beta, float eps, void* workspace,
+                          cudaStream_t s, float** scsh) {
+    unsigned long long* ust = static_cast<unsigned long long*>(workspace);
+    *scsh = reinterpret_cast<float*>(ust + (int64_t)x->B * 128 * 2);
+    SNRSE_CUDA(cudaMemsetAsync(ust, 0, (size_t)x->B * (x->C / 4) * 16, s));
+    SNRSE_TRY(gn_stats_launch(x, ust, s));
+    return gn_finalize_launch(ust, x->C / 4, nullptr, 0, x->B, (int64_t)x->H * x->W * (x->C / 32), gamma, beta, eps,
+                              *scsh, s);
+}
+
 extern "C" {
 
 int snrse_version(void) { return 100; }
@@ -168,12 +180,8 @@ int snrse_groupnorm_nhwc(const void* x, const float* gamma, const float* beta, v
                          int silu, float eps, void* workspace, void* stream) {
     SNRSE_CHECK_ARG(x && gamma && beta && out && workspace, "groupnorm: null pointer");
     const ActView vx = mk_view(x, B, H, W, C, C), vo = mk_view(out, B, H, W, C, C);
-    unsigned long long* ust = static_cast<unsigned long long*>(workspace);
-    float* scsh = reinterpret_cast<float*>(ust + (int64_t)B * 128 * 2);
-    const int64_t hw = (int64_t)H * W;
-    SNRSE_CUDA(cudaMemsetAsync(ust, 0, (size_t)B * (C / 4) * 16, S(stream)));
-    SNRSE_TRY(gn_stats_launch(&vx, ust, S(stream)));
-    SNRSE_TRY(gn_finalize_launch(ust, C / 4, nullptr, 0, B, hw * (C / 32), gamma, beta, eps, scsh, S(stream)));
+    float* scsh;
+    SNRSE_TRY(gn_scale_shift(&vx, gamma, beta, eps, workspace, S(stream), &scsh));
     return gn_apply_launch(&vx, scsh, silu, &vo, S(stream));
 }
 
@@ -189,12 +197,8 @@ int snrse_gn_silu_conv3x3_nhwc(const void* x0, int c0, const float* gamma, const
     if (x1) a1 = mk_view(x1, B, H, W, c1, c1);
     if (res) r = mk_view(res, B, H, W, n, n);
     SNRSE_CHECK_ARG(conv_halo2_eligible(a0.H, a0.W, 9, n), "gn_silu_conv3x3: needs W >= 8, H >= 8, N in {128, 256}");
-    unsigned long long* ust = static_cast<unsigned long long*>(workspace);
-    float* scsh = reinterpret_cast<float*>(ust + (int64_t)B * 128 * 2);
-    const int64_t hw = (int64_t)H * W;
-    SNRSE_CUDA(cudaMemsetAsync(ust, 0, (size_t)B * (c0 / 4) * 16, S(stream)));
-    SNRSE_TRY(gn_stats_launch(&a0, ust, S(stream)));
-    SNRSE_TRY(gn_finalize_launch(ust, c0 / 4, nullptr, 0, B, hw * (c0 / 32), gamma, beta, eps, scsh, S(stream)));
+    float* scsh;
+    SNRSE_TRY(gn_scale_shift(&a0, gamma, beta, eps, workspace, S(stream), &scsh));
     ConvHaloPlan hp;
     SNRSE_TRY(conv_halo2_make_plan(&hp, &a0, x1 ? &a1 : nullptr, static_cast<const bf16*>(wt), n, bias, tbias, tb_stride,
                                    res ? &r : nullptr, scale, static_cast<bf16*>(out), n, scsh, nullptr));
@@ -206,21 +210,6 @@ int snrse_fir_nhwc(const void* x, void* out, int B, int H, int W, int C, int up,
     const ActView vx = mk_view(x, B, H, W, C, C);
     const ActView vo = up ? mk_view(out, B, 2 * H, 2 * W, C, C) : mk_view(out, B, H / 2, W / 2, C, C);
     return up ? fir_up2_launch(&vx, &vo, S(stream)) : fir_down2_launch(&vx, &vo, S(stream));
-}
-
-// FIR resampling of silu(GroupNorm(x)) with the normalisation applied on load (ResnetBlockBigGANpp up / down blocks,
-// ncsnpp_utils/layerspp.py:245-257).  workspace: snrse_groupnorm_workspace_bytes(B).
-int snrse_gn_silu_fir_nhwc(const void* x, const float* gamma, const float* beta, float eps, void* out, int B, int H, int W,
-                           int C, int up, void* workspace, void* stream) {
-    SNRSE_CHECK_ARG(x && gamma && beta && out && workspace, "gn_silu_fir: null pointer");
-    const ActView vx = mk_view(x, B, H, W, C, C);
-    const ActView vo = up ? mk_view(out, B, 2 * H, 2 * W, C, C) : mk_view(out, B, H / 2, W / 2, C, C);
-    unsigned long long* ust = static_cast<unsigned long long*>(workspace);
-    float* scsh = reinterpret_cast<float*>(ust + (int64_t)B * 128 * 2);
-    SNRSE_CUDA(cudaMemsetAsync(ust, 0, (size_t)B * (C / 4) * 16, S(stream)));
-    SNRSE_TRY(gn_stats_launch(&vx, ust, S(stream)));
-    SNRSE_TRY(gn_finalize_launch(ust, C / 4, nullptr, 0, B, (int64_t)H * W * (C / 32), gamma, beta, eps, scsh, S(stream)));
-    return up ? fir_up2_launch(&vx, &vo, S(stream), scsh) : fir_down2_launch(&vx, &vo, S(stream), scsh);
 }
 
 int snrse_upfirdn2d(const float* input, const float* kernel, float* out, int64_t major, int in_h, int in_w, int kernel_h,
@@ -253,22 +242,6 @@ int snrse_attention_nhwc(const void* q, const void* k, const void* v, void* scor
 long long* g_halo_dbg_shared = nullptr;
 // device buffer of [grid][8] cycle counters filled by subsequent conv_halo2 / conv_gemm launches (null: off)
 extern "C" void snrse_conv_halo_set_debug(long long* dev_counters) { g_halo_dbg_shared = dev_counters; }
-
-// The dual-output FIR pass of the NCSN++ up / down residual blocks on its own: out_n = FIR(silu(GroupNorm(x))),
-// out_r = FIR(x).  workspace: snrse_groupnorm_workspace_bytes(B).
-extern "C" int snrse_fir_dual_nhwc(const void* x, const float* gamma, const float* beta, float eps, void* out_n, void* out_r,
-                                   int B, int H, int W, int C, int up, void* workspace, void* stream) {
-    SNRSE_CHECK_ARG(x && gamma && beta && out_n && out_r && workspace, "fir_dual: null pointer");
-    const ActView vx = mk_view(x, B, H, W, C, C);
-    const int oh = up ? 2 * H : H / 2, ow = up ? 2 * W : W / 2;
-    const ActView vn = mk_view(out_n, B, oh, ow, C, C), vr = mk_view(out_r, B, oh, ow, C, C);
-    unsigned long long* ust = static_cast<unsigned long long*>(workspace);
-    float* scsh = reinterpret_cast<float*>(ust + (int64_t)B * 128 * 2);
-    SNRSE_CUDA(cudaMemsetAsync(ust, 0, (size_t)B * (C / 4) * 16, S(stream)));
-    SNRSE_TRY(gn_stats_launch(&vx, ust, S(stream)));
-    SNRSE_TRY(gn_finalize_launch(ust, C / 4, nullptr, 0, B, (int64_t)H * W * (C / 32), gamma, beta, eps, scsh, S(stream)));
-    return fir_dual_launch(&vx, &vn, &vr, up, scsh, S(stream));
-}
 
 // ---- the NCSN++ executor's launchers (include/snrse_b200_layers.h), one entry point each, on caller-made views
 // (channel slices of concatenation buffers, views into the fused qkv buffer).  Each converts its arguments and calls the
@@ -323,9 +296,10 @@ int snrse_dbg_gn_apply(const snrse_view* x, const float* scsh, int silu, const s
     return gn_apply_launch(&vx, scsh, silu, &vo, S(stream));
 }
 
-int snrse_dbg_fir(const snrse_view* x, const snrse_view* out, int up, const float* scsh, void* stream) {
+// not launched by the executor: the stand-alone single-output FIR that the dual pass is compared with
+int snrse_dbg_fir(const snrse_view* x, const snrse_view* out, int up, void* stream) {
     const ActView vx = AV(x), vo = AV(out);
-    return up ? fir_up2_launch(&vx, &vo, S(stream), scsh) : fir_down2_launch(&vx, &vo, S(stream), scsh);
+    return up ? fir_up2_launch(&vx, &vo, S(stream)) : fir_down2_launch(&vx, &vo, S(stream));
 }
 
 int snrse_dbg_fir_dual(const snrse_view* x, const snrse_view* out_n, const snrse_view* out_r, int up, const float* scsh,

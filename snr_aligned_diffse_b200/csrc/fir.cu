@@ -19,36 +19,6 @@ __device__ __forceinline__ V8 ld8(const bf16* p) {
     return r;
 }
 
-// Optional GroupNorm + SiLU on load (ResnetBlockBigGANpp up / down blocks: h = FIR(silu(GroupNorm(x))),
-// layerspp.py:245-257): the loaders apply y = silu(x*scale + shift) with the per-(sample, channel) scale/shift of
-// gn_finalize; positions outside the image contribute zero (the FIR pads the NORMALISED tensor).  Same arithmetic as
-// gn_apply_kernel followed by a bf16 round trip, so fusing does not change a bit.
-struct Norm8 {
-    float sc[8], sh[8];
-    bool on;
-};
-__device__ __forceinline__ Norm8 load_norm(const float* __restrict__ scsh, int b, int C, int c0) {
-    Norm8 n;
-    n.on = scsh != nullptr;
-    if (n.on) {
-        const float4* a = reinterpret_cast<const float4*>(scsh + ((int64_t)b * 2) * C + c0);
-        const float4* c = reinterpret_cast<const float4*>(scsh + ((int64_t)b * 2 + 1) * C + c0);
-        const float4 a0 = __ldg(a), a1 = __ldg(a + 1), c0v = __ldg(c), c1 = __ldg(c + 1);
-        n.sc[0] = a0.x; n.sc[1] = a0.y; n.sc[2] = a0.z; n.sc[3] = a0.w; n.sc[4] = a1.x; n.sc[5] = a1.y; n.sc[6] = a1.z; n.sc[7] = a1.w;
-        n.sh[0] = c0v.x; n.sh[1] = c0v.y; n.sh[2] = c0v.z; n.sh[3] = c0v.w; n.sh[4] = c1.x; n.sh[5] = c1.y; n.sh[6] = c1.z; n.sh[7] = c1.w;
-    }
-    return n;
-}
-// unpack 8 bf16 and, when enabled, normalise + SiLU + round to bf16 (what the separate pass would have stored)
-template <bool NORM>
-__device__ __forceinline__ void unpack_norm(const uint4& raw, const Norm8& n, bool inside, float* f) {
-    unpack8(raw, f);
-    if (NORM && inside) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) f[j] = __bfloat162float(__float2bfloat16(silu_f(fmaf(f[j], n.sc[j], n.sh[j]))));
-    }
-}
-
 // Both bf16 kernels are separable and walk a band of rows with a sliding window in registers: thread = (column,
 // 8-channel chunk); every input row is filtered horizontally once (3 or 4 loads, neighbours shared through L1)
 // and reused by the two output rows it contributes to, so the kernels move ~1x the tensor instead of issuing
@@ -61,29 +31,24 @@ __device__ __forceinline__ void zero8(float* a) {
 }
 
 // raw 16-byte loads of the 4 input columns around output column wo of input row hh (zero outside the image)
-// returns the mask of columns that lie inside the image
-__device__ __forceinline__ int load_row_down(const bf16* __restrict__ img, int ld, int H, int W, int hh, int wo, int c0,
-                                             uint4* raw) {
+__device__ __forceinline__ void load_row_down(const bf16* __restrict__ img, int ld, int H, int W, int hh, int wo, int c0,
+                                              uint4* raw) {
     const bool row_ok = hh >= 0 && hh < H;
     const bf16* row = img + (int64_t)(row_ok ? hh : 0) * W * ld + c0;
-    int mask = 0;
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
         const int ww = 2 * wo - 1 + t;
         const bool ok = row_ok && ww >= 0 && ww < W;
         raw[t] = ok ? __ldg(reinterpret_cast<const uint4*>(row + (int64_t)ww * ld)) : make_uint4(0, 0, 0, 0);
-        mask |= ok ? (1 << t) : 0;
     }
-    return mask;
 }
 // horizontal [1,3,3,1]/8
-template <bool NORM>
-__device__ __forceinline__ void hfilt_down(const uint4* raw, int mask, const Norm8& nm, float* r) {
+__device__ __forceinline__ void hfilt_down(const uint4* raw, float* r) {
     float f0[8], f1[8], f2[8], f3[8];
-    unpack_norm<NORM>(raw[0], nm, mask & 1, f0);
-    unpack_norm<NORM>(raw[1], nm, (mask >> 1) & 1, f1);
-    unpack_norm<NORM>(raw[2], nm, (mask >> 2) & 1, f2);
-    unpack_norm<NORM>(raw[3], nm, (mask >> 3) & 1, f3);
+    unpack8(raw[0], f0);
+    unpack8(raw[1], f1);
+    unpack8(raw[2], f2);
+    unpack8(raw[3], f3);
 #pragma unroll
     for (int j = 0; j < 8; ++j) r[j] = fmaf(0.125f, f3[j], fmaf(0.375f, f2[j], fmaf(0.375f, f1[j], fmaf(0.125f, f0[j], 0.f))));
 }
@@ -94,9 +59,8 @@ __device__ __forceinline__ void load_row_down_fast(const bf16* __restrict__ p, i
     for (int t = 0; t < 4; ++t) raw[t] = __ldg(reinterpret_cast<const uint4*>(p + (int64_t)t * ld));
 }
 
-template <bool NORM>
 __device__ __forceinline__ void fir_down2_body(const bf16* __restrict__ x, int ld, int C, int H, int W, bf16* __restrict__ out,
-                                               int out_ld, int band, const float* __restrict__ scsh) {
+                                               int out_ld, int band) {
     const int tpp = C >> 3, cols = blockDim.x / tpp;
     const int c0 = (threadIdx.x % tpp) * 8;
     const int Ho = H >> 1, Wo = W >> 1;
@@ -106,34 +70,30 @@ __device__ __forceinline__ void fir_down2_body(const bf16* __restrict__ x, int l
     const bf16* img = x + (int64_t)b * H * W * ld;
     const int ho0 = blockIdx.y * band;
     const int ho1 = min(ho0 + band, Ho);
-    const Norm8 nm = load_norm(scsh, b, C, c0);
     // columns 2wo-1 .. 2wo+2 all inside the image: rows inside the image need no bounds logic at all
     const bool col_in = wo > 0 && 2 * wo + 2 < W;
     const int64_t rstride = (int64_t)W * ld;
     const bf16* pcol = img + (int64_t)(2 * wo - 1) * ld + c0;   // column 2wo-1 of row 0 (only dereferenced when col_in)
-    auto load_row = [&](int hh, uint4* raw) -> int {
-        if (col_in && hh >= 0 && hh < H) {
-            load_row_down_fast(pcol + hh * rstride, ld, raw);
-            return 15;
-        }
-        return load_row_down(img, ld, H, W, hh, wo, c0, raw);
+    auto load_row = [&](int hh, uint4* raw) {
+        if (col_in && hh >= 0 && hh < H) load_row_down_fast(pcol + hh * rstride, ld, raw);
+        else load_row_down(img, ld, H, W, hh, wo, c0, raw);
     };
     float r0[8], r1[8], r2[8], r3[8];   // horizontally filtered rows 2ho-1 .. 2ho+2
     uint4 ra[4], rb[4];
-    int ma = load_row(2 * ho0 - 1, ra);
-    int mb = load_row(2 * ho0, rb);
-    hfilt_down<NORM>(ra, ma, nm, r0);
-    hfilt_down<NORM>(rb, mb, nm, r1);
-    ma = load_row(2 * ho0 + 1, ra);   // the two new rows of the first output row
-    mb = load_row(2 * ho0 + 2, rb);
+    load_row(2 * ho0 - 1, ra);
+    load_row(2 * ho0, rb);
+    hfilt_down(ra, r0);
+    hfilt_down(rb, r1);
+    load_row(2 * ho0 + 1, ra);   // the two new rows of the first output row
+    load_row(2 * ho0 + 2, rb);
     bf16* op = out + (((int64_t)b * Ho + ho0) * Wo + wo) * out_ld + c0;
     const int64_t ostride = (int64_t)Wo * out_ld;
     for (int ho = ho0; ho < ho1; ++ho, op += ostride) {
-        hfilt_down<NORM>(ra, ma, nm, r2);
-        hfilt_down<NORM>(rb, mb, nm, r3);
+        hfilt_down(ra, r2);
+        hfilt_down(rb, r3);
         if (ho + 1 < ho1) {   // next output row's loads are in flight while this one is finished
-            ma = load_row(2 * ho + 3, ra);
-            mb = load_row(2 * ho + 4, rb);
+            load_row(2 * ho + 3, ra);
+            load_row(2 * ho + 4, rb);
         }
         float o[8];
 #pragma unroll
@@ -145,34 +105,32 @@ __device__ __forceinline__ void fir_down2_body(const bf16* __restrict__ x, int l
 }
 
 // horizontal interpolation of input row hh at input column wi: ea -> output column 2wi, eb -> 2wi+1
-template <bool NORM>
-__device__ __forceinline__ void hfilt_up(const bf16* __restrict__ img, int ld, int H, int W, int hh, int wi, int c0,
-                                         const Norm8& nm, float* ea, float* eb) {
+__device__ __forceinline__ void hfilt_up(const bf16* __restrict__ img, int ld, int H, int W, int hh, int wi, int c0, float* ea,
+                                         float* eb) {
     zero8(ea);
     zero8(eb);
     if (hh < 0 || hh >= H) return;
     const bf16* row = img + (int64_t)hh * W * ld + c0;
     float m[8];
-    unpack_norm<NORM>(__ldg(reinterpret_cast<const uint4*>(row + (int64_t)wi * ld)), nm, true, m);
+    unpack8(__ldg(reinterpret_cast<const uint4*>(row + (int64_t)wi * ld)), m);
 #pragma unroll
     for (int j = 0; j < 8; ++j) { ea[j] = 0.75f * m[j]; eb[j] = 0.75f * m[j]; }
     if (wi > 0) {
         float l[8];
-        unpack_norm<NORM>(__ldg(reinterpret_cast<const uint4*>(row + (int64_t)(wi - 1) * ld)), nm, true, l);
+        unpack8(__ldg(reinterpret_cast<const uint4*>(row + (int64_t)(wi - 1) * ld)), l);
 #pragma unroll
         for (int j = 0; j < 8; ++j) ea[j] = fmaf(0.25f, l[j], ea[j]);
     }
     if (wi + 1 < W) {
         float rr[8];
-        unpack_norm<NORM>(__ldg(reinterpret_cast<const uint4*>(row + (int64_t)(wi + 1) * ld)), nm, true, rr);
+        unpack8(__ldg(reinterpret_cast<const uint4*>(row + (int64_t)(wi + 1) * ld)), rr);
 #pragma unroll
         for (int j = 0; j < 8; ++j) eb[j] = fmaf(0.25f, rr[j], eb[j]);
     }
 }
 
-template <bool NORM>
 __device__ __forceinline__ void fir_up2_body(const bf16* __restrict__ x, int ld, int C, int H, int W, bf16* __restrict__ out,
-                                             int out_ld, int band, const float* __restrict__ scsh) {
+                                             int out_ld, int band) {
     const int tpp = C >> 3, cols = blockDim.x / tpp;
     const int c0 = (threadIdx.x % tpp) * 8;
     const int wi = blockIdx.x * cols + threadIdx.x / tpp;
@@ -184,11 +142,10 @@ __device__ __forceinline__ void fir_up2_body(const bf16* __restrict__ x, int ld,
     const int h0 = blockIdx.y * band;
     const int h1 = min(h0 + band, H);
     float pa[8], pb[8], ca[8], cb[8], na[8], nb[8];   // rows hi-1, hi, hi+1 (a: even output column, b: odd)
-    const Norm8 nm = load_norm(scsh, b, C, c0);
-    hfilt_up<NORM>(img, ld, H, W, h0 - 1, wi, c0, nm, pa, pb);
-    hfilt_up<NORM>(img, ld, H, W, h0, wi, c0, nm, ca, cb);
+    hfilt_up(img, ld, H, W, h0 - 1, wi, c0, pa, pb);
+    hfilt_up(img, ld, H, W, h0, wi, c0, ca, cb);
     for (int hi = h0; hi < h1; ++hi) {
-        hfilt_up<NORM>(img, ld, H, W, hi + 1, wi, c0, nm, na, nb);
+        hfilt_up(img, ld, H, W, hi + 1, wi, c0, na, nb);
         float o[8];
         bf16* r_even = oimg + ((int64_t)(2 * hi) * Wo + 2 * wi) * out_ld;
         bf16* r_odd = r_even + (int64_t)Wo * out_ld;
@@ -209,29 +166,47 @@ __device__ __forceinline__ void fir_up2_body(const bf16* __restrict__ x, int ld,
     }
 }
 
-template <bool NORM>
 __global__ void __launch_bounds__(256)
-fir_down2_kernel(const bf16* __restrict__ x, int ld, int C, int H, int W, bf16* __restrict__ out, int out_ld, int band,
-                 const float* __restrict__ scsh) {
+fir_down2_kernel(const bf16* __restrict__ x, int ld, int C, int H, int W, bf16* __restrict__ out, int out_ld, int band) {
     pdl_sync();
-    fir_down2_body<NORM>(x, ld, C, H, W, out, out_ld, band, scsh);
+    fir_down2_body(x, ld, C, H, W, out, out_ld, band);
 }
-template <bool NORM>
 __global__ void __launch_bounds__(256)
-fir_up2_kernel(const bf16* __restrict__ x, int ld, int C, int H, int W, bf16* __restrict__ out, int out_ld, int band,
-               const float* __restrict__ scsh) {
+fir_up2_kernel(const bf16* __restrict__ x, int ld, int C, int H, int W, bf16* __restrict__ out, int out_ld, int band) {
     pdl_sync();
-    fir_up2_body<NORM>(x, ld, C, H, W, out, out_ld, band, scsh);
+    fir_up2_body(x, ld, C, H, W, out, out_ld, band);
 }
 
 // ---- dual-output variants for the up / down residual blocks (layerspp.py:245-257): the block filters BOTH
 // h = silu(GroupNorm(x)) and the raw x with the same FIR.  One launch produces FIR(h) and FIR(x) from ONE pass over x:
 // every input row segment of the block (its columns + halo, all channels) is staged in shared memory once, raw and
 // normalised (silu(x*scale + shift) rounded to bf16 -- what the separate GroupNorm pass would have stored), and both
-// filters read their taps from there.  Each element is loaded and normalised once per block (the single-output kernels
-// with the normalisation on load evaluate SiLU 2x (down) / 3x (up) per element and are issue-bound on it).  Against the
-// three-pass form (gn_apply: read x, write h; FIR: read h; FIR: read x) the DRAM traffic per element of x drops from
-// 3 reads + 1 write (+ outputs) to 1 read (+ outputs).  Same arithmetic and rounding points: bit-identical results.
+// filters read their taps from there.  Rows are staged so that each element is normalised once per block: neighbouring
+// output columns share input columns, so normalising the taps as they are loaded would evaluate SiLU 2x (down) / 3x (up)
+// per element.  Against the three-pass form (gn_apply: read x, write h; FIR: read h; FIR: read x) the DRAM traffic per
+// element of x drops from 3 reads + 1 write (+ outputs) to 1 read (+ outputs).  Same arithmetic and rounding points:
+// bit-identical results.
+
+// GroupNorm scale / shift of one 8-channel chunk (per (sample, channel), from gn_finalize)
+struct Norm8 {
+    float sc[8], sh[8];
+};
+__device__ __forceinline__ Norm8 load_norm(const float* __restrict__ scsh, int b, int C, int c0) {
+    Norm8 n;
+    const float4* a = reinterpret_cast<const float4*>(scsh + ((int64_t)b * 2) * C + c0);
+    const float4* c = reinterpret_cast<const float4*>(scsh + ((int64_t)b * 2 + 1) * C + c0);
+    const float4 a0 = __ldg(a), a1 = __ldg(a + 1), c0v = __ldg(c), c1 = __ldg(c + 1);
+    n.sc[0] = a0.x; n.sc[1] = a0.y; n.sc[2] = a0.z; n.sc[3] = a0.w; n.sc[4] = a1.x; n.sc[5] = a1.y; n.sc[6] = a1.z; n.sc[7] = a1.w;
+    n.sh[0] = c0v.x; n.sh[1] = c0v.y; n.sh[2] = c0v.z; n.sh[3] = c0v.w; n.sh[4] = c1.x; n.sh[5] = c1.y; n.sh[6] = c1.z; n.sh[7] = c1.w;
+    return n;
+}
+// unpack 8 bf16, normalise + SiLU and round to bf16: the same arithmetic as gn_apply_kernel and its bf16 store
+__device__ __forceinline__ void unpack_norm(const uint4& raw, const Norm8& n, float* f) {
+    unpack8(raw, f);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) f[j] = __bfloat162float(__float2bfloat16(silu_f(fmaf(f[j], n.sc[j], n.sh[j]))));
+}
+
 // Staging is split in two so that the global loads of the NEXT rows are in flight while the current rows are filtered:
 // fir_stage_load issues up to MAXI 16-byte loads of a row segment into registers (nothing depends on them yet),
 // fir_stage_store normalises them and writes the raw and the normalised copy to shared memory.
@@ -267,7 +242,7 @@ __device__ __forceinline__ void fir_stage_store(const StageRegs<MAXI>& r, int nc
             uint4 nr = make_uint4(0, 0, 0, 0);
             if ((r.ok >> i) & 1u) {
                 float f[8];
-                unpack_norm<true>(r.raw[i], nm, true, f);
+                unpack_norm(r.raw[i], nm, f);
                 nr = pack8(f);                     // already bf16 values: exact
             }
             s_raw[col * tpp + chunk] = r.raw[i];
@@ -584,7 +559,7 @@ int upfirdn2d_launch(const float* x, const float* kernel, float* out, int64_t ma
     return SNRSE_OK;
 }
 
-int fir_down2_launch(const ActView* x, const ActView* out, cudaStream_t s, const float* scsh) {
+int fir_down2_launch(const ActView* x, const ActView* out, cudaStream_t s) {
     SNRSE_CHECK_ARG(x->H % 2 == 0 && x->W % 2 == 0 && x->C % 8 == 0, "fir_down2: H, W must be even, C %% 8 == 0");
     SNRSE_CHECK_ARG(x->C <= 2048 && x->B <= 65535, "fir_down2: C <= 2048, B <= 65535");
     const int tpp = x->C / 8, nthr = tpp * (256 / tpp > 0 ? 256 / tpp : 1), cols = nthr / tpp;
@@ -592,21 +567,19 @@ int fir_down2_launch(const ActView* x, const ActView* out, cudaStream_t s, const
     int band = FIR_BAND;
     while (band > 1 && (int64_t)cdiv(x->W / 2, cols) * cdiv(x->H / 2, band) * x->B < 592) band >>= 1;
     dim3 grid((unsigned)cdiv(x->W / 2, cols), (unsigned)cdiv(x->H / 2, band), (unsigned)x->B);
-    if (scsh) snrse_launch(fir_down2_kernel<true>, dim3(grid), dim3(nthr), 0, s, x->ptr, x->ld, x->C, x->H, x->W, out->ptr, out->ld, band, scsh);
-    else snrse_launch(fir_down2_kernel<false>, dim3(grid), dim3(nthr), 0, s, x->ptr, x->ld, x->C, x->H, x->W, out->ptr, out->ld, band, scsh);
+    snrse_launch(fir_down2_kernel, dim3(grid), dim3(nthr), 0, s, x->ptr, x->ld, x->C, x->H, x->W, out->ptr, out->ld, band);
     SNRSE_LAUNCH_CHECK();
     return SNRSE_OK;
 }
 
-int fir_up2_launch(const ActView* x, const ActView* out, cudaStream_t s, const float* scsh) {
+int fir_up2_launch(const ActView* x, const ActView* out, cudaStream_t s) {
     SNRSE_CHECK_ARG(x->C % 8 == 0, "fir_up2: C %% 8 == 0");
     SNRSE_CHECK_ARG(x->C <= 2048 && x->B <= 65535, "fir_up2: C <= 2048, B <= 65535");
     const int tpp = x->C / 8, nthr = tpp * (256 / tpp > 0 ? 256 / tpp : 1), cols = nthr / tpp;
     int band = FIR_BAND;
     while (band > 1 && (int64_t)cdiv(x->W, cols) * cdiv(x->H, band) * x->B < 592) band >>= 1;
     dim3 grid((unsigned)cdiv(x->W, cols), (unsigned)cdiv(x->H, band), (unsigned)x->B);
-    if (scsh) snrse_launch(fir_up2_kernel<true>, dim3(grid), dim3(nthr), 0, s, x->ptr, x->ld, x->C, x->H, x->W, out->ptr, out->ld, band, scsh);
-    else snrse_launch(fir_up2_kernel<false>, dim3(grid), dim3(nthr), 0, s, x->ptr, x->ld, x->C, x->H, x->W, out->ptr, out->ld, band, scsh);
+    snrse_launch(fir_up2_kernel, dim3(grid), dim3(nthr), 0, s, x->ptr, x->ld, x->C, x->H, x->W, out->ptr, out->ld, band);
     SNRSE_LAUNCH_CHECK();
     return SNRSE_OK;
 }

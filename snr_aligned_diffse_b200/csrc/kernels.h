@@ -115,9 +115,8 @@ int gn_finalize_launch(const unsigned long long* src0, int U0, const unsigned lo
 int gn_apply_launch(const ActView* x, const float* scsh, int silu, const ActView* out, cudaStream_t s);
 
 // ----------------------------------------------------------------------------- fir.cu
-// scsh (nullable): GroupNorm scale/shift [B][2][C]; the input is replaced by bf16(silu(x*scale + shift)) on load
-int fir_up2_launch(const ActView* x, const ActView* out, cudaStream_t s, const float* scsh = nullptr);
-int fir_down2_launch(const ActView* x, const ActView* out, cudaStream_t s, const float* scsh = nullptr);
+int fir_up2_launch(const ActView* x, const ActView* out, cudaStream_t s);
+int fir_down2_launch(const ActView* x, const ActView* out, cudaStream_t s);
 // out_n = FIR(silu(GroupNorm(x))) and out_r = FIR(x) in one pass over x (up / down residual blocks)
 int fir_dual_launch(const ActView* x, const ActView* out_n, const ActView* out_r, int up, const float* scsh, cudaStream_t s);
 int fir_up2_f4_launch(const float* x, float* out, int B, int H, int W, cudaStream_t s);      // in [B,H,W,4]

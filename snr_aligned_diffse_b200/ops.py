@@ -222,30 +222,6 @@ def conv3x3_nhwc_stats(x0, wt, x1=None, bias=None, tbias=None, res=None, scale=1
     return out, dec, ust
 
 
-def gn_silu_fir_nhwc(x, gamma, beta, up, eps=1e-6):
-    """FIR x2 resampling of silu(GroupNorm32(x)) in one pass over x (bf16 NHWC)."""
-    lib = _lib_dev()
-    B, H, W, C = x.shape
-    out = torch.empty((B, 2 * H, 2 * W, C) if up else (B, H // 2, W // 2, C), dtype=x.dtype, device=x.device)
-    ws = torch.empty(int(lib.snrse_groupnorm_workspace_bytes(B)), dtype=torch.uint8, device=x.device)
-    _lib.check(lib.snrse_gn_silu_fir_nhwc(_lib.ptr(x), _lib.ptr(gamma), _lib.ptr(beta), eps, _lib.ptr(out), B, H, W, C,
-                                          int(up), _lib.ptr(ws), _lib.stream_ptr()), "gn_silu_fir")
-    return out
-
-
-def fir_dual_nhwc(x, gamma, beta, up, eps=1e-6):
-    """(FIR x2 resampling of silu(GroupNorm32(x)), FIR x2 resampling of x) in one pass over x (bf16 NHWC)."""
-    lib = _lib_dev()
-    B, H, W, C = x.shape
-    shape = (B, 2 * H, 2 * W, C) if up else (B, H // 2, W // 2, C)
-    out_n = torch.empty(shape, dtype=x.dtype, device=x.device)
-    out_r = torch.empty(shape, dtype=x.dtype, device=x.device)
-    ws = torch.empty(int(lib.snrse_groupnorm_workspace_bytes(B)), dtype=torch.uint8, device=x.device)
-    _lib.check(lib.snrse_fir_dual_nhwc(_lib.ptr(x), _lib.ptr(gamma), _lib.ptr(beta), eps, _lib.ptr(out_n), _lib.ptr(out_r),
-                                       B, H, W, C, int(up), _lib.ptr(ws), _lib.stream_ptr()), "fir_dual")
-    return out_n, out_r
-
-
 def fir_nhwc(x, up):
     lib = _lib_dev()
     B, H, W, C = x.shape

@@ -35,10 +35,9 @@ class GraphedPCLoop:
     Step i = corrector update(s) + predictor update at t_i: 1 + n_steps network evaluations, the complex noise draws
     and the fused state updates; all N steps are recorded back to back into a single graph (N x ~720 kernel nodes).
     The per-step scalars (t_i, step size, SDE coefficients) are host constants baked into the nodes of step i; the state
-    lives in static buffers.  Noise comes from torch's CUDA generator, which advances its Philox offset on every replay.
-    `per_step=True` keeps the earlier layout (one graph per step, replayed in order) for comparison."""
+    lives in static buffers.  Noise comes from torch's CUDA generator, which advances its Philox offset on every replay."""
 
-    def __init__(self, predictor, corrector, timesteps, Y, per_step=False):
+    def __init__(self, predictor, corrector, timesteps, Y):
         dev = Y.device
         self.Y = Y.clone()
         self.x = torch.empty_like(self.Y)
@@ -67,20 +66,11 @@ class GraphedPCLoop:
             self.x.copy_(self.Y)
             one(0)                                   # eager warm-up: plans, workspaces, function attributes
             self.stream.synchronize()
-            if per_step:
-                pool = None
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, stream=self.stream):
                 for i in range(n):
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g, pool=pool, stream=self.stream):
-                        one(i)
-                    pool = g.pool()
-                    self.graphs.append(g)
-            else:
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g, stream=self.stream):
-                    for i in range(n):
-                        one(i)
-                self.graphs.append(g)
+                    one(i)
+            self.graphs.append(g)
         torch.cuda.current_stream(dev).wait_stream(self.stream)
         torch.cuda.set_rng_state(rng, dev)
 
@@ -105,8 +95,7 @@ def get_pc_sampler(predictor_name, corrector_name, sde, score_fn, Y, Y_prior=Non
     draws, state updates) is replayed from ONE CUDA graph captured on first use (`GraphedPCLoop`); False = host loop
     with eager launches; None (default) = eager the first time a (shape, settings) combination is seen through
     `graph_cache`, captured and replayed from the second time on, i.e. whenever shapes repeat.  `graph_cache` (a dict,
-    e.g. one per model: `ScoreModel.get_pc_sampler` supplies it) keeps the captured loops across sampler objects;
-    `graph="per_step"` keeps one graph per reverse step."""
+    e.g. one per model: `ScoreModel.get_pc_sampler` supplies it) keeps the captured loops across sampler objects."""
     predictor_cls = PredictorRegistry.get_by_name(predictor_name)
     corrector_cls = CorrectorRegistry.get_by_name(corrector_name)
     predictor = predictor_cls(sde, score_fn, probability_flow=probability_flow)
@@ -128,7 +117,7 @@ def get_pc_sampler(predictor_name, corrector_name, sde, score_fn, Y, Y_prior=Non
             use_graph = graph
             cache = graph_cache if graph_cache is not None else _local_graphs
             key = (predictor_name, corrector_name, tuple(Y.shape), int(sde.N), float(sde.T), float(eps), float(snr),
-                   int(corrector_steps), bool(probability_flow), type(sde).__name__, graph == "per_step")
+                   int(corrector_steps), bool(probability_flow), type(sde).__name__)
             if use_graph is None:
                 # shapes repeat -> capture: the first call of a combination runs the host loop, later calls replay.
                 # Only with a caller-supplied cache, i.e. through ScoreModel.get_pc_sampler, whose score function is known
@@ -142,7 +131,7 @@ def get_pc_sampler(predictor_name, corrector_name, sde, score_fn, Y, Y_prior=Non
                 if loop is None:
                     # the entry holds score_fn alive, so a cache shared between models cannot hand a loop captured for a
                     # collected model to a new object that reuses its id()
-                    loop = GraphedPCLoop(predictor, corrector, timesteps, Y, per_step=graph == "per_step")
+                    loop = GraphedPCLoop(predictor, corrector, timesteps, Y)
                     cache[key] = loop
                     loop.score_fn = score_fn
                 if getattr(loop, "score_fn", score_fn) is not score_fn:

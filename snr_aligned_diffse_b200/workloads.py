@@ -112,8 +112,7 @@ def run_pc60(dev, rank, world, batch=16, seconds=4.0, enhancers=2, reps=1, N=30,
         y = synth_waves(batch, L, seed=2000 + rank + 100 * e).to(dev)
         peak = ops.absmax(y)
         Y = ops.stft(y, scale=peak, scale_is_divisor=True)[:, None]
-        sampler = model.get_pc_sampler("reverse_diffusion", "ald", Y, N=N, corrector_steps=1, snr=0.5,
-                                       graph=graph if isinstance(graph, str) else bool(graph))
+        sampler = model.get_pc_sampler("reverse_diffusion", "ald", Y, N=N, corrector_steps=1, snr=0.5, graph=bool(graph))
         sampler()                                       # warm-up: plans, weights, graph capture
         keep.append((model, Y))
         peaks.append(peak)

@@ -341,7 +341,7 @@ def test_si_sdr_on_device_matches_reference_formula():
 
 @pytest.mark.parametrize("sde_name", ["ouve", "bbed"])
 def test_pc_sampler_graph_replay_equals_eager_loop(sd, sde_name):
-    """get_pc_sampler(graph=True): the reverse loop replayed from per-step CUDA graphs returns the same bits as the
+    """get_pc_sampler(graph=True): the reverse loop replayed from one CUDA graph returns the same bits as the
     eager host loop when both see the same noise draws (the generator is re-seeded before each run; eager and captured
     `randn_like` calls consume the same Philox sequence), and a second run with a new seed differs (fresh noise per
     replay).  BBED exercises the host-tagged time vector (no device->host read of t inside the loop)."""

@@ -105,7 +105,6 @@ def test_operators_on_odd_shapes_stay_inside_their_buffers(guard):
     ops.gn_silu_conv3x3_nhwc(x, gam, bet, wt[:128].contiguous())
     ops.fir_nhwc(x, True)
     ops.fir_nhwc(x, False)
-    ops.gn_silu_fir_nhwc(x, gam, bet, True)
     for n in (200, 128, 12):                                                                 # CUDA-core and tensor-core paths
         q = torch.randn(2, n, 256, generator=g).to(torch.bfloat16).to(dev)
         ops.attention_nhwc(q, q, q)
@@ -115,7 +114,7 @@ def test_operators_on_odd_shapes_stay_inside_their_buffers(guard):
     ops.stft(w, planar=True, transform=False, pad_multiple=16)
     ops.absmax(w)
     ops.si_sdr(w, w * 0.9 + 0.01)
-    assert guard.check() >= 15
+    assert guard.check() >= 13
 
 
 def test_pc_loop_stays_inside_its_buffers(guard):

@@ -121,6 +121,14 @@ def gn_apply(lib, x, scsh, silu, out):
     _check(lib, lib.snrse_dbg_gn_apply(_ref(x), _ptr(scsh), int(silu), _ref(out), _stream()), "dbg_gn_apply")
 
 
+def fir(lib, x, out, up):
+    _check(lib, lib.snrse_dbg_fir(_ref(x), _ref(out), int(up), _stream()), "dbg_fir")
+
+
+def fir_dual(lib, x, out_n, out_r, up, scsh):
+    _check(lib, lib.snrse_dbg_fir_dual(_ref(x), _ref(out_n), _ref(out_r), int(up), _ptr(scsh), _stream()), "dbg_fir_dual")
+
+
 def fir_f4(lib, x, up):
     B, H, W, _ = x.shape
     out = torch.empty((B, 2 * H, 2 * W, 4) if up else (B, H // 2, W // 2, 4), dtype=torch.float32, device=DEV)
@@ -230,8 +238,8 @@ def test_conv_on_slices_equals_dense(lib, case, path):
 
 @pytest.mark.parametrize("C", [128, 256, 384, 512])
 def test_groupnorm_and_fir_on_slices_equal_dense(lib, C):
-    """gn_stats, gn_apply (with and without SiLU), the FIR passes with the normalisation on load and the dual-output FIR
-    pass on slices == on dense copies, bit for bit; nothing outside the written slices changes."""
+    """gn_stats, gn_apply (with and without SiLU), the FIR pass and the dual-output FIR pass on slices == on dense copies,
+    bit for bit; nothing outside the written slices changes."""
     g = torch.Generator().manual_seed(C)
     B, H, W = 2, 16, 24
     x = bf16(g, B, H, W, C, scale=1.5, shift=0.3)
@@ -246,24 +254,44 @@ def test_groupnorm_and_fir_on_slices_equal_dense(lib, C):
         do = torch.empty_like(x)
         gn_apply(lib, dense(x), scsh, silu, dense(do))
         assert same_bits(so.t, do) and so.intact(), silu
+    sh = so                                           # silu(GroupNorm(x)) as a channel slice
     for up in (1, 0):
         oh, ow = (2 * H, 2 * W) if up else (H // 2, W // 2)
         sn, sr = Slice(B, oh, ow, C, coff=64, after=0), Slice(B, oh, ow, C, coff=C, after=64)
-        _check(lib, lib.snrse_dbg_fir_dual(_ref(sx.view()), _ref(sn.view()), _ref(sr.view()), up, _ptr(scsh), _stream()),
-               "fir_dual")
+        fir_dual(lib, sx.view(), sn.view(), sr.view(), up, scsh)
         dn, dr = (torch.empty(B, oh, ow, C, dtype=torch.bfloat16, device=DEV) for _ in range(2))
-        _check(lib, lib.snrse_dbg_fir_dual(_ref(dense(x)), _ref(dense(dn)), _ref(dense(dr)), up, _ptr(scsh), _stream()),
-               "fir_dual")
+        fir_dual(lib, dense(x), dense(dn), dense(dr), up, scsh)
         assert torch.isfinite(dn.float()).all() and torch.isfinite(dr.float()).all()
         assert same_bits(sn.t, dn) and same_bits(sr.t, dr) and sn.intact() and sr.intact(), up
-        for sc in (None, scsh):
+        for src, dual in ((sx, dr), (sh, dn)):
             so = Slice(B, oh, ow, C, coff=64, after=64)
-            _check(lib, lib.snrse_dbg_fir(_ref(sx.view()), _ref(so.view()), up, _ptr(sc), _stream()), "fir")
+            fir(lib, src.view(), so.view(), up)
             do = torch.empty(B, oh, ow, C, dtype=torch.bfloat16, device=DEV)
-            _check(lib, lib.snrse_dbg_fir(_ref(dense(x)), _ref(dense(do)), up, _ptr(sc), _stream()), "fir")
-            assert same_bits(so.t, do) and so.intact(), (up, sc is None)
-            assert same_bits(so.t, dn if sc is not None else dr), (up, sc is None)   # dual pass == single passes
-    assert sx.intact()
+            fir(lib, dense(src.t.contiguous()), dense(do), up)
+            assert same_bits(so.t, do) and so.intact(), (up, src is sx)
+            assert same_bits(so.t, dual), (up, src is sx)   # dual pass == single passes
+    assert sx.intact() and sh.intact()
+
+
+@pytest.mark.parametrize("shape", [(2, 128, 16, 24), (1, 256, 8, 8), (3, 384, 6, 10)])
+@pytest.mark.parametrize("up", [True, False])
+def test_fir_dual_equals_groupnorm_and_two_fir_passes(lib, shape, up):
+    """The dual-output FIR pass of the up / down residual blocks (rows staged in shared memory raw and normalised) ==
+    GroupNorm pass + FIR pass for the normalised branch and FIR pass of x for the raw branch, bit for bit."""
+    B, C, H, W = shape
+    g = torch.Generator().manual_seed(C + H + int(up))
+    x = bf16(g, B, H, W, C, scale=1.5, shift=0.3)
+    gamma, beta = gn_params(g, C)
+    scsh = gn_finalize(lib, gn_stats(lib, dense(x), B, C), None, B, H * W * C // 32, gamma, beta)
+    oh, ow = (2 * H, 2 * W) if up else (H // 2, W // 2)
+    out_n, out_r, want_n, want_r = (torch.empty(B, oh, ow, C, dtype=torch.bfloat16, device=DEV) for _ in range(4))
+    fir_dual(lib, dense(x), dense(out_n), dense(out_r), up, scsh)
+    h = torch.empty_like(x)
+    gn_apply(lib, dense(x), scsh, 1, dense(h))
+    fir(lib, dense(h), dense(want_n), up)
+    fir(lib, dense(x), dense(want_r), up)
+    assert torch.isfinite(want_n.float()).all() and torch.isfinite(want_r.float()).all()
+    assert same_bits(out_n, want_n) and same_bits(out_r, want_r)
 
 
 @pytest.mark.parametrize("H,W", [(4, 1), (16, 4), (16, 32)], ids=["n4-cudacore", "n64", "n512"])

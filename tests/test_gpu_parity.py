@@ -425,33 +425,6 @@ def test_upfirdn2d_general_matches_reference_vectors(ops, golden_dir):
         ops.upfirdn2d(xb[0].to(DEV), kb.to(DEV))                      # not [N, C, H, W]
 
 
-@pytest.mark.parametrize("shape", [(2, 128, 16, 24), (1, 256, 8, 8), (3, 384, 6, 10)])
-@pytest.mark.parametrize("up", [True, False])
-def test_gn_silu_fir_fused_equals_two_passes(ops, shape, up):
-    """FIR with GroupNorm+SiLU applied on load == GroupNorm pass followed by the FIR pass, bit for bit."""
-    B, C, H, W = shape
-    g = torch.Generator().manual_seed(C + H + int(up))
-    x = (torch.randn(B, H, W, C, generator=g) * 1.5 + 0.3).to(torch.bfloat16).to(DEV)
-    gamma, beta = (torch.rand(C, generator=g) + 0.5).to(DEV), (torch.randn(C, generator=g) * 0.2).to(DEV)
-    fused = ops.gn_silu_fir_nhwc(x, gamma, beta, up)
-    two = ops.fir_nhwc(ops.groupnorm_nhwc(x, gamma, beta, silu=True), up)
-    assert torch.equal(fused, two)
-
-
-@pytest.mark.parametrize("shape", [(2, 128, 16, 24), (1, 256, 8, 8), (3, 384, 6, 10)])
-@pytest.mark.parametrize("up", [True, False])
-def test_fir_dual_equals_groupnorm_and_two_fir_passes(ops, shape, up):
-    """The dual-output FIR pass of the up / down residual blocks (rows staged in shared memory raw and normalised) ==
-    GroupNorm pass + FIR pass for the normalised branch and FIR pass of x for the raw branch, bit for bit."""
-    B, C, H, W = shape
-    g = torch.Generator().manual_seed(C + H + int(up))
-    x = (torch.randn(B, H, W, C, generator=g) * 1.5 + 0.3).to(torch.bfloat16).to(DEV)
-    gamma, beta = (torch.rand(C, generator=g) + 0.5).to(DEV), (torch.randn(C, generator=g) * 0.2).to(DEV)
-    out_n, out_r = ops.fir_dual_nhwc(x, gamma, beta, up)
-    assert torch.equal(out_n, ops.fir_nhwc(ops.groupnorm_nhwc(x, gamma, beta, silu=True), up))
-    assert torch.equal(out_r, ops.fir_nhwc(x, up))
-
-
 @pytest.mark.parametrize("n", [4, 12, 64, 200, 128, 512, 1984])   # n % 64 == 0: tensor-core path
 def test_attention(ops, n):
     g = torch.Generator().manual_seed(n)

@@ -101,7 +101,7 @@ def test_bbed_loop_matches_reference_fixture(sd, golden_dir, monkeypatch, graph)
 def test_whole_loop_graph_is_default_when_shapes_repeat(sd):
     """get_pc_sampler() without a `graph` argument: the first call of a (shape, settings) combination runs the host
     loop, the second captures the WHOLE N-step loop as one CUDA graph and later calls replay it; with the generator
-    re-seeded the three agree bit for bit, and so does the older one-graph-per-step layout."""
+    re-seeded the three agree bit for bit."""
     m = _model(sd, "ouve", theta=1.5, sigma_min=0.05, sigma_max=0.5)
     g = torch.Generator().manual_seed(3)
     Y = torch.view_as_complex(torch.randn(2, 1, 256, 64, 2, generator=g) * 0.05).cuda()
@@ -116,10 +116,6 @@ def test_whole_loop_graph_is_default_when_shapes_repeat(sd):
     assert len(loops) == 1 and len(loops[0].graphs) == 1            # one graph holds all three steps
     assert torch.equal(torch.view_as_real(outs[0]), torch.view_as_real(outs[1]))
     assert torch.equal(torch.view_as_real(outs[1]), torch.view_as_real(outs[2]))
-    torch.manual_seed(5)
-    torch.cuda.manual_seed_all(5)
-    per_step, _ = m.get_pc_sampler("reverse_diffusion", "ald", Y, N=3, corrector_steps=1, snr=0.5, graph="per_step")()
-    assert torch.equal(torch.view_as_real(per_step), torch.view_as_real(outs[2]))
 
 
 def test_lincomb_rejects_mismatched_operands_and_accepts_strided_ones():

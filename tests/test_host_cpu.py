@@ -22,7 +22,7 @@ def test_abi_exports_every_declared_symbol():
     debug = set(re.findall(r"\b(snrse_[a-z0-9_]+)\s*\(", dbg))
     # measurement / debug entry points live in their own header, not in the product ABI
     assert debug == {"snrse_ncsnpp_num_launch_groups", "snrse_ncsnpp_profile_forward", "snrse_ncsnpp_read_tap",
-                     "snrse_conv_halo_set_debug", "snrse_fir_dual_nhwc"} and not (debug & product)
+                     "snrse_conv_halo_set_debug"} and not (debug & product)
     declared = product | debug
     lib = _lib.load()
     assert declared, "no declarations found"

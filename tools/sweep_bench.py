@@ -5,7 +5,7 @@ its line; this tool exists for ad-hoc runs with other sizes.
 
     python tools/sweep_bench.py --workload vbd [--fixed-snr 0.31623] [--count 824] [--graphs 0]
     python tools/sweep_bench.py --workload long --count 2
-    python tools/sweep_bench.py --workload pc [--graphs per_step|0|1]
+    python tools/sweep_bench.py --workload pc [--graphs 0|1]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/sweep_bench.py --workload vbd
 """
 import argparse
@@ -31,7 +31,7 @@ def main():
                     help="vbd: padded frames per batch (0: at most --max-batch utterances per batch)")
     ap.add_argument("--repeat", type=int, default=2, help="passes over the list; the last one is timed")
     ap.add_argument("--enhancers", type=int, default=2, help="pc workload: independent batches in flight per GPU (graph mode)")
-    ap.add_argument("--graphs", default="1", help="1: CUDA graphs (default), 0: eager launches, per_step (pc only)")
+    ap.add_argument("--graphs", default="1", choices=["0", "1"], help="1: CUDA graphs (default), 0: eager launches")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -41,7 +41,7 @@ def main():
     if world > 1:
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
-    graphs = {"0": False, "1": True}.get(args.graphs, args.graphs)
+    graphs = args.graphs == "1"
     if args.workload == "pc":
         out = wl.run_pc60(dev, rank, world, batch=bench.BATCH, seconds=bench.SECONDS, enhancers=args.enhancers,
                           reps=max(1, args.repeat - 1), graph=graphs)
@@ -49,9 +49,9 @@ def main():
         model, _ = bench.build_models(dev, fixed_snr=args.fixed_snr)
         if args.workload == "vbd":
             out = wl.run_sweep824(model, dev, rank, world, count=args.count or 824, max_batch=args.max_batch,
-                                  graphs=bool(graphs), repeat=args.repeat, target_frames=args.target_frames)
+                                  graphs=graphs, repeat=args.repeat, target_frames=args.target_frames)
         else:
-            out = wl.run_longform60(model, dev, rank, world, count=args.count or 2, graphs=bool(graphs), repeat=args.repeat)
+            out = wl.run_longform60(model, dev, rank, world, count=args.count or 2, graphs=graphs, repeat=args.repeat)
     if rank == 0:
         print(json.dumps(dict(workload=args.workload, unit=bench.UNIT, n_gpus=world, **out)), flush=True)
     if world > 1:
