@@ -86,6 +86,12 @@ LAYER_PROTOTYPES = {
     "snrse_dbg_attention": (i32, [vp, vp, vp, vp, vp, i32, vp]),
 }
 
+# every symbol declared in include/snrse_b200_plans.h (the executor's convolution plans, for the plan tests)
+PLAN_PROTOTYPES = {
+    "snrse_ncsnpp_dbg_convs": (i32, [vp, i32, i32, i32, i32, i32, vp, i32, POINTER(i32)]),
+    "snrse_dbg_conv_plan": (i32, [vp, i32, vp, vp, i32, vp, vp, vp, i32, vp]),
+}
+
 
 def load():
     """Load the shared library (once).  Raises RuntimeError when it has not been built."""
@@ -97,7 +103,7 @@ def load():
             f"{LIB_PATH} is missing: build it with `python -m snr_aligned_diffse_b200.build` "
             "(nvcc, sm_100a).  This package has no CPU or PyTorch fallback.")
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (res, args) in {**PROTOTYPES, **LAYER_PROTOTYPES}.items():
+    for name, (res, args) in {**PROTOTYPES, **LAYER_PROTOTYPES, **PLAN_PROTOTYPES}.items():
         # one flag per parameter makes a call with more arguments than the prototype a TypeError; a plain ctypes
         # function would pass the extra ones on, e.g. a stale argument list's pointer in place of the stream.
         # AttributeError if the ABI and the header drifted apart.

@@ -35,6 +35,7 @@ def _newest_header():
     hs.append(os.path.join(os.path.dirname(HERE), "include", "snrse_b200.h"))
     hs.append(os.path.join(os.path.dirname(HERE), "include", "snrse_b200_debug.h"))
     hs.append(os.path.join(os.path.dirname(HERE), "include", "snrse_b200_layers.h"))
+    hs.append(os.path.join(os.path.dirname(HERE), "include", "snrse_b200_plans.h"))
     return max(os.path.getmtime(h) for h in hs if os.path.exists(h))
 
 

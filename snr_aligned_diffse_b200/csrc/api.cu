@@ -280,6 +280,36 @@ int snrse_dbg_conv(const snrse_view* x0, int taps0, const snrse_view* x1, const 
     return conv_gemm_launch(&g, S(stream));
 }
 
+// The plan fields snrse_dbg_conv (path 0 / 2) or, for path 0 with n = 4, snrse_dbg_conv_out4 (out: the fp32 [B][H][W][4]
+// result) makes for these views, from the launcher's own make_plan with the device's SM count; nothing is launched.
+int snrse_dbg_conv_plan(const snrse_view* x0, int taps0, const snrse_view* x1, const void* wt, int n, const snrse_view* res,
+                        const snrse_view* out, const float* scsh, int path, void* plan) {
+    SNRSE_CHECK_ARG(x0 && wt && out && plan, "dbg_conv_plan: null pointer");
+    const ActView a0 = AV(x0), a1 = x1 ? AV(x1) : ActView{}, r = res ? AV(res) : ActView{};
+    const bf16* w = static_cast<const bf16*>(wt);
+    ConvPlanFields* f = static_cast<ConvPlanFields*>(plan);
+    if (path == 0 && n == 4) {
+        ConvHaloPlan hp;
+        float* o4 = static_cast<float*>(out->ptr);
+        SNRSE_TRY(conv_halo2_make_plan_out4(&hp, &a0, w, o4 /* a bias pointer the plan only stores */, nullptr, o4, scsh));
+        *f = conv_plan_fields(hp);
+        return SNRSE_OK;
+    }
+    if (path == 0) {
+        ConvHaloPlan hp;
+        SNRSE_TRY(conv_halo2_make_plan(&hp, &a0, x1 ? &a1 : nullptr, w, n, nullptr, nullptr, 0, res ? &r : nullptr, 1.0f,
+                                       static_cast<bf16*>(out->ptr), out->ld, scsh, nullptr));
+        *f = conv_plan_fields(hp);
+        return SNRSE_OK;
+    }
+    SNRSE_CHECK_ARG(path == 2 && !scsh, "dbg_conv_plan: path must be 0 or 2 (scsh: path 0 only)");
+    ConvGemmPlan g;
+    SNRSE_TRY(conv_gemm_make_plan(&g, &a0, taps0, x1 ? &a1 : nullptr, w, n, 0, 0, nullptr, nullptr, 0, res ? &r : nullptr,
+                                  1.0f, out->ptr, out->ld, 0));
+    *f = conv_plan_fields(g);
+    return SNRSE_OK;
+}
+
 int snrse_dbg_gn_stats(const snrse_view* x, void* ustats, void* stream) {
     const ActView vx = AV(x);
     return gn_stats_launch(&vx, static_cast<unsigned long long*>(ustats), S(stream));

@@ -277,28 +277,23 @@ int conv_gemm_make_plan(ConvGemmPlan* p, const ActView* a0, int taps0, const Act
                                   scale, out, out_ld, out_f32, 0);
 }
 
-int conv_gemm_make_plan_ex(ConvGemmPlan* p, const ActView* a0, int taps0, const ActView* a1, const bf16* wt, int n_rows,
-                           int64_t wt_batch_stride, int b_batched, const float* bias, const float* tbias, int tb_stride,
-                           const ActView* res, float scale, void* out, int out_ld, int out_f32, int64_t wt_row_pitch) {
+int conv_gemm_plan_shape(ConvGemmPlan* p, int B, int H, int W, int taps0, int C0, int C1, int n_rows, int num_sms) {
     SNRSE_CHECK_ARG(taps0 == 1 || taps0 == 9, "conv_gemm: taps0 must be 1 or 9");
-    SNRSE_CHECK_ARG(a0->C % 64 == 0 && a0->ld % 8 == 0, "conv_gemm: Cin must be a multiple of 64 (got %d)", a0->C);
-    SNRSE_CHECK_ARG(!a1 || (a1->C % 64 == 0 && a1->ld % 8 == 0), "conv_gemm: Cin1 must be a multiple of 64");
-    SNRSE_CHECK_ARG(!a1 || (a1->B == a0->B && a1->H == a0->H && a1->W == a0->W), "conv_gemm: segment shapes differ");
+    SNRSE_CHECK_ARG(C0 % 64 == 0, "conv_gemm: Cin must be a multiple of 64 (got %d)", C0);
+    SNRSE_CHECK_ARG(C1 % 64 == 0, "conv_gemm: Cin1 must be a multiple of 64");
     SNRSE_CHECK_ARG(n_rows % 32 == 0, "conv_gemm: N must be a multiple of 32 (got %d)", n_rows);
-    SNRSE_CHECK_ARG(out_ld % (out_f32 ? 4 : 8) == 0, "conv_gemm: output pitch must be a multiple of 16 bytes");
-    SNRSE_CHECK_ARG(!res || res->ld % 8 == 0, "conv_gemm: residual pitch must be a multiple of 8");
     memset(p, 0, sizeof(*p));
     p->taps0 = taps0;
-    p->c0_chunks = a0->C / 64;
-    p->c1_chunks = a1 ? a1->C / 64 : 0;
-    p->B = a0->B;
-    p->H = a0->H;
-    p->W = a0->W;
+    p->c0_chunks = C0 / 64;
+    p->c1_chunks = C1 / 64;
+    p->B = B;
+    p->H = H;
+    p->W = W;
     // tile shape: th*tw = 128, fewest tiles; ties -> prefer 8x16 (small halo for the 3x3 taps)
     int best_tw = 128, best_tiles = 1 << 30, best_rank = 1 << 30;
     for (int tw = 1; tw <= 128; tw <<= 1) {
         const int th = 128 / tw;
-        const int tiles = cdiv(a0->H, th) * cdiv(a0->W, tw);
+        const int tiles = cdiv(H, th) * cdiv(W, tw);
         const int rank = abs(ilog2(tw) - 4);
         if (tiles < best_tiles || (tiles == best_tiles && rank < best_rank)) {
             best_tiles = tiles;
@@ -309,18 +304,41 @@ int conv_gemm_make_plan_ex(ConvGemmPlan* p, const ActView* a0, int taps0, const 
     const int tw = best_tw, th = 128 / tw;
     p->tw_log2 = ilog2(tw);
     p->th_log2 = ilog2(th);
-    p->tiles_h = cdiv(a0->H, th);
-    p->tiles_w = cdiv(a0->W, tw);
+    p->tiles_h = cdiv(H, th);
+    p->tiles_w = cdiv(W, tw);
     p->N = n_rows;
     p->n_tile = n_rows >= 256 ? 256 : (n_rows >= 128 ? 128 : 64);
     // Few pixel tiles (small feature maps): one CTA walks the whole K loop alone and is bound by the TMA latency per
     // K block, not by the tensor pipe.  Split N into 64-column tiles (4x the CTAs, a quarter of the MMA time each) and
     // give every CTA a whole SM's shared memory for a deep TMA ring.
+    const int64_t pixel_tiles = (int64_t)B * p->tiles_h * p->tiles_w;
+    const bool small = pixel_tiles * cdiv(n_rows, p->n_tile) * 2 <= num_sms && n_rows % 64 == 0;
+    if (small) p->n_tile = 64;
+    p->small = small;
+    const int stage_bytes = A_STAGE_BYTES + p->n_tile * BLOCK_K * 2;
+    // two CTAs per SM when possible (overlaps one tile's epilogue with the other's main loop)
+    int stages = ((small ? 196 : 110) * 1024) / stage_bytes;
+    if (stages > MAX_STAGES) stages = MAX_STAGES;
+    if (stages < 2) stages = 2;
+    const int nkb = taps0 * p->c0_chunks + p->c1_chunks;
+    if (stages > nkb) stages = nkb < 2 ? 2 : nkb;
+    p->stages = stages;
+    p->smem_bytes = stages * stage_bytes + 1024;
+    p->a_box_bytes = th * tw * 128;
+    return SNRSE_OK;
+}
+
+int conv_gemm_make_plan_ex(ConvGemmPlan* p, const ActView* a0, int taps0, const ActView* a1, const bf16* wt, int n_rows,
+                           int64_t wt_batch_stride, int b_batched, const float* bias, const float* tbias, int tb_stride,
+                           const ActView* res, float scale, void* out, int out_ld, int out_f32, int64_t wt_row_pitch) {
+    SNRSE_CHECK_ARG(a0->ld % 8 == 0, "conv_gemm: the operand pitch must be a multiple of 8");
+    SNRSE_CHECK_ARG(!a1 || a1->ld % 8 == 0, "conv_gemm: the shortcut operand pitch must be a multiple of 8");
+    SNRSE_CHECK_ARG(!a1 || (a1->B == a0->B && a1->H == a0->H && a1->W == a0->W), "conv_gemm: segment shapes differ");
+    SNRSE_CHECK_ARG(out_ld % (out_f32 ? 4 : 8) == 0, "conv_gemm: output pitch must be a multiple of 16 bytes");
+    SNRSE_CHECK_ARG(!res || res->ld % 8 == 0, "conv_gemm: residual pitch must be a multiple of 8");
     int dev = 0, sms = 148;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int64_t pixel_tiles = (int64_t)a0->B * p->tiles_h * p->tiles_w;
-    const bool small = pixel_tiles * cdiv(n_rows, p->n_tile) * 2 <= sms && n_rows % 64 == 0;
-    if (small) p->n_tile = 64;
+    SNRSE_TRY(conv_gemm_plan_shape(p, a0->B, a0->H, a0->W, taps0, a0->C, a1 ? a1->C : 0, n_rows, sms));
     p->b_batched = b_batched;
     p->bias = bias;
     p->tbias = tbias;
@@ -331,22 +349,11 @@ int conv_gemm_make_plan_ex(ConvGemmPlan* p, const ActView* a0, int taps0, const 
     p->out = out;
     p->out_ld = out_ld;
     p->out_f32 = out_f32;
-    const int stage_bytes = A_STAGE_BYTES + p->n_tile * BLOCK_K * 2;
-    // two CTAs per SM when possible (overlaps one tile's epilogue with the other's main loop)
-    int stages = ((small ? 196 : 110) * 1024) / stage_bytes;
-    if (stages > MAX_STAGES) stages = MAX_STAGES;
-    if (stages < 2) stages = 2;
-    const int nkb = taps0 * p->c0_chunks + p->c1_chunks;
-    if (stages > nkb) stages = nkb < 2 ? 2 : nkb;
-    p->stages = stages;
-    p->smem_bytes = stages * stage_bytes + 1024;
-
-    const int64_t ktot = (int64_t)64 * nkb;
-    const int box_h = th;
-    p->a_box_bytes = box_h * tw * 128;
-    SNRSE_TRY(tma_make_act_map(&p->mapA0, a0->ptr, a0->C, a0->W, a0->H, a0->B, a0->ld, 64, tw, box_h));
+    const int64_t ktot = (int64_t)64 * (taps0 * p->c0_chunks + p->c1_chunks);
+    const int tw = 1 << p->tw_log2, th = 1 << p->th_log2;
+    SNRSE_TRY(tma_make_act_map(&p->mapA0, a0->ptr, a0->C, a0->W, a0->H, a0->B, a0->ld, 64, tw, th));
     if (a1) {
-        SNRSE_TRY(tma_make_act_map(&p->mapA1, a1->ptr, a1->C, a1->W, a1->H, a1->B, a1->ld, 64, tw, box_h));
+        SNRSE_TRY(tma_make_act_map(&p->mapA1, a1->ptr, a1->C, a1->W, a1->H, a1->B, a1->ld, 64, tw, th));
     } else {
         p->mapA1 = p->mapA0;
     }

@@ -664,33 +664,36 @@ conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
 
 int g_num_sms2 = 0;
 
-// Zeroes the plan and fills in what both plans share: the tiling (SUB, tile counts), the N split, the TMEM
-// accumulator count and the persistent grid.
-int halo_plan_tiles(ConvHaloPlan* p, const ActView* a0, int n_rows) {
+int device_num_sms() {
     if (g_num_sms2 == 0) {
         int dev = 0;
         SNRSE_CUDA(cudaGetDevice(&dev));
         SNRSE_CUDA(cudaDeviceGetAttribute(&g_num_sms2, cudaDevAttrMultiProcessorCount, dev));
     }
+    return g_num_sms2;
+}
+
+// Zeroes the plan and fills in what both plans share: the tiling (SUB, tile counts), the N split, the TMEM
+// accumulator count and the persistent grid.
+void halo_plan_tiles(ConvHaloPlan* p, int B, int H, int W, int C0, int n_rows, int num_sms) {
     memset(p, 0, sizeof(*p));
-    const int tiles_w = cdiv(a0->W, TW);
+    const int tiles_w = cdiv(W, TW);
     int sub = 2;
-    if (a0->H < 2 * SUB_ROWS || (int64_t)a0->B * cdiv(a0->H, 2 * SUB_ROWS) * tiles_w < g_num_sms2) sub = 1;
+    if (H < 2 * SUB_ROWS || (int64_t)B * cdiv(H, 2 * SUB_ROWS) * tiles_w < num_sms) sub = 1;
     p->sub = sub;
-    p->c0_chunks = a0->C / 64;
-    p->B = a0->B; p->H = a0->H; p->W = a0->W;
-    p->tiles_h = cdiv(a0->H, SUB_ROWS * sub);
+    p->c0_chunks = C0 / 64;
+    p->B = B; p->H = H; p->W = W;
+    p->tiles_h = cdiv(H, SUB_ROWS * sub);
     p->tiles_w = tiles_w;
-    p->n_tiles = a0->B * p->tiles_h * p->tiles_w;
+    p->n_tiles = B * p->tiles_h * p->tiles_w;
     // N-split: with so few pixel tiles that twice as many clusters still fit the GPU, every tile is computed by two
     // clusters, 128 output channels each (half the MMA and weight-tile time per cluster on the latency-bound small maps)
-    const int n_ctiles = (p->n_tiles + 1) / 2, max_clusters = g_num_sms2 / 2;
+    const int n_ctiles = (p->n_tiles + 1) / 2, max_clusters = num_sms / 2;
     p->nsplit = (n_rows == 256 && 2 * n_ctiles <= max_clusters) ? 2 : 1;
     p->n_total = n_rows;
     p->N = n_rows / p->nsplit;
     p->acc_bufs = (sub * p->N <= 256) ? 2 : 1;
     p->grid = p->nsplit == 2 ? 4 * n_ctiles : 2 * (n_ctiles < max_clusters ? n_ctiles : max_clusters);
-    return SNRSE_OK;
 }
 }  // namespace
 extern long long* g_halo_dbg_shared;
@@ -701,17 +704,12 @@ bool conv_halo2_eligible(int H, int W, int taps0, int n_rows) {
     return taps0 == 9 && conv_halo2_fits(H, W) && (n_rows == 128 || n_rows == 256);
 }
 
-int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, const bf16* wt, int n_rows,
-                         const float* bias, const float* tbias, int tb_stride, const ActView* res, float scale, bf16* out,
-                         int out_ld, const float* scsh, unsigned long long* ustats) {
-    SNRSE_CHECK_ARG(conv_halo2_eligible(a0->H, a0->W, 9, n_rows), "conv_halo2: shape not eligible");
-    SNRSE_CHECK_ARG(a0->C % 64 == 0 && a0->ld % 8 == 0, "conv_halo2: Cin must be a multiple of 64");
-    SNRSE_CHECK_ARG(!a1 || (a1->C % 64 == 0 && a1->ld % 8 == 0 && a1->H == a0->H && a1->W == a0->W && a1->B == a0->B),
-                    "conv_halo2: bad shortcut operand");
-    SNRSE_CHECK_ARG(a0->C / 64 + (a1 ? a1->C / 64 : 0) <= 16, "conv_halo2: at most 16 channel chunks (1024 channels)");
-    SNRSE_CHECK_ARG(out_ld % 8 == 0 && (!res || res->ld % 8 == 0), "conv_halo2: pitches must be multiples of 8");
-    SNRSE_TRY(halo_plan_tiles(p, a0, n_rows));
-    p->c1_chunks = a1 ? a1->C / 64 : 0;
+int conv_halo2_plan_shape(ConvHaloPlan* p, int B, int H, int W, int C0, int C1, int n_rows, int norm, int num_sms) {
+    SNRSE_CHECK_ARG(conv_halo2_eligible(H, W, 9, n_rows), "conv_halo2: shape not eligible");
+    SNRSE_CHECK_ARG(C0 % 64 == 0 && C1 % 64 == 0, "conv_halo2: channel counts must be multiples of 64");
+    SNRSE_CHECK_ARG(C0 / 64 + C1 / 64 <= 16, "conv_halo2: at most 16 channel chunks (1024 channels)");
+    halo_plan_tiles(p, B, H, W, C0, n_rows, num_sms);
+    p->c1_chunks = C1 / 64;
     const int sub = p->sub, n_loc = p->N;
     const int a_bytes = (int)halo_stage_bytes(sub), b_bytes = (n_loc / 2) * 128;
     // dynamic shared memory (static: barriers + per-warp bias slices, ~4.3 KB)
@@ -720,7 +718,7 @@ int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, 
     // normalisation the slot also waits for the normalising warps (load + ~2500 clk); at N=128 (64-clock MMAs) that
     // needs a third slot, paid for with single-buffered epilogue staging.
     int na = 2, stg = 2, nsc = 0;
-    if (scsh && n_loc == 128 && sub == 2) { na = 3; stg = 1; }
+    if (norm && n_loc == 128 && sub == 2) { na = 3; stg = 1; }
     int nb = (budget - na * a_bytes - stg * EPI_WARPS * 4096) / b_bytes;
     if (nb < 6 && stg == 2) {
         stg = 1;
@@ -736,7 +734,7 @@ int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, 
     // Only for the 128-output-channel layers (where N = 128 whatever the batch): the K order then depends on the layer alone,
     // never on the batch-dependent tiling, so results stay batch-invariant bit for bit.  The 256-channel layers keep the
     // shared ring: at N = 256 / SUB = 2 two extra slots leave room for only two weight slots.
-    if (a1 && n_rows == 128) {
+    if (C1 > 0 && n_rows == 128) {
         const int sc_bytes = SUB_ROWS * sub * TW * 128;
         const int limit = 227 * 1024 - 1024 /*alignment*/ - 768 /*static: barriers*/ - (int)halo_bsum_bytes(n_loc);
         const int nb2 = (limit - 2 * a_bytes - MAX_SC * sc_bytes - EPI_WARPS * 4096) / b_bytes;
@@ -745,6 +743,19 @@ int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, 
     p->na = na; p->nb = nb; p->stg_bufs = stg; p->nsc = nsc;
     p->smem_bytes = na * a_bytes + nsc * SUB_ROWS * sub * TW * 128 + nb * b_bytes + stg * EPI_WARPS * 4096 +
                     (int)halo_bsum_bytes(n_loc) + 1024;
+    return SNRSE_OK;
+}
+
+int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, const bf16* wt, int n_rows,
+                         const float* bias, const float* tbias, int tb_stride, const ActView* res, float scale, bf16* out,
+                         int out_ld, const float* scsh, unsigned long long* ustats) {
+    SNRSE_CHECK_ARG(a0->ld % 8 == 0, "conv_halo2: the operand pitch must be a multiple of 8");
+    SNRSE_CHECK_ARG(!a1 || (a1->ld % 8 == 0 && a1->H == a0->H && a1->W == a0->W && a1->B == a0->B),
+                    "conv_halo2: bad shortcut operand");
+    SNRSE_CHECK_ARG(out_ld % 8 == 0 && (!res || res->ld % 8 == 0), "conv_halo2: pitches must be multiples of 8");
+    SNRSE_TRY(conv_halo2_plan_shape(p, a0->B, a0->H, a0->W, a0->C, a1 ? a1->C : 0, n_rows, scsh != nullptr,
+                                    device_num_sms()));
+    const int sub = p->sub, n_loc = p->N;
     p->bias = bias; p->tbias = tbias; p->tb_stride = tb_stride;
     p->res = res ? res->ptr : nullptr; p->res_ld = res ? res->ld : 0;
     p->scale = scale; p->out = out; p->out_ld = out_ld;
@@ -765,15 +776,20 @@ int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, 
 
 // Thin output convolution on the same kernel: 3x3, C -> 4 (weights packed as 16 rows, rows 4..15 zero), optional
 // GroupNorm+SiLU of the operand in flight, fp32 output [B,H,W,4] = conv + bias (+ addend4).
+int conv_halo2_plan_shape_out4(ConvHaloPlan* p, int B, int H, int W, int C0, int num_sms) {
+    SNRSE_CHECK_ARG(conv_halo2_fits(H, W) && C0 % 64 == 0 && C0 / 64 <= 16, "conv_halo2 out4: shape not eligible");
+    halo_plan_tiles(p, B, H, W, C0, 16, num_sms);
+    p->na = 3; p->nb = MAX_B; p->stg_bufs = 0;   // no epilogue staging: the result leaves from registers
+    p->smem_bytes = p->na * (int)halo_stage_bytes(p->sub) + p->nb * 1024 + (int)halo_bsum_bytes(16) + 1024;
+    return SNRSE_OK;
+}
+
 int conv_halo2_make_plan_out4(ConvHaloPlan* p, const ActView* a0, const bf16* wt16, const float* bias4, const float* addend4,
                               float* out4, const float* scsh) {
-    SNRSE_CHECK_ARG(conv_halo2_fits(a0->H, a0->W) && a0->C % 64 == 0 && a0->ld % 8 == 0, "conv_halo2 out4: shape not eligible");
+    SNRSE_CHECK_ARG(a0->ld % 8 == 0, "conv_halo2 out4: the operand pitch must be a multiple of 8");
     SNRSE_CHECK_ARG(bias4 && out4, "conv_halo2 out4: null pointer");
-    SNRSE_TRY(halo_plan_tiles(p, a0, 16));
+    SNRSE_TRY(conv_halo2_plan_shape_out4(p, a0->B, a0->H, a0->W, a0->C, device_num_sms()));
     const int sub = p->sub;
-    const int a_bytes = (int)halo_stage_bytes(sub);
-    p->na = 3; p->nb = MAX_B; p->stg_bufs = 0;   // no epilogue staging: the result leaves from registers
-    p->smem_bytes = p->na * a_bytes + p->nb * 1024 + (int)halo_bsum_bytes(16) + 1024;
     p->bias = bias4; p->scale = 1.0f;
     p->scsh = scsh;
     p->out4 = out4; p->addend4 = addend4;

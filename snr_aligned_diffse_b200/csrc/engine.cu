@@ -83,6 +83,14 @@ struct Plan {
         return reinterpret_cast<unsigned long long*>(ws + tens[t_stats].off) + (int64_t)entry * B * 256;
     }
     std::map<int, std::pair<int, int>> cat_children;
+    // every convolution rec_conv / rec_conv_out records, in order (snrse_ncsnpp_dbg_convs); tensor ids < 0 are absent
+    struct ConvRec {
+        int x, taps, shortcut, res, out, n_rows;
+        int path;   // 0 2-CTA kernel, 1 CUDA cores, 2 single-CTA implicit GEMM (the path codes of snrse_dbg_conv)
+        bool norm, stats, tbias, bias, out4, addend;
+        float scale;
+    };
+    std::vector<ConvRec> convs;
     int step = 0;
     int64_t ws_bytes = 0;
     uint8_t* ws = nullptr;
@@ -135,14 +143,15 @@ struct Plan {
         cat_children[c] = {a, b};
         return c;
     }
+    int chan_off(int id) const {   // first channel of tensor id inside its root buffer
+        int coff = 0;
+        for (int r = id; tens[r].parent >= 0; r = tens[r].parent) coff += tens[r].coff;
+        return coff;
+    }
     ActView view(int id) const {
-        int r = id, coff = 0;
-        while (tens[r].parent >= 0) {
-            coff += tens[r].coff;
-            r = tens[r].parent;
-        }
+        const int r = root(id);
         ActView v;
-        v.ptr = reinterpret_cast<bf16*>(ws + tens[r].off) + coff;
+        v.ptr = reinterpret_cast<bf16*>(ws + tens[r].off) + chan_off(id);
         v.B = tens[id].B; v.H = tens[id].H; v.W = tens[id].W; v.C = tens[id].C;
         v.ld = tens[r].C;
         return v;
@@ -381,6 +390,8 @@ struct Conv {
     bool norm = false;    // x is normalised in flight: GroupNorm + SiLU with the scale/shift in t_scsh
 };
 
+int dbg_path(ConvPath path) { return path == CONV_HALO2 ? 0 : path == CONV_SIMT ? 1 : 2; }
+
 int rec_conv(Plan& P, const Conv& c) {
     const ConvPath path = conv_path(P, P.tens[c.x].H, P.tens[c.x].W, c.taps, c.n_rows);
     int st = -1;
@@ -388,6 +399,8 @@ int rec_conv(Plan& P, const Conv& c) {
         st = P.n_stat_entries++;
         P.stats_of[c.out] = st;
     }
+    P.convs.push_back({c.x, c.taps, c.shortcut, c.res, c.out, c.n_rows, dbg_path(path), c.norm, st >= 0, c.tb_row >= 0,
+                       c.bias >= 0, false, false, c.scale});
     P.record({c.x, c.norm ? P.t_scsh : -1, c.shortcut, c.res, c.out, c.tb_row >= 0 ? P.t_tb : -1}, [=](Plan& p) -> int {
         Engine& e = *p.eng;
         ActView va0 = p.view(c.x), va1, vres, vout = p.view(c.out);
@@ -641,6 +654,8 @@ int rec_conv_out(Plan& P, const Mod& mg, const Mod& mc, int h, int prev) {
     const int a = rec_gn_silu_operand(P, h, mg.gn_g, mg.gn_b, tc);
     const int np = P.new_t(th.B, th.H, th.W, 4, 4);
     const int up = prev >= 0 ? P.new_t(th.B, th.H, th.W, 4, 4) : -1;
+    P.convs.push_back({a, 9, -1, -1, np, 4, dbg_path(tc ? CONV_HALO2 : CONV_SIMT), tc, false, false, true, true, prev >= 0,
+                       1.0f});
     P.record({a, np, tc ? P.t_scsh : -1, prev, up}, [=](Plan& p) -> int {
         Engine& e = *p.eng;
         const ActView va = p.view(a);
@@ -794,6 +809,32 @@ __global__ void tap_f32_kernel(const float* __restrict__ x, int C, int64_t hw, f
     out[i] = x[(b * hw + p) * C + c];
 }
 
+// F and T positive multiples of 2^(levels-1), F the image size the attention placement was built for, known flags
+bool plan_args_ok(const Engine* e, int B, int F, int T, int flags) {
+    if (flags & ~3) {
+        snrse_set_error("plan: unknown flags 0x%x (bit0: keep every activation, bit1: CUDA-core cross-check)", flags);
+        return false;
+    }
+    if (!e || B < 1 || F < 1 || T < 1 || (F % (1 << (e->n_levels - 1))) || (T % (1 << (e->n_levels - 1)))) {
+        snrse_set_error("plan: F and T must be positive multiples of 2^(levels-1) (got B=%d F=%d T=%d)", B, F, T);
+        return false;
+    }
+    if (F != e->image_size) {
+        snrse_set_error("plan: F=%d differs from the image_size=%d the attention placement was built for", F, e->image_size);
+        return false;
+    }
+    return true;
+}
+
+// One row of snrse_ncsnpp_dbg_convs (snrse_conv_row of include/snrse_b200_plans.h mirrors this struct)
+struct ConvRow {
+    int path, out4, B, H, W;
+    int c0, ld0, off0, c1, ld1, off1, res, ld_res, off_res, ld_out, off_out;
+    int taps, n, norm, bias, tbias, tb_stride, stats, addend;
+    float scale;
+    ConvPlanFields plan;
+};
+
 Plan* find_plan(Engine* e, int B, int F, int T) {
     auto it = e->plans.find(std::make_tuple(B, F, T));
     return it == e->plans.end() ? nullptr : it->second;
@@ -877,18 +918,7 @@ int snrse_ncsnpp_set_weights(void* handle, const void* device_blob) {
 //        attention and input packing); no other bit is defined
 int64_t snrse_ncsnpp_plan_bytes(void* handle, int B, int F, int T, int flags) {
     Engine* e = static_cast<Engine*>(handle);
-    if (flags & ~3) {
-        snrse_set_error("plan: unknown flags 0x%x (bit0: keep every activation, bit1: CUDA-core cross-check)", flags);
-        return -1;
-    }
-    if (!e || B < 1 || F < 1 || T < 1 || (F % (1 << (e->n_levels - 1))) || (T % (1 << (e->n_levels - 1)))) {
-        snrse_set_error("plan: F and T must be positive multiples of 2^(levels-1) (got B=%d F=%d T=%d)", B, F, T);
-        return -1;
-    }
-    if (F != e->image_size) {
-        snrse_set_error("plan: F=%d differs from the image_size=%d the attention placement was built for", F, e->image_size);
-        return -1;
-    }
+    if (!plan_args_ok(e, B, F, T, flags)) return -1;
     Plan* p = find_plan(e, B, F, T);
     if (p && p->flags != flags) {
         delete p;
@@ -973,6 +1003,50 @@ int snrse_ncsnpp_profile_forward(void* handle, int B, int F, int T, const void* 
     }
     for (auto& v : ev) cudaEventDestroy(v);
     *n_groups = n;
+    return SNRSE_OK;
+}
+
+// Debug: the convolutions of the (B,F,T) plan with these flags, recorded as snrse_ncsnpp_plan_bytes records them but
+// into a plan of its own (nothing cached, no weights, no device), with their plan fields for num_sms SMs.
+int snrse_ncsnpp_dbg_convs(void* handle, int B, int F, int T, int flags, int num_sms, void* rows, int cap, int* n) {
+    Engine* e = static_cast<Engine*>(handle);
+    SNRSE_CHECK_ARG(n && num_sms >= 2, "dbg_convs: bad arguments");
+    if (!plan_args_ok(e, B, F, T, flags)) return SNRSE_ERR_ARG;
+    Plan P;
+    P.eng = e; P.B = B; P.F = F; P.T = T; P.flags = flags;
+    P.cross_check = (flags & 2) != 0;
+    SNRSE_TRY(record_plan(P));
+    *n = (int)P.convs.size();
+    if (!rows) return SNRSE_OK;
+    SNRSE_CHECK_ARG(cap >= *n, "dbg_convs: %d rows do not fit %d", *n, cap);
+    ConvRow* out = static_cast<ConvRow*>(rows);
+    for (const Plan::ConvRec& c : P.convs) {
+        ConvRow r{};
+        const LT& x = P.tens[c.x];
+        r.path = c.path; r.out4 = c.out4; r.B = x.B; r.H = x.H; r.W = x.W;
+        r.c0 = x.C; r.ld0 = P.tens[P.root(c.x)].C; r.off0 = P.chan_off(c.x);
+        if (c.shortcut >= 0) {
+            r.c1 = P.tens[c.shortcut].C; r.ld1 = P.tens[P.root(c.shortcut)].C; r.off1 = P.chan_off(c.shortcut);
+        }
+        if (c.res >= 0) {
+            r.res = 1; r.ld_res = P.tens[P.root(c.res)].C; r.off_res = P.chan_off(c.res);
+        }
+        r.ld_out = P.tens[P.root(c.out)].C; r.off_out = P.chan_off(c.out);
+        r.taps = c.taps; r.n = c.n_rows; r.norm = c.norm; r.bias = c.bias; r.tbias = c.tbias;
+        r.tb_stride = c.tbias ? e->dense_rows : 0;
+        r.stats = c.stats; r.addend = c.addend; r.scale = c.scale;
+        if (c.path == 0) {
+            ConvHaloPlan hp;
+            SNRSE_TRY(c.out4 ? conv_halo2_plan_shape_out4(&hp, r.B, r.H, r.W, r.c0, num_sms)
+                             : conv_halo2_plan_shape(&hp, r.B, r.H, r.W, r.c0, r.c1, r.n, r.norm, num_sms));
+            r.plan = conv_plan_fields(hp);
+        } else if (c.path == 2) {
+            ConvGemmPlan gp;
+            SNRSE_TRY(conv_gemm_plan_shape(&gp, r.B, r.H, r.W, r.taps, r.c0, r.c1, r.n, num_sms));
+            r.plan = conv_plan_fields(gp);
+        }
+        *out++ = r;
+    }
     return SNRSE_OK;
 }
 

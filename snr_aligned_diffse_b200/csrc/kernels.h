@@ -37,6 +37,7 @@ struct ConvGemmPlan {
     int stages;
     int a_box_bytes;  // bytes per activation TMA box (box height = min(tile rows, H))
     int smem_bytes;
+    int small;        // few pixel tiles: 64-column N tiles and a deep ring
 };
 // a0: segment-0 input view (taps0 taps); a1: optional segment-1 input (1 tap, may be null).
 // wt: [n_rows, Ktot] bf16, K-major, Ktot = (taps0*C0 + C1); for b_batched the matrix of batch b starts at
@@ -49,6 +50,10 @@ int conv_gemm_make_plan_ex(ConvGemmPlan* p, const ActView* a0, int taps0, const 
                            int64_t wt_batch_stride, int b_batched, const float* bias, const float* tbias, int tb_stride,
                            const ActView* res, float scale, void* out, int out_ld, int out_f32, int64_t wt_row_pitch);
 int conv_gemm_launch(const ConvGemmPlan* p, cudaStream_t s);
+// The shape-only part of conv_gemm_make_plan_ex: tile shape, N tile, small-map mode, ring depth and shared memory of a
+// convolution of a B x H x W map (C0 channels, taps0 taps, C1 shortcut channels) to n_rows outputs on num_sms SMs.
+// Touches no device and no tensor map; conv_gemm_make_plan_ex calls it with the device's SM count.
+int conv_gemm_plan_shape(ConvGemmPlan* p, int B, int H, int W, int taps0, int C0, int C1, int n_rows, int num_sms);
 
 // ----------------------------------------------------------------------------- conv_halo2.cu
 // Plan of the persistent 2-CTA halo-reuse kernel: 3x3 convolutions with W >= 8, H >= 8, N in {128, 256}.
@@ -82,11 +87,38 @@ int conv_halo2_make_plan(ConvHaloPlan* p, const ActView* a0, const ActView* a1, 
 // ustats (nullable): the epilogue also accumulates the GroupNorm sums of the result into [B][N/4][2] (zeroed by the
 // caller; gn_finalize_launch source format), so the following GroupNorm needs no pass over the tensor.
 int conv_halo2_launch(const ConvHaloPlan* p, cudaStream_t s);
+// The shape-only parts of conv_halo2_make_plan (norm: operand normalised in flight) and conv_halo2_make_plan_out4: SUB,
+// tiles, N split, accumulator buffers, ring depths, shortcut ring, persistent grid and shared memory on num_sms SMs.
+// They touch no device and no tensor map; the make_plan functions call them with the device's SM count.
+int conv_halo2_plan_shape(ConvHaloPlan* p, int B, int H, int W, int C0, int C1, int n_rows, int norm, int num_sms);
+int conv_halo2_plan_shape_out4(ConvHaloPlan* p, int B, int H, int W, int C0, int num_sms);
 
 // Thin 3x3 output convolution C -> 4 on the 2-CTA kernel (N = 16, weights [16][9*C] bf16 with rows 4..15 zero), fp32
 // result [B,H,W,4] = conv + bias4 (+ addend4); scsh as above.  Needs W >= 8, H >= 8.
 int conv_halo2_make_plan_out4(ConvHaloPlan* p, const ActView* a0, const bf16* wt16, const float* bias4, const float* addend4,
                               float* out4, const float* scsh);
+
+// The integer fields of either convolution plan, as the debug entry points report them (snrse_conv_plan of
+// include/snrse_b200_plans.h mirrors this struct); fields of the other kernel stay 0.
+struct ConvPlanFields {
+    int sub, nsplit, n_loc, acc_bufs, na, nb, stg_bufs, nsc;   // 2-CTA kernel (n_loc: output channels per cluster)
+    int th, tw, n_tile, small, stages;                         // single-CTA implicit GEMM
+    int tiles_h, tiles_w, n_tiles, grid, smem_bytes;           // both (grid: CTAs launched, GEMM: both grid dimensions)
+};
+inline ConvPlanFields conv_plan_fields(const ConvHaloPlan& p) {
+    ConvPlanFields f{};
+    f.sub = p.sub; f.nsplit = p.nsplit; f.n_loc = p.N; f.acc_bufs = p.acc_bufs;
+    f.na = p.na; f.nb = p.nb; f.stg_bufs = p.stg_bufs; f.nsc = p.nsc;
+    f.tiles_h = p.tiles_h; f.tiles_w = p.tiles_w; f.n_tiles = p.n_tiles; f.grid = p.grid; f.smem_bytes = p.smem_bytes;
+    return f;
+}
+inline ConvPlanFields conv_plan_fields(const ConvGemmPlan& p) {
+    ConvPlanFields f{};
+    f.th = 1 << p.th_log2; f.tw = 1 << p.tw_log2; f.n_tile = p.n_tile; f.small = p.small; f.stages = p.stages;
+    f.tiles_h = p.tiles_h; f.tiles_w = p.tiles_w; f.n_tiles = p.B * p.tiles_h * p.tiles_w;
+    f.grid = f.n_tiles * cdiv(p.N, p.n_tile); f.smem_bytes = p.smem_bytes;
+    return f;
+}
 
 // ----------------------------------------------------------------------------- conv_simt.cu
 // Reference-grade direct convolution on CUDA cores (debug / cross-check path, fp32 accumulate).

@@ -20,6 +20,13 @@ FLAG_SIMT_CONV = 2    # CUDA-core cross-check convolutions instead of tcgen05
 
 MODE_RAW, MODE_SEBRIDGE, MODE_NEG = 0, 1, 2
 
+# snrse_conv_plan / snrse_conv_row of include/snrse_b200_plans.h, field for field
+CONV_PLAN_FIELDS = ("sub", "nsplit", "n_loc", "acc_bufs", "na", "nb", "stg_bufs", "nsc", "th", "tw", "n_tile", "small",
+                    "stages", "tiles_h", "tiles_w", "n_tiles", "grid", "smem_bytes")
+CONV_ROW_FIELDS = ("path", "out4", "B", "H", "W", "c0", "ld0", "off0", "c1", "ld1", "off1", "res", "ld_res", "off_res",
+                   "ld_out", "off_out", "taps", "n", "norm", "bias", "tbias", "tb_stride", "stats", "addend", "scale") \
+    + CONV_PLAN_FIELDS
+
 
 class NCSNppEngine:
     """One packed copy of the weights on one GPU + per-(B,F,T) launch plans."""
@@ -251,6 +258,18 @@ class NCSNppEngine:
                                                          _lib.ptr(t), _lib.ptr(out), mode, _lib.stream_ptr(), n, kinds,
                                                          fl, by, ms, byref(cnt)), "profile_forward")
         return [dict(kind=kinds[i], flops=fl[i], bytes=by[i], ms=ms[i]) for i in range(cnt.value)]
+
+    def conv_rows(self, B, F, T, flags=0, num_sms=148):
+        """Every convolution the (B,F,T) plan records, with its operand views and its plan for num_sms SMs
+        (snrse_ncsnpp_dbg_convs; no device needed): a numpy structured array with the fields CONV_ROW_FIELDS."""
+        import numpy as np
+        dtype = np.dtype([(f, np.float32 if f == "scale" else np.int32) for f in CONV_ROW_FIELDS])
+        n = c_int()
+        _lib.check(self.lib.snrse_ncsnpp_dbg_convs(self.h, B, F, T, flags, num_sms, None, 0, byref(n)), "dbg_convs")
+        rows = np.zeros(n.value, dtype)
+        _lib.check(self.lib.snrse_ncsnpp_dbg_convs(self.h, B, F, T, flags, num_sms, rows.ctypes.data, n.value, byref(n)),
+                   "dbg_convs")
+        return rows
 
     def num_launch_groups(self, B, F, T):
         return int(self.lib.snrse_ncsnpp_num_launch_groups(self.h, B, F, T))
