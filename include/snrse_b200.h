@@ -81,6 +81,27 @@ int snrse_snr_ratio(const float* g, float* ratio, int B, void* stream);  /* est_
  * and X_T = Y + sigma*t*Z (model.py:822-823). */
 int snrse_lincomb(const void* x, const void* y, const void* s, const void* z, const float* a, const float* b,
                   const float* c, const float* d, void* out_mean, void* out_x, int B, int64_t n, void* stream);
+/* snrse_lincomb_keyed: snrse_lincomb with z drawn in the kernel from a per-item key instead of read from memory, so that
+ *   an utterance's noise depends on its key and the seed only, never on its row, its batch or earlier draws.  Same
+ *   arithmetic as snrse_lincomb: out_x is bit-identical to snrse_lincomb(..., z = the draw written to z_out, ...).
+ *   keys: uint64 [B]; n must be 256 * tpad (item b is complex64 [256][tpad], row-major); z_out (optional): the draw,
+ *   complex64 [B][n].  len (optional, int32 [B]): an item whose own padded width 64*ceil((1 + len[b]/128)/64) is not
+ *   tpad is written as NaN in out_mean, out_x and z_out, since enhancing it at width tpad is not enhancing it alone.
+ *
+ *   Keyed noise (a stable format): complex element i (0 <= i < n) of item b with key k and seed s is
+ *     (x0, x1, x2, x3) = Philox4x32-10(counter = (i >> 1, 0, lo32(k), hi32(k)), key = (lo32(s), hi32(s)))
+ *   (Salmon et al., "Parallel random numbers: as easy as 1, 2, 3", SC'11; curand's Philox4_32_10), with
+ *     (xa, xb) = (x0, x1) for even i, (x2, x3) for odd i,
+ *     u1 = ((xa >> 8) + 1) * 2^-24 in (0, 1],  u2 = (xb >> 8) * 2^-24 in [0, 1)   (both exact in fp32),
+ *     r = sqrtf(-logf(u1)),  z = r * cospi(2 u2) + i r * sinpi(2 u2)   (accurate logf / sqrtf / sincospif).
+ *   re z and im z are independent N(0, 1/2), so E|z|^2 = 1 as torch.randn_like draws on complex64; |z|^2 ~ Exp(1)
+ *   truncated at 24 ln 2 (probability 6e-8 per draw).  The counter's second word is 0 here and reserved.
+ *   Known answers: counter (0,0,0,0), key (0,0) -> 6627e8d5 e169c58d bc57ac4c 9b00dbd8; all ones ->
+ *   408f276d 41c83b0e a20bc7c6 6d5451fd; counter (243f6a88, 85a308d3, 13198a2e, 03707344), key (a4093822, 299f31d0)
+ *   -> d16cfe09 94fdcceb 5001e420 24126ea1. */
+int snrse_lincomb_keyed(const void* x, const void* y, const void* s, const float* a, const float* b, const float* c,
+                        const float* d, const uint64_t* keys, uint64_t seed, const int* len, int tpad, void* z_out,
+                        void* out_mean, void* out_x, int B, int64_t n, void* stream);
 
 /* Embedded Runge-Kutta helpers for the probability-flow ODE sampler kept on the device (replaces the numpy round trip
  * per RHS evaluation of `ode_sampler`, sampling/__init__.py:149-161; step control follows scipy.integrate RK45, the

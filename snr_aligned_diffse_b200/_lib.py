@@ -6,14 +6,14 @@ fallback implementation behind these calls.
 """
 import ctypes
 import os
-from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int64, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int64, c_uint64, c_void_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libsnrse_b200.so")
 
 _lib = None
 
-vp, i32, i64, f32, f64 = c_void_p, c_int, c_int64, c_float, c_double
+vp, i32, i64, u64, f32, f64 = c_void_p, c_int, c_int64, c_uint64, c_float, c_double
 
 # name -> (restype, argtypes); every symbol declared in include/snrse_b200.h
 PROTOTYPES = {
@@ -31,6 +31,7 @@ PROTOTYPES = {
     "snrse_v3_scalars": (i32, [vp, vp, f64, f32, vp, vp, vp, vp, i32, vp]),
     "snrse_snr_ratio": (i32, [vp, vp, i32, vp]),
     "snrse_lincomb": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i64, vp]),
+    "snrse_lincomb_keyed": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, u64, vp, i32, vp, vp, vp, i32, i64, vp]),
     "snrse_rk_combine": (i32, [vp, vp, i32, i64, f32, vp, vp, vp]),
     "snrse_rk_partials": (i32, [i64]),
     "snrse_rk_scaled_sqnorm": (i32, [vp, i32, i64, f32, vp, vp, vp, f32, f32, vp, vp]),

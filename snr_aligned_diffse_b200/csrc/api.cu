@@ -117,6 +117,15 @@ int snrse_lincomb(const void* x, const void* y, const void* sc, const void* z, c
                           static_cast<float2*>(out_x), B, n, S(stream));
 }
 
+int snrse_lincomb_keyed(const void* x, const void* y, const void* sc, const float* a, const float* b, const float* c,
+                        const float* d, const uint64_t* keys, uint64_t seed, const int* len, int tpad, void* z_out,
+                        void* out_mean, void* out_x, int B, int64_t n, void* stream) {
+    return lincomb_keyed_launch(static_cast<const float2*>(x), static_cast<const float2*>(y),
+                                static_cast<const float2*>(sc), a, b, c, d, reinterpret_cast<const unsigned long long*>(keys),
+                                (unsigned long long)seed, len, tpad, static_cast<float2*>(z_out),
+                                static_cast<float2*>(out_mean), static_cast<float2*>(out_x), B, n, S(stream));
+}
+
 int snrse_rk_combine(const void* y, const void* K, int nk, int64_t n, float h, const float* coef, void* out, void* stream) {
     return rk_combine_launch(static_cast<const float2*>(y), static_cast<const float2*>(K), nk, n, h, coef,
                              static_cast<float2*>(out), S(stream));

@@ -185,6 +185,10 @@ int final_launch(const float* p4, const float* t, const float* w, const float* b
 // out_mean = a*x + b*y + c*s ; out_x = out_mean + d*z   (per-batch coefficient arrays, any pointer may alias)
 int lincomb_launch(const float2* x, const float2* y, const float2* sc, const float2* z, const float* a, const float* b,
                    const float* c, const float* d, float2* out_mean, float2* out_x, int B, int64_t n, cudaStream_t s);
+int lincomb_keyed_launch(const float2* x, const float2* y, const float2* sc, const float* a, const float* b,
+                         const float* c, const float* d, const unsigned long long* keys, unsigned long long seed,
+                         const int* len, int tpad, float2* z_out, float2* out_mean, float2* out_x, int B, int64_t n,
+                         cudaStream_t s);
 
 // embedded Runge-Kutta helpers of the on-device ODE sampler (coef: nk host floats; K: nk stages of n complex values)
 int rk_combine_launch(const float2* y, const float2* K, int nk, int64_t n, float h, const float* coef, float2* out,

@@ -7,6 +7,7 @@
 //   lincomb    : x_mean = a*x + b*y + c*s,  x' = x_mean + d*z   -- covers prior sampling
 //                (sdes.py:225-232), annealed Langevin (correctors.py:69-81) and the reverse-diffusion
 //                predictor (predictors.py:75-80, sdes.py:73-91,132-140) with host-computed coefficients.
+//   lincomb_keyed : the same with z drawn in the kernel from a per-item key (the keyed noise of snrse_b200.h).
 #include "kernels.h"
 
 namespace {
@@ -75,10 +76,58 @@ final_kernel(const float4* __restrict__ p4, const float* __restrict__ t, const f
     out[(int64_t)b * n + i] = make_float2(re, im);
 }
 
+// Noise operand of lincomb_kernel.  NoiseIn reads z from memory (snrse_lincomb); NoiseKeyed draws it from
+// (key[b], seed, element index) as snrse_b200.h specifies (snrse_lincomb_keyed).
+struct NoiseIn {
+    const float2* z;
+    __device__ bool present() const { return z != nullptr; }
+    __device__ bool item_ok(int) const { return true; }
+    __device__ float2 operator()(int, int64_t, int64_t o) const { return __ldg(z + o); }
+};
+
+// Philox4x32-10 (Salmon et al., SC'11; curand's Philox4_32_10)
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    return c;
+}
+
+struct NoiseKeyed {
+    const unsigned long long* keys;
+    unsigned long long seed;
+    const int* len;    // optional: item b is NaN unless its own padded width equals tpad
+    int tpad;
+    float2* z_out;     // optional copy of the draw
+    __device__ bool present() const { return true; }
+    __device__ bool item_ok(int b) const { return !len || 64 * ((1 + len[b] / 128 + 63) / 64) == tpad; }
+    __device__ float2 operator()(int b, int64_t i, int64_t o) const {
+        const unsigned long long k = keys[b];
+        const uint4 r = philox4x32_10(make_uint4((uint32_t)(i >> 1), 0u, (uint32_t)k, (uint32_t)(k >> 32)),
+                                      (uint32_t)seed, (uint32_t)(seed >> 32));
+        const uint32_t xa = (i & 1) ? r.z : r.x, xb = (i & 1) ? r.w : r.y;
+        const float u1 = (float)((xa >> 8) + 1u) * 0x1p-24f;     // (0, 1], exact
+        const float u2 = (float)(xb >> 8) * 0x1p-24f;            // [0, 1), exact
+        const float rad = sqrtf(-logf(u1));
+        float sn, cs;
+        sincospif(2.f * u2, &sn, &cs);
+        float2 v = make_float2(rad * cs, rad * sn);
+        if (!item_ok(b)) v = make_float2(__int_as_float(0x7fc00000), __int_as_float(0x7fc00000));
+        if (z_out) z_out[o] = v;
+        return v;
+    }
+};
+
+template <class Noise>
 __global__ void __launch_bounds__(256)
-lincomb_kernel(const float2* __restrict__ x, const float2* __restrict__ y, const float2* __restrict__ sc,
-               const float2* __restrict__ z, const float* __restrict__ a, const float* __restrict__ bq,
-               const float* __restrict__ c, const float* __restrict__ d, float2* out_mean, float2* out_x, int64_t n) {
+lincomb_kernel(const float2* __restrict__ x, const float2* __restrict__ y, const float2* __restrict__ sc, Noise z,
+               const float* __restrict__ a, const float* __restrict__ bq, const float* __restrict__ c,
+               const float* __restrict__ d, float2* out_mean, float2* out_x, int64_t n) {
     pdl_sync();
     const int b = blockIdx.y;
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -88,8 +137,11 @@ lincomb_kernel(const float2* __restrict__ x, const float2* __restrict__ y, const
     if (x) { const float2 v = x[o]; const float k = a[b]; re = k * v.x; im = k * v.y; }
     if (y) { const float2 v = y[o]; const float k = bq[b]; re = fmaf(k, v.x, re); im = fmaf(k, v.y, im); }
     if (sc) { const float2 v = sc[o]; const float k = c[b]; re = fmaf(k, v.x, re); im = fmaf(k, v.y, im); }
+    float2 zv = make_float2(0.f, 0.f);
+    if (z.present()) zv = z(b, i, o);     // before the first store: NoiseIn's z must not wait for out_mean
+    if (!z.item_ok(b)) re = im = __int_as_float(0x7fc00000);
     if (out_mean) out_mean[o] = make_float2(re, im);
-    if (z) { const float2 v = z[o]; const float k = d[b]; re = fmaf(k, v.x, re); im = fmaf(k, v.y, im); }
+    if (z.present()) { const float k = d[b]; re = fmaf(k, zv.x, re); im = fmaf(k, zv.y, im); }
     if (out_x) out_x[o] = make_float2(re, im);
 }
 
@@ -252,7 +304,21 @@ int final_launch(const float* p4, const float* t, const float* w, const float* b
 int lincomb_launch(const float2* x, const float2* y, const float2* sc, const float2* z, const float* a, const float* b,
                    const float* c, const float* d, float2* out_mean, float2* out_x, int B, int64_t n, cudaStream_t s) {
     dim3 grid((unsigned)cdiv64(n, 256), B);
-    snrse_launch(lincomb_kernel, dim3(grid), dim3(256), 0, s, x, y, sc, z, a, b, c, d, out_mean, out_x, n);
+    snrse_launch(lincomb_kernel<NoiseIn>, dim3(grid), dim3(256), 0, s, x, y, sc, NoiseIn{z}, a, b, c, d, out_mean, out_x, n);
+    SNRSE_LAUNCH_CHECK();
+    return SNRSE_OK;
+}
+
+int lincomb_keyed_launch(const float2* x, const float2* y, const float2* sc, const float* a, const float* b,
+                         const float* c, const float* d, const unsigned long long* keys, unsigned long long seed,
+                         const int* len, int tpad, float2* z_out, float2* out_mean, float2* out_x, int B, int64_t n,
+                         cudaStream_t s) {
+    SNRSE_CHECK_ARG(keys && d, "lincomb_keyed: null keys or noise coefficient");
+    SNRSE_CHECK_ARG(tpad >= 1 && n == 256 * (int64_t)tpad, "lincomb_keyed: n = %lld is not 256 x tpad (tpad %d)",
+                    (long long)n, tpad);
+    dim3 grid((unsigned)cdiv64(n, 256), B);
+    snrse_launch(lincomb_kernel<NoiseKeyed>, dim3(grid), dim3(256), 0, s, x, y, sc, NoiseKeyed{keys, seed, len, tpad, z_out},
+                 a, b, c, d, out_mean, out_x, n);
     SNRSE_LAUNCH_CHECK();
     return SNRSE_OK;
 }

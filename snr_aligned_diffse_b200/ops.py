@@ -104,29 +104,34 @@ def v3_scalars(ratio, peak, fixed_snr):
     return t, nf, idx
 
 
+def _lincomb_operands(name, ops_):
+    """Validated operands of lincomb / lincomb_keyed: (first operand, B, {key: tensor}, {key: coefficient})."""
+    present = [(k, t, co) for k, (t, co) in ops_.items() if t is not None]
+    if not present:
+        raise ValueError(f"{name}: no operand given")
+    ref = present[0][1]
+    B = ref.shape[0]
+    tensors, coefs = {}, {}
+    for k, t, co in present:
+        if not (torch.is_tensor(t) and t.is_cuda and t.dtype == torch.complex64):
+            raise ValueError(f"{name}: operand {k} must be a CUDA complex64 tensor (got "
+                             f"{getattr(t, 'dtype', type(t))} on {getattr(t, 'device', 'host')})")
+        if t.shape != ref.shape or t.device != ref.device:
+            raise ValueError(f"{name}: operand {k} has shape {tuple(t.shape)} on {t.device}, expected "
+                             f"{tuple(ref.shape)} on {ref.device} (operands must match exactly; no broadcasting)")
+        if co is None or not (torch.is_tensor(co) and co.is_cuda and co.dtype == torch.float32 and co.numel() == B):
+            raise ValueError(f"{name}: coefficient of {k} must be a CUDA float32 vector with {B} elements")
+        tensors[k], coefs[k] = t.contiguous(), co.contiguous()
+    return ref, B, tensors, coefs
+
+
 def lincomb(x=None, y=None, s=None, z=None, a=None, b=None, c=None, d=None, want_mean=True, want_x=True):
     """out_mean = a x + b y + c s; out_x = out_mean + d z  on complex64 [B, ...] tensors; a..d are [B] float32
     coefficient vectors (one per operand present).  Every sampler state update is built on this call, so operands are
     validated here: all on one CUDA device, complex64, identical shapes (the reference's elementwise ops would raise a
     broadcast error on a mismatch), made contiguous before their raw pointers are handed to the kernel."""
     lib = _lib_dev()
-    ops_ = {"x": (x, a), "y": (y, b), "s": (s, c), "z": (z, d)}
-    present = [(k, t, co) for k, (t, co) in ops_.items() if t is not None]
-    if not present:
-        raise ValueError("lincomb: no operand given")
-    ref = present[0][1]
-    B = ref.shape[0]
-    tensors, coefs = {}, {}
-    for k, t, co in present:
-        if not (torch.is_tensor(t) and t.is_cuda and t.dtype == torch.complex64):
-            raise ValueError(f"lincomb: operand {k} must be a CUDA complex64 tensor (got "
-                             f"{getattr(t, 'dtype', type(t))} on {getattr(t, 'device', 'host')})")
-        if t.shape != ref.shape or t.device != ref.device:
-            raise ValueError(f"lincomb: operand {k} has shape {tuple(t.shape)} on {t.device}, expected "
-                             f"{tuple(ref.shape)} on {ref.device} (operands must match exactly; no broadcasting)")
-        if co is None or not (torch.is_tensor(co) and co.is_cuda and co.dtype == torch.float32 and co.numel() == B):
-            raise ValueError(f"lincomb: coefficient of {k} must be a CUDA float32 vector with {B} elements")
-        tensors[k], coefs[k] = t.contiguous(), co.contiguous()
+    ref, B, tensors, coefs = _lincomb_operands("lincomb", {"x": (x, a), "y": (y, b), "s": (s, c), "z": (z, d)})
     n = ref.numel() // B
     shape = ref.shape
     out_mean = torch.empty(shape, dtype=torch.complex64, device=ref.device) if want_mean else None
@@ -137,6 +142,58 @@ def lincomb(x=None, y=None, s=None, z=None, a=None, b=None, c=None, d=None, want
                                  _lib.ptr(g(coefs, "s")), _lib.ptr(g(coefs, "z")), _lib.ptr(out_mean), _lib.ptr(out_x), B, n,
                                  _lib.stream_ptr()), "lincomb")
     return out_mean, out_x
+
+
+def key_tensor(keys, B=None):
+    """Per-item 64-bit noise keys as an int64 tensor (the kernel reads its bits as uint64).  keys: a sequence of Python
+    ints in [-2^63, 2^64) (values >= 2^63 wrap to their two's complement) or an integer tensor, host or device."""
+    if torch.is_tensor(keys):
+        if keys.dtype not in (torch.int64, torch.int32, torch.int16, torch.int8, torch.uint8):
+            raise ValueError(f"keys must be an integer tensor (got {keys.dtype})")
+        kt = keys.reshape(-1).to(torch.int64)
+    else:
+        vals = [int(k) for k in keys]
+        if any(not -(1 << 63) <= k < (1 << 64) for k in vals):
+            raise ValueError("keys must lie in [-2^63, 2^64)")
+        kt = torch.tensor([k - (1 << 64) if k >= (1 << 63) else k for k in vals], dtype=torch.int64)
+    if B is not None and kt.numel() != B:
+        raise ValueError(f"keys: expected {B} keys, got {kt.numel()}")
+    return kt
+
+
+def lincomb_keyed(x=None, y=None, s=None, a=None, b=None, c=None, d=None, keys=None, seed=0, lengths=None,
+                  want_mean=True, want_x=True, want_z=False):
+    """`lincomb` with z drawn in the kernel from the keyed noise of include/snrse_b200.h: item b's draw depends on
+    (keys[b], seed, element index) only.  Operands complex64 [B, ..., 256, Tpad]; d: [B] float32 coefficient of the
+    draw; keys: int64 [B] (CUDA, read as uint64; see `key_tensor`); seed: int in [0, 2^64); lengths: optional CUDA int32
+    [B], items whose own padded width is not Tpad come out NaN.  Returns (out_mean, out_x, z)."""
+    lib = _lib_dev()
+    ref, B, tensors, coefs = _lincomb_operands("lincomb_keyed", {"x": (x, a), "y": (y, b), "s": (s, c)})
+    if ref.dim() < 3 or ref.shape[-2] != N_BINS or ref.numel() // B != N_BINS * ref.shape[-1]:
+        raise ValueError(f"lincomb_keyed: operands must be [B, ..., {N_BINS}, Tpad] (got {tuple(ref.shape)})")
+    if d is None or not (torch.is_tensor(d) and d.is_cuda and d.dtype == torch.float32 and d.numel() == B):
+        raise ValueError(f"lincomb_keyed: coefficient of z must be a CUDA float32 vector with {B} elements")
+    if not (torch.is_tensor(keys) and keys.is_cuda and keys.dtype == torch.int64 and keys.numel() == B
+            and keys.device == ref.device):
+        raise ValueError(f"lincomb_keyed: keys must be a CUDA int64 vector with {B} elements on {ref.device}")
+    if lengths is not None and not (torch.is_tensor(lengths) and lengths.is_cuda and lengths.dtype == torch.int32
+                                    and lengths.numel() == B):
+        raise ValueError(f"lincomb_keyed: lengths must be a CUDA int32 vector with {B} elements")
+    seed = int(seed)
+    if not 0 <= seed < (1 << 64):
+        raise ValueError(f"lincomb_keyed: seed must lie in [0, 2^64) (got {seed})")
+    tpad = ref.shape[-1]
+    n = ref.numel() // B
+    shape = ref.shape
+    new = lambda on: torch.empty(shape, dtype=torch.complex64, device=ref.device) if on else None  # noqa: E731
+    out_mean, out_x, z = new(want_mean), new(want_x), new(want_z)
+    g = lambda d_, k: d_.get(k)  # noqa: E731
+    _lib.check(lib.snrse_lincomb_keyed(_lib.ptr(g(tensors, "x")), _lib.ptr(g(tensors, "y")), _lib.ptr(g(tensors, "s")),
+                                       _lib.ptr(g(coefs, "x")), _lib.ptr(g(coefs, "y")), _lib.ptr(g(coefs, "s")),
+                                       _lib.ptr(d.contiguous()), _lib.ptr(keys.contiguous()), seed,
+                                       _lib.ptr(None if lengths is None else lengths.contiguous()), tpad, _lib.ptr(z),
+                                       _lib.ptr(out_mean), _lib.ptr(out_x), B, n, _lib.stream_ptr()), "lincomb_keyed")
+    return out_mean, out_x, z
 
 
 def rk_combine(y, K, coef, h):

@@ -216,39 +216,70 @@ class ScoreModel(CheckpointedModule):
 
     # ------------------------------------------------------------------------------ enhancement
     def enhance_batch(self, y, lengths=None, oracle=False, noise_over_clean=None, noise=None, return_aux=False,
-                      generator=None):
+                      generator=None, keys=None, seed=0):
         """sebridge_v3 / snr_conditioned='true' enhancement of a padded batch, entirely on the GPU.
 
         y: [B, Lmax] float32 (host or device); lengths: optional [B] valid sample counts;
         noise_over_clean: [B] noise_rms/clean_rms when oracle=True; noise: optional explicit complex
         normal Z [B,1,256,Tpad], otherwise drawn from `generator` (a CUDA torch.Generator; default: torch's
         default CUDA generator).  Returns the enhanced batch [B, Lmax] on the GPU (zeros past each length).
-        One pass = model.py:713-752,810-830 for every utterance, with no host synchronisation."""
+        One pass = model.py:713-752,810-830 for every utterance, with no host synchronisation.
+
+        keys: optional per-utterance 64-bit noise keys (int64 [B] or a list of ints, host or device; see
+        `ops.key_tensor`) with `seed` (int in [0, 2^64)).  Then every utterance is enhanced as if alone: Z is the keyed
+        noise of include/snrse_b200.h (a function of key, seed and element only) and the SNR estimate (oracle=False)
+        covers the utterance's own 16-frame clusters (`SNRModel.estimate_batch`), so item b equals
+        `enhance(None, y[b:b+1, :len_b], key=keys[b], seed=seed)` bit for bit whatever its row or batch.  Every
+        utterance must pad to the batch's Tpad (64*ceil((1 + len//128)/64) frames): host lengths that do not raise
+        ValueError, device lengths that do not make that item NaN.  keys cannot be combined with noise= or
+        generator=.  return_aux then also holds the draw Z [B,1,256,Tpad]."""
         if not (self.snr_conditioned == 'true' and self.model_type == 'sebridge_v3'):
             raise NotImplementedError("enhance_batch implements the sebridge_v3 SNR-conditioned path")
+        if keys is not None and (noise is not None or generator is not None):
+            raise ValueError("enhance_batch: keys= draws the noise itself; it cannot be combined with noise= or generator=")
         self.dnn._ensure_device_weights()
         yd = (y if y.is_cuda else y.cuda()).to(torch.float32).contiguous()
         B, L = yd.shape
         ld = None if lengths is None else lengths.to("cuda", torch.int32).contiguous()
         tr, alpha, beta = self._spec_params()
-        peak = ops.absmax(yd, ld)                                                  # y.abs().max()  (:715,726)
-        if oracle:
-            ratio = torch.as_tensor(noise_over_clean, dtype=torch.float32).reshape(-1).to("cuda")
-            if ratio.numel() == 1 and B > 1:
-                ratio = ratio.expand(B).contiguous()
+        if keys is not None:
+            kd = ops.key_tensor(keys, B).to(yd.device)
+            if lengths is not None and not torch.as_tensor(lengths).is_cuda:
+                tp = ops.padded_frames(L)
+                own = [ops.padded_frames(int(n)) for n in torch.as_tensor(lengths).reshape(-1).tolist()]
+                if any(t_ != tp for t_ in own):
+                    raise ValueError(f"enhance_batch: with keys every utterance must pad to the batch's {tp} frames "
+                                     f"(lengths {torch.as_tensor(lengths).tolist()} pad to {own})")
+        if keys is not None and not oracle:
+            ratio, est_aux = get_snr_model().estimate_batch(yd, lengths, return_aux=True)   # per file (:715-721)
+            peak = est_aux["peak"]
         else:
-            est = get_snr_model()
-            feat = ops.stft(yd, ld, scale=peak, scale_is_divisor=True, transform=False, planar=True, pad_multiple=16)
-            g = est.dnn.forward(feat)[:, 0].contiguous()                           # n/(s+n)  (:716-720)
-            ratio = est.dnn.engine.noise_over_clean(g)                             # (:721)
+            peak = ops.absmax(yd, ld)                                              # y.abs().max()  (:715,726)
+            if oracle:
+                ratio = torch.as_tensor(noise_over_clean, dtype=torch.float32).reshape(-1).to("cuda")
+                if ratio.numel() == 1 and B > 1:
+                    ratio = ratio.expand(B).contiguous()
+            else:
+                est = get_snr_model()
+                feat = ops.stft(yd, ld, scale=peak, scale_is_divisor=True, transform=False, planar=True, pad_multiple=16)
+                g = est.dnn.forward(feat)[:, 0].contiguous()                       # n/(s+n)  (:716-720)
+                ratio = est.dnn.engine.noise_over_clean(g)                         # (:721)
         t, norm, idx = ops.v3_scalars(ratio, peak, self.fixed_snr)                # (:732-740)
         Y = ops.stft(yd, ld, scale=norm, scale_is_divisor=True, transform=tr, alpha=alpha, beta=beta)   # (:746-751)
-        Z = torch.randn_like(Y, generator=generator) if noise is None else noise.to("cuda").reshape(Y.shape).contiguous()
-        X_T = axpby(y=Y, b=1.0, z=Z, d=t * float(self.sigma_max))                 # (:822-823)
+        if keys is not None:                                                       # (:822-823), keyed Z
+            ones = torch.ones(B, dtype=torch.float32, device=Y.device)
+            _, X_T, Z = ops.lincomb_keyed(y=Y, b=ones, d=t * float(self.sigma_max), keys=kd, seed=seed, lengths=ld,
+                                          want_mean=False, want_z=return_aux)
+        else:
+            Z = torch.randn_like(Y, generator=generator) if noise is None else noise.to("cuda").reshape(Y.shape).contiguous()
+            X_T = axpby(y=Y, b=1.0, z=Z, d=t * float(self.sigma_max))             # (:822-823)
         sample = self.dnn.engine.forward(X_T, Y, t, mode=MODE_SEBRIDGE)           # (:824, 537-541)
         x_hat = ops.istft(sample, L, ld, scale=norm, transform=tr, alpha=alpha, beta=beta)   # (:828-830)
         if return_aux:
-            return x_hat, dict(t=t, t_index=idx, norm_factor=norm, Y=Y, X_T=X_T, sample=sample, ratio=ratio)
+            aux = dict(t=t, t_index=idx, norm_factor=norm, Y=Y, X_T=X_T, sample=sample, ratio=ratio)
+            if keys is not None:
+                aux["Z"] = Z[:, None]
+            return x_hat, aux
         return x_hat
 
     def enhance_snr_sweep(self, x, noise, snrs=range(0, 41, 5), oracle=True, noise_draws=None):
@@ -270,15 +301,21 @@ class ScoreModel(CheckpointedModule):
     def enhance(self, x, y, sampler_type="pc", predictor="reverse_diffusion", corrector="ald", N=30,
                 corrector_steps=1, snr=0.5, timeit=False, oracle=False, clean_rms=1, noise_rms=1, **kwargs):
         """One-call enhancement of noisy speech `y` [1,L] (model.py:702-839).  `x` (clean) is accepted for
-        signature compatibility and unused.  Extra keyword `noise=` supplies the complex normal draw."""
+        signature compatibility and unused.  Extra keyword `noise=` supplies the complex normal draw; `key=k, seed=s`
+        (sebridge_v3) draw it as keyed noise instead, which is what `enhance_batch(..., keys=, seed=)` gives this file in
+        any batch."""
         sr = 16000
         start = time.time()
         noise = kwargs.pop("noise", None)
+        key, seed = kwargs.pop("key", None), kwargs.pop("seed", 0)
+        if key is not None and not (self.snr_conditioned == 'true' and self.model_type == 'sebridge_v3'):
+            raise NotImplementedError("key= (keyed noise) is implemented for the sebridge_v3 SNR-conditioned path")
         T_orig = y.size(1)
         nfe = 1
         if self.snr_conditioned == 'true' and self.model_type == 'sebridge_v3':
             ratio = None if not oracle else [noise_rms / clean_rms]
-            x_hat = self.enhance_batch(y, oracle=oracle, noise_over_clean=ratio, noise=noise)
+            x_hat = self.enhance_batch(y, oracle=oracle, noise_over_clean=ratio, noise=noise,
+                                       keys=None if key is None else [key], seed=seed)
         elif self.snr_conditioned == 'fixed':
             raise NotImplementedError("snr fixed is only for experiment purpose, not real inference.")
         elif self.snr_conditioned == 'false':

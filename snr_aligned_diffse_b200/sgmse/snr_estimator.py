@@ -30,7 +30,8 @@ class SNRModel(CheckpointedModule):
         16 frames, SNRNet over those clusters only.
 
         y: [B, L] float32, host or device; lengths: optional integer [B] valid sample counts, host or device (None: all
-        L).  Returns float32 [B] on the device; with return_aux also dict(g = n/(s+n) [B], clusters = int32 [B]).
+        L).  Returns float32 [B] on the device; with return_aux also dict(g = n/(s+n) [B], clusters = int32 [B],
+        peak = max|y| over each item's samples [B]).
         Lengths given on the host are checked there (1 <= len <= L, else ValueError).  Nothing synchronises with the
         host, so with device-resident lengths the call can be captured in a CUDA graph."""
         yd = (y if y.is_cuda else y.cuda()).to(torch.float32).contiguous()
@@ -55,7 +56,7 @@ class SNRModel(CheckpointedModule):
         g = self.dnn.forward(feat, clusters)[:, 0].contiguous()                              # n/(s+n)  (:716-720)
         ratio = self.dnn.engine.noise_over_clean(g)                                          # (:721)
         if return_aux:
-            return ratio, dict(g=g, clusters=clusters)
+            return ratio, dict(g=g, clusters=clusters, peak=peak)
         return ratio
 
     def calculate_normfac_direct(self, s, n, fixed_snr):

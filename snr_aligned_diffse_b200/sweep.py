@@ -32,7 +32,7 @@ def pack_batch(waves, idx, tpad, pin=False):
 
 
 def enhance_sweep(enhance_fn, waves, rank=0, world=1, max_batch=16, device=None, keep_audio=False, references=None,
-                  on_audio=None, target_frames=None):
+                  on_audio=None, target_frames=None, keys=None, seed=None):
     """Enhance the utterances `waves` (list of 1-D float tensors) this rank owns.
 
     enhance_fn(y [B, L] , lengths [B] int32) -> enhanced [B, L] (e.g. `lambda y, n: model.enhance_batch(y, lengths=n)`).
@@ -41,8 +41,17 @@ def enhance_sweep(enhance_fn, waves, rank=0, world=1, max_batch=16, device=None,
     target_frames: batches of about that many padded frames instead of at most `max_batch` utterances (`shard.bucket_batches`).
     on_audio(i, waveform): optional sink called with every enhanced utterance (host tensor) right after its batch, while
     the following batches are still being enqueued (used by `wavio.enhance_files` to write wavs off the critical path).
+    seed: keyed noise.  enhance_fn is then called as enhance_fn(y, lengths, keys [B] int64, seed), e.g.
+    `lambda y, n, k, s: model.enhance_batch(y, lengths=n, keys=k, seed=s)` or a `pipeline.GraphedEnhancerCache`, with
+    keys[i] (default: i, the utterance's index in `waves`; 64-bit ints) for utterance i, so that every utterance's
+    result depends on its samples, its key and the seed only -- not on the batching, the rank count or its neighbours.
     Returns dict(ids, samples, checksum, si_sdr, seconds, batches, audio) for this rank's shard."""
     lengths = [int(w.numel()) for w in waves]
+    if seed is not None:
+        from .ops import key_tensor
+        all_keys = key_tensor(range(len(waves)) if keys is None else keys, len(waves))
+    elif keys is not None:
+        raise ValueError("enhance_sweep: keys need a seed")
     batches = batch_shards(lengths, world, max_batch, target_frames=target_frames)[rank]
     ids, samples, checks, sdrs, audio = [], [], [], [], {}
     on_gpu = device is not None and torch.device(device).type == "cuda"
@@ -74,7 +83,11 @@ def enhance_sweep(enhance_fn, waves, rank=0, world=1, max_batch=16, device=None,
             refill()
             if device is not None:
                 y, lens = y.to(device, non_blocking=True), lens.to(device, non_blocking=True)
-            out = enhance_fn(y, lens)
+            if seed is None:
+                out = enhance_fn(y, lens)
+            else:
+                kt = all_keys[list(idx)]
+                out = enhance_fn(y, lens, kt if device is None else kt.to(device, non_blocking=True), seed)
             pos = torch.arange(out.shape[1], device=out.device)[None, :]
             valid = pos < lens.to(out.device)[:, None].to(pos.dtype)
             cs = (out.double() * valid).sum(1)            # per-utterance checksum over the valid samples only

@@ -8,6 +8,7 @@ batches, SI-SDR on the device when clean files are given), and a writer pool enc
 (float -> PCM16, what soundfile writes for .wav by default) while later batches are still on the GPU.
 Only the Python standard library's `wave` module is used for the container format.
 """
+import hashlib
 import os
 import wave
 from concurrent.futures import ThreadPoolExecutor
@@ -38,12 +39,20 @@ def write_wav(path, samples, sr=16000):
         w.writeframes(pcm.tobytes())
 
 
+def name_key(name):
+    """64-bit noise key of a file: blake2b-64 of its basename's UTF-8 bytes, as an unsigned int (stable across runs and
+    machines, unlike Python's salted `hash`)."""
+    return int.from_bytes(hashlib.blake2b(os.path.basename(name).encode("utf-8"), digest_size=8).digest(), "little")
+
+
 def enhance_files(enhance_fn, noisy_files, target_dir, clean_dir=None, rank=0, world=1, max_batch=16, device=None,
-                  io_threads=8, sr=16000):
+                  io_threads=8, sr=16000, seed=None):
     """The eval.py file loop over `noisy_files` (this rank's shard of it): returns the `enhance_sweep` metrics dict with
     `files` (basename per id) added; enhanced wavs are written to `target_dir/<basename>`.
 
-    enhance_fn(y [B, L], lengths [B]) -> enhanced [B, L]   (e.g. `lambda y, n: model.enhance_batch(y, lengths=n)`)."""
+    enhance_fn(y [B, L], lengths [B]) -> enhanced [B, L]   (e.g. `lambda y, n: model.enhance_batch(y, lengths=n)`).
+    seed: keyed noise (see `sweep.enhance_sweep`; enhance_fn then also takes keys and seed), each file keyed by
+    `name_key(basename)`, so a file's output does not depend on which other files are in the list."""
     from .sweep import enhance_sweep
     names = [os.path.basename(f) for f in noisy_files]
     with ThreadPoolExecutor(max_workers=io_threads) as pool:
@@ -64,7 +73,7 @@ def enhance_files(enhance_fn, noisy_files, target_dir, clean_dir=None, rank=0, w
         pending.append(writers.submit(write_wav, os.path.join(target_dir, names[i]), audio, sr))
 
     res = enhance_sweep(enhance_fn, waves, rank=rank, world=world, max_batch=max_batch, device=device, references=refs,
-                        on_audio=sink)
+                        on_audio=sink, keys=None if seed is None else [name_key(n) for n in names], seed=seed)
     for p in pending:
         p.result()
     writers.shutdown()
